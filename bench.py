@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps 2 --warmup 1      # CPU port of the reference path
+    python bench.py --steps 20 --warmup 5 --dump-outputs DIR   # also DIR/*.npy: loss, gradients, parameters of the last timed step
 
 One step = one pass of the hot path over one batch of 32 synthetic patient graphs per GPU
 (MultilevelGNN forward, BCE + feature loss, backward, gradient all-reduce, Adam), SURVEY.md section 8(d)
@@ -47,7 +48,13 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="do not capture the step as a CUDA graph")
     ap.add_argument("--nccl-update", action="store_true",
                     help="N>1: NCCL all-reduce + replicated Adam instead of the fused NVLink peer-memory update kernel")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (loss, every trained parameter's gradient and updated "
+                         "value) as DIR/<name>.npy, so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 train step; it has no meaning with --impl %s" % a.impl)
+    return a
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -183,6 +190,34 @@ KERNEL_INFO = {
                        "alg": "4*C*B*N (output) + 4*B*N + 8*nnz + 8*C*N (tables), C = 64: 137 MB, write bound"},
     "pool_bwd": {"ncu": ["pool_bwd_c32_kernel<2, 2>"], "alg": "2 * 4*C*B*N + 4*B*C*S*P: x read, g_x written, pooled gradient read"},
 }
+
+
+DUMP_BUDGET = 64 * 10 ** 6      # bytes --dump-outputs may write, all files together
+DUMP_SAMPLE = 1 << 20           # elements kept of a longer tensor (kirc's classifier head alone has 43 M)
+
+
+def last_step_outputs(tr, loss):
+    """What one Trainer.step hands its caller, as float32 numpy arrays: the loss it returns and, for every trained
+    parameter, the gradient of that step (grad.<name>) and the value Adam left (param.<name>).  A tensor of more than
+    DUMP_SAMPLE elements is reduced to the same seeded sample of its flattened elements in every run and every build."""
+    names = {id(p): n for n, p in tr.model.named_parameters()}
+    out = {"loss": loss.detach().float().cpu().numpy()}
+    for p in tr.params:
+        for kind, t in (("param", p.detach()), ("grad", p.grad)):
+            if t.numel() > DUMP_SAMPLE:
+                idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+                t = t.reshape(-1)[idx.to(t.device)]
+            out["%s.%s" % (kind, names[id(p)])] = t.float().cpu().numpy()
+    nbytes = sum(v.nbytes for v in out.values())
+    assert nbytes <= DUMP_BUDGET, "--dump-outputs: %d bytes > %d; lower DUMP_SAMPLE" % (nbytes, DUMP_BUDGET)
+    return out
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), v)
 
 
 def max_over_ranks(ms, world, dev):
@@ -546,6 +581,10 @@ def run_b200(a):
     clocks = sampler.stop() if sampler else None
     launches = launches_per_step * a.steps
     loss_value = float(loss.item())
+    dumped = None
+    if a.dump_outputs:          # read now: the legs below step the same trainer further
+        dumped = last_step_outputs(tr, loss) if rank == 0 else None
+        barrier(world)          # the other ranks wait here, not in a fused peer-update kernel that gives up after seconds
 
     # ---- end-to-end legs: pinned host batch -> device EVERY step (train.py:42), loss read back (train.py:62) ----
     # graph mode: the next batch's H2D runs on a copy stream while the current step's graph executes; the loss of EVERY step
@@ -705,6 +744,8 @@ def run_b200(a):
                                           % (cb, cores)}
     if world == 1 and not a.no_diffpool:
         line["diffpool"] = diffpool_legs(dev)
+    if dumped is not None:
+        write_outputs(a.dump_outputs, dumped)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
