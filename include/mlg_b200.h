@@ -345,6 +345,17 @@ int64_t mlg_wcolsum_workspace_bytes(int64_t rows, int64_t C);
 int mlg_wcolsum(const float* G, int64_t ld, const float* a, int64_t rows, int64_t C, float* u, float* v, void* workspace,
                 int64_t workspace_bytes, void* stream);
 
+/* Metrics of an evaluation split (train.py:71-109 of the reference), one kernel after a 32-byte memset of the workspace:
+ * out[0] = torch.nn.BCELoss(weight) of pred [n,2] against y [n,2] (mean over the 2n elements, logs clamped at -100, weight =
+ * the class row class_w [2], NULL = 1); out[1] = accuracy of argmax(pred) against argmax(y) (ties -> index 0, NaN is the
+ * maximum, as torch.argmax); out[2] = ROC AUC of pred[:,1] for the labels argmax(y), exactly: the Mann-Whitney count (2 per
+ * positive/negative pair with s_pos > s_neg, 1 per tie) in 64-bit integers over 2 P N -- NaN when one class is absent.
+ * Deterministic (integer atomics, fixed-order BCE sum): bit-identical results for the same inputs.  1 <= n <= 65 536
+ * (O(n^2) pair count).  workspace (8-byte aligned) >= mlg_eval_metrics_workspace_bytes(n). */
+int64_t mlg_eval_metrics_workspace_bytes(int64_t n);
+int mlg_eval_metrics(const float* pred, const float* y, int64_t n, const float* class_w, float* out, void* ws,
+                     int64_t ws_bytes, void* stream);
+
 /* Skinny Linear forward: out[rows,N] = act(x[rows,K] * W[N,K]^T + bias), rows <= 32, any K (long reduction).
  * MultilevelGNN's head Linear(6913 -> 256) on a batch of <= 32 graphs (models/multilevel_gnn.py:104-110): a batched
  * GEMV bound by the one pass over W.  act: 0 none, 1 LeakyReLU(slope) (slope 0 = ReLU).  fp32 FMA, fixed summation

@@ -119,6 +119,8 @@ _SIGNATURES = {
     "mlg_gen_aggr_bwd_affine_workspace_bytes": (_c_i64, [_c_i64, _c_i64, _c_i64]),
     "mlg_wcolsum_workspace_bytes": (_c_i64, [_c_i64, _c_i64]),
     "mlg_wcolsum": (_c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_i64, _c_vp]),
+    "mlg_eval_metrics_workspace_bytes": (_c_i64, [_c_i64]),
+    "mlg_eval_metrics": (_c_int, [_c_vp, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_i64, _c_vp]),
     "mlg_xty": (_c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_i64, _c_vp]),
     "mlg_bias_act": (_c_int, [_c_vp, _c_vp, _c_i64, _c_i64, _c_f32, _c_vp]),
     "mlg_embed_scale_fwd": (_c_int, [_c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_vp, _c_vp]),

@@ -121,7 +121,10 @@ class TopologyLoader:
     def set_epoch(self, epoch):
         self.epoch = epoch
 
-    def _index_batches(self):
+    def index_batches(self):
+        """The epoch's index tensors, one per batch of this rank.  Unshuffled without drop_last (evaluation): step s takes rows
+        [s*B*world + rank*B, ... + B) clipped to the dataset -- a tail batch may be short, a rank's last one empty, and every
+        rank has the same number of steps.  ``__iter__`` skips the empty ones."""
         n = len(self.dataset)
         if self.shuffle:
             return shard_indices(n, self.rank, self.world, self.batch_size, epoch_seed=self.seed + self.epoch,
@@ -133,10 +136,10 @@ class TopologyLoader:
                 for s in range(n_steps)]
 
     def __len__(self):
-        return len(self._index_batches())
+        return len(self.index_batches())
 
     def __iter__(self):
-        for idx in self._index_batches():
+        for idx in self.index_batches():
             if idx.numel() == 0:
                 continue
             yield collate([self.dataset[int(i)] for i in idx], self.topo, pin=self.pin)

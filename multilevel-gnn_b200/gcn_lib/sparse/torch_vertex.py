@@ -182,8 +182,12 @@ class SAGEConv(nn.Module):
             # x0 = xs * emb consumed in factored form when the whole layer is fused and the batch is replicated
             if slope is not None and topo.replicas > 1 and topo.n_single == x.emb.shape[0]:
                 lin = self.nn[0]
+                # with autograd off (MultilevelGNN.predict) no output gradient will ever need masking: the forward kernel then
+                # writes no sign bits.  Decided here -- inside a Function's forward the grad mode is always off, and
+                # ctx.needs_input_grad follows the inputs' requires_grad, not the caller's grad mode.
+                no_backward = not torch.is_grad_enabled()
                 return Fn.SageLayer.apply(x.emb, x.xs, self.lin_r.weight, lin.weight, lin.bias, topo, self.relative, slope,
-                                          None, out_premasked, link, None)
+                                          None, out_premasked or no_backward, link, None)
             x = x.materialize()
         x = x.unsqueeze(-1) if x.dim() == 1 else x
         if prod_link is not None and prod_link.get("h1_nm") and slope is None:

@@ -109,11 +109,12 @@ class MultilevelGNN(nn.Module):
         self.init_weight()
 
     # ------------------------------------------------------------------------------------------
-    def pool_genes(self, input_batch, x=None, gene_pca_match=None, raw_indice=None, value_mask=True):
+    def pool_genes(self, input_batch, x=None, gene_pca_match=None, raw_indice=None, value_mask=True, fused=False):
         """Level 1 -> level 2 (models/multilevel_gnn.py:140-239): embed-scale, the GraphConv stack on the gene graph, the
         value mask and the gene -> pathway projection pool.  Returns the pooled tensor [B, C, 438, P] (a permuted view of the
         channel-last buffer the pool kernel writes).  ``value_mask=False``: the VAE encoder's variant (models/vae.py:128-190,
-        where the mask lines are commented out)."""
+        where the mask lines are commented out).  ``fused``: take the fused layer chain even when autograd records nothing
+        (``predict``); by default it is taken only when it does."""
         args = self.args
         if x is not None:
             mask_x = x
@@ -157,7 +158,7 @@ class MultilevelGNN(nn.Module):
         # of y_i multiplies its input gradient by LeakyReLU'(y_i) inside its own backward kernel (it has y_i in
         # hand), and layer i takes that gradient as dL/dz -- one 3-tensor elementwise pass per layer saved.
         plain = self.FUSE_ACT_BACKWARD and xs.is_cuda and not args.dense_gnn and not args.resgnn \
-            and not args.repeat_mask and torch.is_grad_enabled()
+            and not args.repeat_mask and (fused or torch.is_grad_enabled())
         slopes = [getattr(l, "grad_fusion_slope", lambda: None)() if plain else None for l in self.gnn_model]
         pool_masks = plain and slopes[-1] is not None and (not (args.value_att_mask and value_mask) or args.merge_mode == 'mult')
         pool_link, layer_links = {}, {}
@@ -222,13 +223,13 @@ class MultilevelGNN(nn.Module):
                 and getattr(conv, "in_channels", 0) % 4 == 0)
 
     def forward(self, input_batch, x=None, gene_pca_match=None, raw_indice=None, age=None, require_grad=True,
-                _loss_args=None):
+                _loss_args=None, _fused=False):
         args = self.args
         loss_args = _loss_args
         with torch.enable_grad() if require_grad else torch.no_grad():
             if x is None:
                 age = input_batch.age
-            x = self.pool_genes(input_batch, x, gene_pca_match, raw_indice, value_mask=True)     # [B, C, 438, P]
+            x = self.pool_genes(input_batch, x, gene_pca_match, raw_indice, value_mask=True, fused=_fused)     # [B, C, 438, P]
             x = x.reshape(x.shape[0], x.shape[1], 146, self.pca_dim * 3)
             if args.reorder_pathway and self.reorder_idxs is not None:
                 x = x[:, :, self.reorder_idxs.to(x.device), :]
@@ -270,6 +271,21 @@ class MultilevelGNN(nn.Module):
             # wide first Linear (6913 / 84096 inputs): weight gradient through mlg_xty (cuBLAS picks a slow large-k kernel)
             x = Fn.tall_linear(x, mod, min_rows=1) if (isinstance(mod, nn.Linear) and mod.in_features >= 1024) else mod(x)
         return x, pca_feature
+
+    def predict(self, input_batch):
+        """Forward-only evaluation: ``(pred, pca_feature)`` as ``forward`` returns them, in eval semantics (no dropout) whatever
+        ``self.training`` and the grad mode, on the kernel route of the training forward -- the factored first layer, node-major
+        rows into the transform-first second layer, the fused pool and the fused head -- with no backward state: nothing is
+        recorded for autograd and no tensor outlives the call but the two outputs.  Configurations outside the fused chain (dense
+        / residual GNN, repeat_mask, hooked layers, unfused heads) run the same generic route as ``forward``.
+        ``model(batch)`` under ``torch.no_grad()`` keeps its own (generic) route."""
+        was = self.training
+        self.train(False)
+        try:
+            with torch.no_grad():
+                return self.forward(input_batch, require_grad=False, _fused=True)
+        finally:
+            self.train(was)
 
     def forward_with_loss(self, input_batch, target, weight=None):
         """(pred, pca_feature, bce): ``forward`` plus torch.nn.BCELoss(weight)(pred, target) (train.py:60,118) computed by

@@ -9,6 +9,7 @@ gradient (``lin_l.weight`` of every SAGEConv, ``info_mask``) are left out of the
 optimizer state.
 """
 import os
+from typing import NamedTuple, Optional
 
 import torch
 import torch.distributed as dist
@@ -298,7 +299,106 @@ class _PendingLoss:
         return float(self.slot[0])
 
 
-class Trainer:
+class StaticBatchFeed:
+    """Host -> device feeding of a captured CUDA graph's static input buffers (``self.static_batch``), shared by ``Trainer``
+    and ``Evaluator``: ``load_batch`` copies a (pinned) host batch in on the current stream; ``prefetch`` starts the copy of
+    the NEXT batch on a side stream into staging buffers while the current replay runs, and ``_take_staged`` moves it into
+    the static buffers (device-to-device) right before the next replay."""
+
+    # fields that are dataset constants when a batch carries a ``topology_key``: the key promises that the edge list,
+    # edge weights, node->graph vector and pooling layout are identical for every batch with that key (one gene network
+    # shared by all patients, dataloader/multiloader.py:687-698) -- exactly what MultilevelGNN.forward already assumes
+    # when it caches the CSR / pool layout under that key.  They are uploaded once, not per step.
+    STATIC_TOPOLOGY_FIELDS = ("edge_index", "edge_attr", "batch", "gene_pca_match", "raw_indice")
+
+    def _step_fields(self, host_batch):
+        key = getattr(self.static_batch, "topology_key", None)
+        same = key is not None and getattr(host_batch, "topology_key", None) == key
+        return [k for k, v in vars(self.static_batch).items()
+                if torch.is_tensor(v) and not (same and k in self.STATIC_TOPOLOGY_FIELDS)]
+
+    def h2d_bytes(self, host_batch):
+        """Bytes ``load_batch`` / ``prefetch`` copy host -> device for this batch."""
+        return sum(getattr(host_batch, k).numel() * getattr(host_batch, k).element_size()
+                   for k in self._step_fields(host_batch))
+
+    def _check_topology(self, host_batch):
+        """The CSR, pooling layout, degree tables and visiting orders are built in the warm-up steps and BAKED into the
+        captured graph: a batch with another edge list / match table would silently train on the stale topology.  A keyed
+        batch (data.collate / data.TopologyLoader) must carry the key the graph was captured with.  A batch WITHOUT a key
+        (the reference's loader: every batch re-sends its own copy of the topology, train.py:42) is accepted, uploaded in
+        full, and its topology fields are compared ON THE DEVICE with the captured ones; a mismatch raises when the host
+        next reads a loss (``loss_to_host(...).get()``) or calls ``check_topology_flag()``."""
+        key = getattr(self.static_batch, "topology_key", None)
+        other = getattr(host_batch, "topology_key", None)
+        if other is not None and other != key:
+            raise ValueError("Trainer: the topology is frozen at capture(); this batch has topology_key=%r, the captured "
+                             "graph %r -- re-capture for a new topology, or step eagerly" % (other, key))
+
+    def _verify_uploaded_topology(self, fields):
+        """After a full upload into the static buffers: flag |= any(static != captured) per topology field (device only)."""
+        ref = getattr(self, "_topo_ref", None)
+        if ref is None:
+            return
+        for k in fields:
+            if k in ref:
+                self._topo_bad.logical_or_((getattr(self.static_batch, k) != ref[k]).any())
+                self._topo_compared = True      # from now on the flag travels to the host with every loss
+
+    def check_topology_flag(self):
+        """Host-side check (one sync) that no keyless batch with a different topology was fed to the captured graph."""
+        if getattr(self, "_topo_bad", None) is not None and bool(self._topo_bad.item()):
+            raise RuntimeError("Trainer: a batch uploaded after capture() carried a different edge list / pooling layout than "
+                               "the captured graph was built for (topology is frozen at capture())")
+
+    def load_batch(self, host_batch):
+        """Copy a (pinned) host batch into the captured graph's static device buffers (async H2D).  Only per-step
+        fields are copied: the topology fields are frozen at capture()."""
+        self._check_topology(host_batch)
+        fields = self._step_fields(host_batch)
+        for k in fields:
+            self._fill(getattr(self.static_batch, k), getattr(host_batch, k))
+        self._verify_uploaded_topology(fields)
+
+    def prefetch(self, host_batch):
+        """Start the H2D copy of the NEXT batch on a side stream into staging buffers while the current step's
+        graph is still running; ``step_prefetched`` then moves it into the static buffers (device-to-device)
+        and replays.  This is the double buffering the reference's synchronous ``batch.to(device)``
+        (train.py:42) lacks."""
+        self._check_topology(host_batch)
+        if self._copy_stream is None or set(self._staging) != set(self._step_fields(host_batch)):
+            if self._copy_stream is not None:
+                torch.cuda.current_stream().synchronize()        # switching keyed <-> keyless batches: new staging set
+            self._copy_stream = torch.cuda.Stream()
+            self._staging = {k: torch.empty_like(getattr(self.static_batch, k)) for k in self._step_fields(host_batch)}
+            self._staged = torch.cuda.Event()
+            self._consumed = torch.cuda.Event()
+            self._consumed.record()
+        self._copy_stream.wait_event(self._consumed)        # staging may not be overwritten before it was consumed
+        with torch.cuda.stream(self._copy_stream):
+            if set(self._staging) != set(self._step_fields(host_batch)):
+                raise ValueError("prefetch: this batch's topology_key differs from the one the staging buffers were "
+                                 "sized for; use step(batch) for a batch with a different topology")
+            for k, v in self._staging.items():
+                self._fill(v, getattr(host_batch, k))
+            self._staged.record()
+
+    @staticmethod
+    def _fill(dst, src):
+        """The H2D copy of one field into its device buffer (static or staging)."""
+        dst.copy_(src, non_blocking=True)
+
+    def _take_staged(self):
+        """Move the batch ``prefetch`` staged into the static buffers (device-to-device, on the current stream)."""
+        cur = torch.cuda.current_stream()
+        cur.wait_event(self._staged)
+        # staging -> static buffers: one multi-tensor launch per dtype instead of one copy kernel per field
+        torch._foreach_copy_([getattr(self.static_batch, k) for k in self._staging], list(self._staging.values()))
+        self._consumed.record()
+        self._verify_uploaded_topology(self._staging)
+
+
+class Trainer(StaticBatchFeed):
     """One training step of train.py:38-68 on the B200 kernels; ``capture()`` turns the whole step (forward, loss,
     backward, optimizer update -- with several ranks the fused NVLink reduce-scatter / Adam / all-gather kernels) into ONE
     CUDA graph replayed per step (the NCCL path keeps its all-reduce between two graphs)."""
@@ -448,93 +548,10 @@ class Trainer:
             self.graph_update.replay()
         return self.static_loss
 
-    # fields that are dataset constants when a batch carries a ``topology_key``: the key promises that the edge list,
-    # edge weights, node->graph vector and pooling layout are identical for every batch with that key (one gene network
-    # shared by all patients, dataloader/multiloader.py:687-698) -- exactly what MultilevelGNN.forward already assumes
-    # when it caches the CSR / pool layout under that key.  They are uploaded once, not per step.
-    STATIC_TOPOLOGY_FIELDS = ("edge_index", "edge_attr", "batch", "gene_pca_match", "raw_indice")
-
-    def _step_fields(self, host_batch):
-        key = getattr(self.static_batch, "topology_key", None)
-        same = key is not None and getattr(host_batch, "topology_key", None) == key
-        return [k for k, v in vars(self.static_batch).items()
-                if torch.is_tensor(v) and not (same and k in self.STATIC_TOPOLOGY_FIELDS)]
-
-    def h2d_bytes(self, host_batch):
-        """Bytes ``load_batch`` / ``prefetch`` copy host -> device for this batch."""
-        return sum(getattr(host_batch, k).numel() * getattr(host_batch, k).element_size()
-                   for k in self._step_fields(host_batch))
-
-    def _check_topology(self, host_batch):
-        """The CSR, pooling layout, degree tables and visiting orders are built in the warm-up steps and BAKED into the
-        captured graph: a batch with another edge list / match table would silently train on the stale topology.  A keyed
-        batch (data.collate / data.TopologyLoader) must carry the key the graph was captured with.  A batch WITHOUT a key
-        (the reference's loader: every batch re-sends its own copy of the topology, train.py:42) is accepted, uploaded in
-        full, and its topology fields are compared ON THE DEVICE with the captured ones; a mismatch raises when the host
-        next reads a loss (``loss_to_host(...).get()``) or calls ``check_topology_flag()``."""
-        key = getattr(self.static_batch, "topology_key", None)
-        other = getattr(host_batch, "topology_key", None)
-        if other is not None and other != key:
-            raise ValueError("Trainer: the topology is frozen at capture(); this batch has topology_key=%r, the captured "
-                             "graph %r -- re-capture for a new topology, or step eagerly" % (other, key))
-
-    def _verify_uploaded_topology(self, fields):
-        """After a full upload into the static buffers: flag |= any(static != captured) per topology field (device only)."""
-        ref = getattr(self, "_topo_ref", None)
-        if ref is None:
-            return
-        for k in fields:
-            if k in ref:
-                self._topo_bad.logical_or_((getattr(self.static_batch, k) != ref[k]).any())
-                self._topo_compared = True      # from now on the flag travels to the host with every loss
-
-    def check_topology_flag(self):
-        """Host-side check (one sync) that no keyless batch with a different topology was fed to the captured graph."""
-        if getattr(self, "_topo_bad", None) is not None and bool(self._topo_bad.item()):
-            raise RuntimeError("Trainer: a batch uploaded after capture() carried a different edge list / pooling layout than "
-                               "the captured graph was built for (topology is frozen at capture())")
-
-    def load_batch(self, host_batch):
-        """Copy a (pinned) host batch into the captured graph's static device buffers (async H2D).  Only per-step
-        fields are copied: the topology fields are frozen at capture()."""
-        self._check_topology(host_batch)
-        fields = self._step_fields(host_batch)
-        for k in fields:
-            getattr(self.static_batch, k).copy_(getattr(host_batch, k), non_blocking=True)
-        self._verify_uploaded_topology(fields)
-
-    def prefetch(self, host_batch):
-        """Start the H2D copy of the NEXT batch on a side stream into staging buffers while the current step's
-        graph is still running; ``step_prefetched`` then moves it into the static buffers (device-to-device)
-        and replays.  This is the double buffering the reference's synchronous ``batch.to(device)``
-        (train.py:42) lacks."""
-        self._check_topology(host_batch)
-        if self._copy_stream is None or set(self._staging) != set(self._step_fields(host_batch)):
-            if self._copy_stream is not None:
-                torch.cuda.current_stream().synchronize()        # switching keyed <-> keyless batches: new staging set
-            self._copy_stream = torch.cuda.Stream()
-            self._staging = {k: torch.empty_like(getattr(self.static_batch, k)) for k in self._step_fields(host_batch)}
-            self._staged = torch.cuda.Event()
-            self._consumed = torch.cuda.Event()
-            self._consumed.record()
-        self._copy_stream.wait_event(self._consumed)        # staging may not be overwritten before it was consumed
-        with torch.cuda.stream(self._copy_stream):
-            if set(self._staging) != set(self._step_fields(host_batch)):
-                raise ValueError("prefetch: this batch's topology_key differs from the one the staging buffers were "
-                                 "sized for; use step(batch) for a batch with a different topology")
-            for k, v in self._staging.items():
-                v.copy_(getattr(host_batch, k), non_blocking=True)
-            self._staged.record()
-
     def step_prefetched(self):
         if self.peer is not None and self.opt.failed():
             raise RuntimeError("Trainer: the fused NVLink update timed out waiting for a peer rank")
-        cur = torch.cuda.current_stream()
-        cur.wait_event(self._staged)
-        # staging -> static buffers: one multi-tensor launch per dtype instead of one copy kernel per field
-        torch._foreach_copy_([getattr(self.static_batch, k) for k in self._staging], list(self._staging.values()))
-        self._consumed.record()
-        self._verify_uploaded_topology(self._staging)
+        self._take_staged()
         return self._replay()
 
     def loss_to_host(self, loss):
@@ -567,3 +584,181 @@ class Trainer:
                 self.load_batch(batch)
             return self._replay()
         return self._step_eager(batch)
+
+
+def reassemble(gathered, n_items):
+    """Rows gathered from every rank of an unshuffled plan (data.TopologyLoader(shuffle=False, drop_last=False).index_batches())
+    -- [world, steps, B, ...], slot (r, s, j) holding row j of rank r's batch s, padding included -- back in dataset order: slot
+    (r, s, j) is dataset row s*B*world + r*B + j, so the valid rows are the first ``n_items`` of the (s, r, j)-ordered slots."""
+    w, st, b = gathered.shape[:3]
+    return gathered.transpose(0, 1).reshape(st * w * b, *gathered.shape[3:])[:n_items]
+
+
+class EvalResult(NamedTuple):
+    """The metrics of one split and, when asked for, pred [n, 2] on the host in dataset order."""
+    auc: float
+    acc: float
+    bce: float
+    n: int
+    pred: Optional[torch.Tensor] = None
+
+
+class Evaluator(StaticBatchFeed):
+    """The reference's per-epoch ``eval()`` of a split (train.py:71-109, called on train / valid / test every epoch) on the B200:
+    ``capture()`` records ONE forward-only CUDA graph of ``MultilevelGNN.predict`` (eval mode, its own memory pool) over a
+    batch of ``batch_size`` graphs; ``evaluate(dataset, topo)`` replays it over an unshuffled plan that visits every sample
+    exactly once (data-parallel: each rank its own shard), gathers pred and y, and computes BCE, accuracy and ROC AUC in one
+    kernel (mlg_eval_metrics) -- one host synchronisation per split.
+
+    The graph reads the parameters in place, so it always evaluates the latest optimizer update; if a parameter's storage
+    moved since capture (e.g. a Trainer re-homed it into its flat buffer), ``evaluate`` re-captures first.
+    ``criterion_weight`` is the Trainer's: the BCE uses it, as its class row, only when ``args.weight_balance``."""
+
+    def __init__(self, model, args, batch_size=None, criterion_weight=None, world_size=1):
+        self.model, self.args, self.world = model, args, world_size
+        self.rank = dist.get_rank() if world_size > 1 else 0
+        self.batch_size = int(batch_size or args.batch_size)
+        self.class_w = None
+        if criterion_weight is not None and args.weight_balance:
+            w = torch.as_tensor(criterion_weight, dtype=torch.float32).reshape(-1, 2)
+            if not torch.equal(w, w[:1].expand_as(w)):
+                raise ValueError("Evaluator: a [B, 2] criterion weight must have equal rows (a class weight); per-position "
+                                 "weights have no meaning across a split")
+            self.class_w = w[0].contiguous()
+        self.graph = None
+        self.static_batch = None
+        self._copy_stream = None
+        self._example = None
+
+    def _param_ptrs(self):
+        return [p.data_ptr() for p in self.model.parameters()]
+
+    def capture(self, batch, warmup=2):
+        """Record the forward-only graph over ``batch`` (a device batch of ``batch_size`` graphs with a ``topology_key``, e.g.
+        data.to_device(data.collate(...))).  Its per-sample fields (x, y, age) are cloned into the static input buffers; the
+        topology fields are the batch's own (device-resident, shared).  The CSR / pool layouts are built in the warm-up."""
+        B = int(batch.age.shape[0])
+        if B != self.batch_size:
+            raise ValueError("Evaluator.capture: the batch holds %d graphs, batch_size is %d" % (B, self.batch_size))
+        if getattr(batch, "topology_key", None) is None:
+            raise ValueError("Evaluator.capture: needs a keyed batch (data.collate / data.to_device)")
+        from .synth import GraphBatch
+        from .data import PER_SAMPLE_FIELDS
+        self._example = batch
+        static = GraphBatch(**{k: v for k, v in vars(batch).items()})
+        for k in PER_SAMPLE_FIELDS:
+            if not torch.is_tensor(getattr(batch, k, None)):
+                raise ValueError("Evaluator.capture: the batch has no %r" % k)
+            setattr(static, k, getattr(batch, k).clone())
+        self.static_batch = static
+        self._copy_stream = None
+        dev = static.x.device
+        if self.class_w is not None:
+            self.class_w = self.class_w.to(dev)
+        # predict runs in eval mode and restores the model's mode afterwards
+        cur = torch.cuda.current_stream()
+        side = torch.cuda.Stream()
+        side.wait_stream(cur)
+        with torch.cuda.stream(side):
+            for _ in range(warmup):
+                self.model.predict(static)
+        cur.wait_stream(side)
+        torch.cuda.synchronize()
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            self.static_pred = self.model.predict(static)[0]
+        self._ptrs = self._param_ptrs()
+        return self
+
+    # the batches are built here from the dataset: only the per-sample fields travel, into the first B' sample slots
+    def _step_fields(self, host_batch):
+        from .data import PER_SAMPLE_FIELDS
+        return list(PER_SAMPLE_FIELDS)
+
+    def _check_topology(self, host_batch):
+        pass
+
+    @staticmethod
+    def _fill(dst, src):
+        dst[:src.shape[0]].copy_(src, non_blocking=True)
+
+    def evaluate(self, dataset, topo, with_pred=True):
+        """Forward-only pass over the whole split ``dataset`` (records with x / y / age, as data.collate takes them; ``topo``
+        the split's FoldTopology) -> EvalResult(auc, acc, bce, n, pred).  Data parallel: every rank calls it with the same
+        dataset and gets the same result.  A short tail batch fills the first B' slots of the static buffers (the graphs of
+        a batch do not interact in the forward, so the padding rows only produce predictions that are dropped); a rank whose
+        last batch is empty still replays, so all ranks step together."""
+        from .data import TopologyLoader, collate
+        if self.graph is None:
+            raise RuntimeError("Evaluator: call capture(batch) first")
+        want = "%s-b%d" % (topo.key, self.batch_size)
+        if self.static_batch.topology_key != want:
+            raise ValueError("Evaluator: captured for topology_key=%r, this split's topology is %r"
+                             % (self.static_batch.topology_key, want))
+        if self._param_ptrs() != self._ptrs:
+            self.capture(self._example)          # parameters were re-homed since capture: the graph reads stale storage
+        n = len(dataset)
+        if n == 0:
+            raise ValueError("Evaluator: empty split")
+        B = self.batch_size
+        plan = TopologyLoader(dataset, topo, B, shuffle=False, drop_last=False, rank=self.rank, world=self.world).index_batches()
+        steps = len(plan)
+        dev = self.static_pred.device
+        out = torch.empty(steps, 2, B, 2, dtype=torch.float32, device=dev)      # per step: [pred | y] of the B slots
+        y_static = self.static_batch.y.view(B, 2)
+
+        def host(s):
+            idx = plan[s]
+            return collate([dataset[int(i)] for i in idx], topo) if idx.numel() else None
+
+        nxt = host(0)
+        if nxt is not None:
+            self.prefetch(nxt)
+        for s in range(steps):
+            staged = nxt is not None
+            nxt = host(s + 1) if s + 1 < steps else None      # collated on the host while the device works
+            if staged:
+                self._take_staged()
+            self.graph.replay()
+            out[s, 0].copy_(self.static_pred)        # D2D, outside the graph
+            out[s, 1].copy_(y_static)
+            if nxt is not None:
+                self.prefetch(nxt)
+        if self.world > 1:
+            gathered = torch.empty(self.world * steps, 2, B, 2, dtype=torch.float32, device=dev)
+            dist.all_gather_into_tensor(gathered, out)
+            gathered = gathered.view(self.world, steps, 2, B, 2)
+        else:
+            gathered = out.view(1, steps, 2, B, 2)
+        rows = reassemble(gathered.permute(0, 1, 3, 2, 4), n)         # [n, 2 (pred | y), 2]
+        res = torch.empty(3 + (2 * n if with_pred else 0), dtype=torch.float32, device=dev)
+        pred = rows[:, 0].contiguous()
+        y = rows[:, 1].contiguous()
+        if with_pred:
+            res[3:].copy_(pred.view(-1))
+        eval_metrics(pred, y, self.class_w, out=res[:3])
+        host_res = res.cpu()                     # the one host synchronisation of the split
+        auc, acc, bce = float(host_res[2]), float(host_res[1]), float(host_res[0])
+        return EvalResult(auc, acc, bce, n, host_res[3:].view(n, 2).clone() if with_pred else None)
+
+
+def eval_metrics(pred, y, class_w=None, out=None):
+    """[bce, acc, auc] (float32 device tensor) of pred [n, 2] against y [n, 2] in one launch (mlg_eval_metrics): BCELoss(weight)
+    with the class row ``class_w`` [2], argmax accuracy, and the exact ROC AUC of pred[:, 1] (NaN with one class only)."""
+    from . import _cabi
+    L = _cabi.lib()
+    _cabi.require_cuda(pred, y, class_w)
+    pred = pred.detach().float().contiguous()
+    y = y.detach().float().reshape(-1, 2).contiguous()
+    n = pred.shape[0]
+    if pred.shape != (n, 2) or y.shape[0] != n:
+        raise ValueError("eval_metrics: pred and y must both be [n, 2]")
+    cw = None if class_w is None else class_w.detach().float().reshape(2).contiguous()
+    if out is None:
+        out = torch.empty(3, dtype=torch.float32, device=pred.device)
+    ws_bytes = int(L.mlg_eval_metrics_workspace_bytes(n))
+    ws = torch.empty(-(-ws_bytes // 8), dtype=torch.float64, device=pred.device)
+    with torch.cuda.device(pred.device), _cabi.span("eval_metrics", 16 * n):
+        _cabi.check(L.mlg_eval_metrics(_cabi.fptr(pred), _cabi.fptr(y), n, _cabi.fptr(cw, True), _cabi.fptr(out), _cabi.ptr(ws),
+                                       ws_bytes, _cabi.stream_ptr()), "mlg_eval_metrics")
+    return out
