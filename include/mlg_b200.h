@@ -393,6 +393,10 @@ int64_t mlg_head_mlp_workspace_bytes(int64_t R, int64_t D, int64_t K);
 int mlg_head_mlp_fwd(const float* a0, int64_t ld_a, const float* W0, const float* b0, const float* W3, const float* b3,
                      const int32_t* drop_bits, float drop_p, const float* y, const float* weight, int64_t R, int64_t D,
                      int64_t K, float* a1, float* pred, float* loss, void* workspace, int64_t workspace_bytes, void* stream);
+/* Input-gradient-only mode of both head backward calls: pass NULL for all four weight-gradient outputs (and, for
+ * mlg_head_conv_pool_bwd, a NULL workspace).  The kernels then skip the weight-gradient products: mlg_head_mlp_bwd reads
+ * W0 once for g_a0 and never stages the gW0 slice, mlg_head_conv_pool_bwd skips its per-block partials and their reduce.
+ * With non-NULL outputs both calls run exactly as before. */
 int mlg_head_mlp_bwd(const float* g_pred, const float* g_loss, const float* pred, const float* y, const float* weight,
                      const float* a0, int64_t ld_a, const float* a1, const float* W0, const float* W3, float drop_p,
                      int64_t R, int64_t D, int64_t K, float* g_a0, int64_t ld_g, float* g_W0, float* g_b0, float* g_W3,
@@ -456,6 +460,30 @@ int mlg_embed_scale_fwd(const float* xs, const float* emb, int64_t B, int64_t N,
                         void* stream);
 int mlg_embed_scale_bwd(const float* xs, const float* g_out, int64_t B, int64_t N, int64_t C,
                         float* g_emb, void* stream);
+/* Gradient w.r.t. the node values of the same prologue: g_xs[b*N+n] = <g_out[b*N+n, :], emb[n, :]>  (g_xs [B*N]). */
+int mlg_embed_scale_bwd_xs(const float* g_out, const float* emb, int64_t B, int64_t N, int64_t C, float* g_xs, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Gradient w.r.t. the node values xs [B*N] of the fully factored first SAGE layer (mlg_sage_rank1_fwd_rows):
+ *     g_xs[b,j] = <gz[b,j,:], E_self[j,:]> + sum_{(i,q): idx_q = j} (val_q / cnt_i) <gz[b,i,:], E_nbr[j,:]>
+ * gz [B*n_rows, C] (ld_g) is dL/dz or, with mask_bits (C == 64, the forward's sign bits) or y (the layer output, layout of
+ * gz) given, dL/dy; gz_node_major: its rows are (replica b, node i) at i * B + b.  rowptr / idx / val / order: the
+ * forward (by-target) CSR as for the forward call (cap entries); rowptr_t / fwd_pos_t: the by-source CSR whose entries
+ * are positions in the forward CSR (Topology.bwd.rowptr, Topology.bwd2fwd).  g_xs [B*n_rows] graph-major.  C == 32 or
+ * 64, 1 <= replicas <= 64.  Per-entry values ([cap, B]) and self terms ([n_rows, B]) go to the workspace; the segment sum
+ * runs in a fixed order: bit-identical results from run to run. */
+int64_t mlg_sage_rank1_bwd_xs_workspace_bytes(int64_t cap, int64_t n_rows, int64_t replicas);
+int mlg_sage_rank1_bwd_xs(const float* gz, int64_t ld_g, int gz_node_major, const float* y, const uint64_t* mask_bits,
+                          float slope, const float* e_self, int64_t ld_self, const float* e_nbr, int64_t ld_nbr,
+                          const int32_t* rowptr, const int32_t* idx, const float* val, const int32_t* order,
+                          const int32_t* rowptr_t, const int32_t* fwd_pos_t, int64_t n_rows, int64_t cap, int64_t C,
+                          int64_t replicas, float* g_xs, void* workspace, int64_t workspace_bytes, void* stream);
+
+/* acc[p, c] = (accumulate ? acc[p, c] : 0) + sum_{s = slot_ptr[p]}^{slot_ptr[p+1]-1} w[s] * g[s * ld_g + c],  c < N:
+ * per-slot gradients summed into per-output rows in slot order (integrated gradients' trapezoid sum, also across
+ * replays).  acc [n_out, N], slot_ptr int32 [n_out + 1]. */
+int mlg_attr_accumulate(const float* g, int64_t ld_g, const float* w, const int32_t* slot_ptr, int64_t n_out, int64_t N,
+                        int accumulate, float* acc, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Gene -> pathway pool (models/multilevel_gnn.py:205-239): value mask, gather by gene_pca_match,
@@ -504,6 +532,15 @@ int mlg_pool_bwd_layout(const float* g_out_cl, const float* x, const float* vm, 
                         const int32_t* node_slot, const int32_t* seg_of_slot, int64_t B, int64_t N, int64_t C, int64_t G,
                         int64_t S, int64_t P, int64_t replicas, float* g_x, float* g_w, float* workspace, int mask_input,
                         float mask_slope, const float* w_mask, int gx_node_major, void* stream);
+/* mlg_pool_bwd_layout that also returns the gradient w.r.t. the value mask vm (vm and g_vm [B*N] required):
+ *     g_vm[b,n] = sum_c x[b,n,c] * u[b,n,c],   u[b,n,c] = sum_{slots of n} sum_p w[g,p] * g_out[b,seg,p,c]
+ * (g_x = vm * u, times the activation derivative with mask_input), computed in the same pass as g_x -- never by dividing
+ * g_x by vm.  g_w and workspace may be NULL: then no weight gradient is formed (the input-gradient-only backward);
+ * g_x is always written, in the layout gx_node_major selects. */
+int mlg_pool_bwd_vm(const float* g_out_cl, const float* x, const float* vm, const float* w, const int32_t* node_rowptr,
+                    const int32_t* node_slot, const int32_t* seg_of_slot, int64_t B, int64_t N, int64_t C, int64_t G,
+                    int64_t S, int64_t P, int64_t replicas, float* g_x, float* g_w, float* workspace, int mask_input,
+                    float mask_slope, const float* w_mask, int gx_node_major, float* g_vm, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Dilated kNN graph (models/gcn_lib/sparse/torch_edge.py:53-104, dense/torch_edge.py:32-58):

@@ -12,5 +12,6 @@ from .gcn_lib.sparse import (GENConv, PathwayConv, GenMessagePassing, MsgNorm, G
 from .gcn_lib.dense import DenseDilatedKnnGraph, DenseDilated, dense_knn_matrix  # noqa: F401
 from .models import (MultilevelGNN, VAE, DeeperGCN, DiffPool, DiffPoolLayer, SAGEConvolutions, DenseSAGEConv,  # noqa: F401
                      dense_diff_pool, MODELS, get_model)
+from .attribution import Attributor, AttributionResult  # noqa: F401,E402
 
 __version__ = "0.1.0"

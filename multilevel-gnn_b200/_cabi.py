@@ -125,6 +125,13 @@ _SIGNATURES = {
     "mlg_bias_act": (_c_int, [_c_vp, _c_vp, _c_i64, _c_i64, _c_f32, _c_vp]),
     "mlg_embed_scale_fwd": (_c_int, [_c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_vp, _c_vp]),
     "mlg_embed_scale_bwd": (_c_int, [_c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_vp, _c_vp]),
+    "mlg_embed_scale_bwd_xs": (_c_int, [_c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_vp, _c_vp]),
+    "mlg_sage_rank1_bwd_xs_workspace_bytes": (_c_i64, [_c_i64, _c_i64, _c_i64]),
+    # (gz, ld_g, gz_nm, y, mask_bits, slope, e_self, ld_self, e_nbr, ld_nbr, rowptr, idx, val, order, rowptr_t, fwd_pos_t,
+    #  n_rows, cap, C, replicas, g_xs, workspace, workspace_bytes, stream)
+    "mlg_sage_rank1_bwd_xs": (_c_int, [_c_vp, _c_i64, _c_int, _c_vp, _c_vp, _c_f32, _c_vp, _c_i64, _c_vp, _c_i64, _c_vp, _c_vp,
+                                       _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_vp, _c_vp, _c_i64, _c_vp]),
+    "mlg_attr_accumulate": (_c_int, [_c_vp, _c_i64, _c_vp, _c_vp, _c_i64, _c_i64, _c_int, _c_vp, _c_vp]),
     "mlg_pool_fwd": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64,
                               _c_i64, _c_int, _c_vp, _c_vp]),
     "mlg_pool_bwd_x": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64,
@@ -136,6 +143,8 @@ _SIGNATURES = {
     "mlg_pool_bwd_node_major_supported": (_c_int, [_c_i64, _c_i64]),
     "mlg_pool_bwd_layout": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64,
                                      _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_int, _c_f32, _c_vp, _c_int, _c_vp]),
+    "mlg_pool_bwd_vm": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64,
+                                 _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_int, _c_f32, _c_vp, _c_int, _c_vp, _c_vp]),
     "mlg_gather_sum_nm": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_i64, _c_vp, _c_i64,
                                    _c_vp]),
     "mlg_cast_bf16": (_c_int, [_c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_int, _c_vp, _c_i64, _c_vp]),

@@ -297,6 +297,7 @@ __global__ void __launch_bounds__(kPix) head_conv_pool_bwd_kernel(const ConvPool
       for (int q = 0; q < CIN / 4; ++q) dst[q] = make_float4(gx[4 * q], gx[4 * q + 1], gx[4 * q + 2], gx[4 * q + 3]);
     }
   }
+  if (!P.partial) return;   // input gradient only
   __syncthreads();
   // parameter gradients of this block: gW2 = Gz2^T H1 (64 x 32), gW1 = Gz1^T X (32 x 32), column sums; fixed order over pixels
   float* part = P.partial + (size_t)blockIdx.x * kGradFloats;
@@ -648,7 +649,7 @@ __global__ void __launch_bounds__(512) head_mlp_bwd_kernel(const MlpBwdP P) {
       gz[r] = a1v[r] > 0.f ? (gz2[2 * r] * w30 + gz2[2 * r + 1] * w31) * P.keep_scale : 0.f;
       Gs[r * D + n] = gz[r];
     }
-    if (blockIdx.x == 0) {   // the small parameter gradients, fixed order over the samples
+    if (blockIdx.x == 0 && P.g_W0) {   // the small parameter gradients, fixed order over the samples
       float s = 0.f, u0 = 0.f, u1 = 0.f;
 #pragma unroll
       for (int r = 0; r < RT; ++r) {
@@ -698,6 +699,7 @@ __global__ void __launch_bounds__(512) head_mlp_bwd_kernel(const MlpBwdP P) {
         if (q < rpg && r0 + q < P.R) P.g_a0[(size_t)(r0 + q) * P.ld_g + k0 + k] = acc[q];
     }
   }
+  if (!P.g_W0) return;   // input gradient only
   __syncthreads();
   // ---- weight gradient slice: gW0[n][k0 + k] = sum_r dz1[r][n] a0[r][k0 + k]; staged in Ws, then written row by row ----
   if (unit) {
@@ -788,15 +790,18 @@ extern "C" int mlg_head_conv_pool_bwd(const float* g_a0, int64_t ld, const float
                                       const float* W2, const float* b2, const int32_t* drop_bits, float drop_p, int64_t B,
                                       int64_t H, int64_t W, int64_t kh, int64_t kw, float* g_x_cl, float* g_W1, float* g_b1,
                                       float* g_W2, float* g_b2, void* workspace, int64_t workspace_bytes, void* stream) {
-  MLG_CHECK_ARG(g_a0 && x_cl && W1 && b1 && W2 && b2 && g_x_cl && g_W1 && g_b1 && g_W2 && g_b2 && workspace,
+  // g_W1 = g_b1 = g_W2 = g_b2 = NULL: input gradient only (no workspace needed)
+  const bool wgrad = g_W1 || g_b1 || g_W2 || g_b2;
+  MLG_CHECK_ARG(g_a0 && x_cl && W1 && b1 && W2 && b2 && g_x_cl && (!wgrad || (g_W1 && g_b1 && g_W2 && g_b2 && workspace)),
                 "mlg_head_conv_pool_bwd: null pointer");
   MLG_CHECK_ARG(B >= 1 && H >= 1 && W >= 1 && kh >= 1 && kw >= 1 && kh <= H && kw <= W, "mlg_head_conv_pool_bwd: bad sizes");
   MLG_CHECK_ARG(drop_p == 0.f || drop_bits, "mlg_head_conv_pool_bwd: dropout needs drop_bits");
   ConvPoolP P;
   if (int rc = conv_pool_fill(P, x_cl, W1, b1, W2, b2, drop_bits, drop_p, B, H, W, kh, kw)) return rc;
-  MLG_CHECK_ARG(workspace_bytes >= mlg_head_conv_pool_bwd_workspace_bytes(B, H, W, kh, kw), "mlg_head_conv_pool_bwd: workspace too small");
+  MLG_CHECK_ARG(!wgrad || workspace_bytes >= mlg_head_conv_pool_bwd_workspace_bytes(B, H, W, kh, kw),
+                "mlg_head_conv_pool_bwd: workspace too small");
   MLG_CHECK_ARG((uintptr_t)g_x_cl % 16 == 0, "mlg_head_conv_pool_bwd: g_x_cl must be 16-byte aligned");
-  P.ld = ld; P.g_a0 = g_a0; P.g_x = g_x_cl; P.partial = (float*)workspace;
+  P.ld = ld; P.g_a0 = g_a0; P.g_x = g_x_cl; P.partial = wgrad ? (float*)workspace : nullptr;
   const int blocks = conv_pool_blocks(P);
   const size_t smem = conv_pool_smem(P, true);
   MLG_CHECK_ARG(smem <= 227 * 1024, "mlg_head_conv_pool_bwd: %lld windows per block do not fit shared memory", (long long)P.NB * P.Wo);
@@ -810,8 +815,10 @@ extern "C" int mlg_head_conv_pool_bwd(const float* g_a0, int64_t ld, const float
         reinterpret_cast<float4*>(g_x_cl), (int)B, P.H, P.W, P.Ho * P.kh);
     MLG_CHECK_LAUNCH("mlg_head_conv_pool_bwd(tail)");
   }
-  head_conv_reduce_kernel<<<mlg_ceil_div(kGradFloats, 128), 128, 0, st>>>(P.partial, blocks, g_W1, g_b1, g_W2, g_b2);
-  MLG_CHECK_LAUNCH("mlg_head_conv_pool_bwd(reduce)");
+  if (wgrad) {
+    head_conv_reduce_kernel<<<mlg_ceil_div(kGradFloats, 128), 128, 0, st>>>(P.partial, blocks, g_W1, g_b1, g_W2, g_b2);
+    MLG_CHECK_LAUNCH("mlg_head_conv_pool_bwd(reduce)");
+  }
   return MLG_OK;
 }
 
@@ -862,7 +869,10 @@ extern "C" int mlg_head_mlp_bwd(const float* g_pred, const float* g_loss, const 
                                 const float* weight, const float* a0, int64_t ld_a, const float* a1, const float* W0,
                                 const float* W3, float drop_p, int64_t R, int64_t D, int64_t K, float* g_a0, int64_t ld_g,
                                 float* g_W0, float* g_b0, float* g_W3, float* g_b3, void* stream) {
-  MLG_CHECK_ARG(pred && a0 && a1 && W0 && W3 && g_W0 && g_b0 && g_W3 && g_b3, "mlg_head_mlp_bwd: null pointer");
+  // g_W0 = g_b0 = g_W3 = g_b3 = NULL: input gradient only (one pass over W0 instead of two)
+  const bool wgrad = g_W0 || g_b0 || g_W3 || g_b3;
+  MLG_CHECK_ARG(pred && a0 && a1 && W0 && W3 && (!wgrad || (g_W0 && g_b0 && g_W3 && g_b3)), "mlg_head_mlp_bwd: null pointer");
+  MLG_CHECK_ARG(wgrad || g_a0, "mlg_head_mlp_bwd: no output requested");
   MLG_CHECK_ARG(g_pred || g_loss, "mlg_head_mlp_bwd: neither g_pred nor g_loss given");
   MLG_CHECK_ARG(!g_loss || y, "mlg_head_mlp_bwd: g_loss needs y");
   MLG_CHECK_ARG(R >= 1 && R <= 64 && D >= 32 && D % 32 == 0 && D <= 512 && K >= 1, "mlg_head_mlp_bwd: need rows <= 64, D a multiple of 32 up to 512");

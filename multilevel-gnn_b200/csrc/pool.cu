@@ -369,12 +369,13 @@ pool_bwd_w_kernel(const float* __restrict__ g_cl, const float* __restrict__ x, c
 //   part[b, g, p]          = sum_c vm * x[b*n + row, c] * g_cl[b, seg, p, c]          (g = slot's gene)
 // x is streamed in node order (coalesced) instead of being gathered per gene slot, and the g_cl rows are loaded
 // once for both gradients; g_w = sum_b part[b] is a second, fixed-order pass (deterministic, no atomics).
-template <int P_, int CCH>
+template <int P_, int CCH, bool WG = true>
 __global__ void __launch_bounds__(kThreads)
 pool_bwd_fused_kernel(const float* __restrict__ g_cl, const float* __restrict__ x, const float* __restrict__ vm,
                       const float* __restrict__ w, const int* __restrict__ rowptr, const int* __restrict__ slots,
                       const int* __restrict__ seg_of_slot, int n_rows, int replicas, int S, int C, int G,
-                      float* __restrict__ g_x, float* __restrict__ part, int mask_input, float mask_slope) {
+                      float* __restrict__ g_x, float* __restrict__ part, int mask_input, float mask_slope,
+                      float* __restrict__ g_vm) {
   constexpr int RB = 4;
   const int lane = threadIdx.x & 31;
   const long long wid = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
@@ -432,17 +433,34 @@ pool_bwd_fused_kernel(const float* __restrict__ g_cl, const float* __restrict__ 
 #pragma unroll
           for (int cc = 0; cc < CCH; ++cc) {
             accx[r][cc] = fmaf(gv[r][p][cc], wj[p], accx[r][cc]);
-            dot = fmaf(xr[r][cc], gv[r][p][cc], dot);
+            if constexpr (WG) dot = fmaf(xr[r][cc], gv[r][p][cc], dot);
           }
-          dot = warp_sum(dot);
-          const int b = b0 + r;
-          if (lane == 0 && b < replicas) {
-            // replicated layout: slot ids are per graph (part row = b); general layout: slot ids already span b*G + g
-            const size_t prow = (replicas > 1) ? (size_t)b * G + slotj : (size_t)slotj;
-            part[prow * P_ + p] = dot;
+          if constexpr (WG) {
+            dot = warp_sum(dot);
+            const int b = b0 + r;
+            if (lane == 0 && b < replicas) {
+              // replicated layout: slot ids are per graph (part row = b); general layout: slot ids already span b*G + g
+              const size_t prow = (replicas > 1) ? (size_t)b * G + slotj : (size_t)slotj;
+              part[prow * P_ + p] = dot;
+            }
           }
         }
       }
+    }
+  }
+  if (g_vm) {   // dL/dvm = sum_c x * (the unscaled gradient row); x re-read: xr holds it times vm
+#pragma unroll
+    for (int r = 0; r < RB; ++r) {
+      const int b = min(b0 + r, replicas - 1);
+      const size_t orow = (size_t)b * n_rows + row;
+      float d = 0.f;
+#pragma unroll
+      for (int cc = 0; cc < CCH; ++cc) {
+        const int c = cc * 32 + lane;
+        if (c < C && beg < end) d = fmaf(__ldg(x + orow * C + c), accx[r][cc], d);
+      }
+      d = warp_sum(d);
+      if (lane == 0 && b0 + r < replicas) g_vm[orow] = d;
     }
   }
 #pragma unroll
@@ -507,12 +525,13 @@ __device__ __forceinline__ void stvec(float* p, const float (&d)[VEC]) {
   *reinterpret_cast<T*>(p) = t;
 }
 
-template <int P_, int VEC, int RB2>
+template <int P_, int VEC, int RB2, bool WG = true>
 __global__ void __launch_bounds__(kThreads, (VEC == 1 && RB2 <= 4) ? 4 : 2)
 pool_bwd_fused2_kernel(const float* __restrict__ g_cl, const float* __restrict__ x, const float* __restrict__ vm,
                        const float* __restrict__ w, const int* __restrict__ rowptr, const int* __restrict__ slots,
                        const int* __restrict__ seg_of_slot, int n_rows, int replicas, int S, int G,
-                       float* __restrict__ g_x, float* __restrict__ part, int mask_input, float mask_slope) {
+                       float* __restrict__ g_x, float* __restrict__ part, int mask_input, float mask_slope,
+                       float* __restrict__ g_vm) {
   constexpr int C = 32 * VEC;
   constexpr int P2 = P_ <= 1 ? 1 : (P_ <= 2 ? 2 : (P_ <= 4 ? 4 : 8));
   constexpr int K = RB2 * P2;
@@ -536,6 +555,7 @@ pool_bwd_fused2_kernel(const float* __restrict__ g_cl, const float* __restrict__
 #pragma unroll
     for (int r = 0; r < RB2; ++r)
       if (r < nb) stvec<VEC>(gx0 + (size_t)r * rep_x, z);
+    if (g_vm && lane < nb) g_vm[(size_t)(b0 + lane) * n_rows + row] = 0.f;
     return;
   }
   float xr[RB2][VEC], accx[RB2][VEC], scale[RB2];
@@ -579,19 +599,31 @@ pool_bwd_fused2_kernel(const float* __restrict__ g_cl, const float* __restrict__
 #pragma unroll
             for (int k = 0; k < VEC; ++k) {
               accx[r][k] = fmaf(gv[r][p < P_ ? p : 0][k], wj[p < P_ ? p : 0], accx[r][k]);
-              dot = fmaf(xr[r][k], gv[r][p < P_ ? p : 0][k], dot);
+              if constexpr (WG) dot = fmaf(xr[r][k], gv[r][p < P_ ? p : 0][k], dot);
             }
           }
           d[r * P2 + p] = dot * scale[r];
         }
-      const float tot = reduce_packed<K>(d, lane);
-      const int vi = lane >> KSHIFT;
-      const int r = vi / P2, p = vi % P2;
-      if ((lane & ((1 << KSHIFT) - 1)) == 0 && p < P_ && r < nb) {
-        // replicated layout: slot ids are per graph (part row = b); general layout: slot ids already span b*G + g
-        const size_t prow = (replicas > 1) ? (size_t)(b0 + r) * G + slotj : (size_t)slotj;
-        part[prow * P_ + p] = tot;
+      if constexpr (WG) {
+        const float tot = reduce_packed<K>(d, lane);
+        const int vi = lane >> KSHIFT;
+        const int r = vi / P2, p = vi % P2;
+        if ((lane & ((1 << KSHIFT) - 1)) == 0 && p < P_ && r < nb) {
+          // replicated layout: slot ids are per graph (part row = b); general layout: slot ids already span b*G + g
+          const size_t prow = (replicas > 1) ? (size_t)(b0 + r) * G + slotj : (size_t)slotj;
+          part[prow * P_ + p] = tot;
+        }
       }
+    }
+  }
+  if (g_vm) {   // dL/dvm = sum_c x * (the unscaled gradient row)
+#pragma unroll
+    for (int r = 0; r < RB2; ++r) {
+      float dv = 0.f;
+#pragma unroll
+      for (int k = 0; k < VEC; ++k) dv = fmaf(xr[r][k], accx[r][k], dv);
+      dv = warp_sum(dv);
+      if (lane == 0 && r < nb) g_vm[(size_t)(b0 + r) * n_rows + row] = dv;
     }
   }
 #pragma unroll
@@ -627,12 +659,13 @@ __device__ __forceinline__ float reduce_packed8(float (&v)[K], int sl) {
   return v[0];   // total of value index (sl >> (3 - log2 K)), replicated over the lanes sharing that index
 }
 
-template <int P_, int RBS>
+template <int P_, int RBS, bool WG = true>
 __global__ void __launch_bounds__(kThreads, 4)
 pool_bwd_c32_kernel(const float* __restrict__ g_cl, const float* __restrict__ x, const float* __restrict__ vm,
                     const float* __restrict__ w, const int* __restrict__ rowptr, const int* __restrict__ slots,
                     const int* __restrict__ seg_of_slot, int n_rows, int replicas, int S, int G,
-                    float* __restrict__ g_x, float* __restrict__ part, int mask_input, float mask_slope, int gx_node_major) {
+                    float* __restrict__ g_x, float* __restrict__ part, int mask_input, float mask_slope, int gx_node_major,
+                    float* __restrict__ g_vm) {
   constexpr int C = 32;
   constexpr int P2 = P_ <= 1 ? 1 : (P_ <= 2 ? 2 : (P_ <= 4 ? 4 : 8));
   constexpr int KSHIFT = P2 == 1 ? 3 : (P2 == 2 ? 2 : (P2 == 4 ? 1 : 0));
@@ -660,6 +693,7 @@ pool_bwd_c32_kernel(const float* __restrict__ g_cl, const float* __restrict__ x,
 #pragma unroll
     for (int r = 0; r < RBS; ++r)
       if (r < nb) st4(gx0 + (size_t)r * gx_step, make_float4(0.f, 0.f, 0.f, 0.f));
+    if (g_vm && sl < nb && sl < RBS) g_vm[(size_t)(b0 + sl) * n_rows + row] = 0.f;
     return;
   }
   float4 xr[RBS];
@@ -707,18 +741,35 @@ pool_bwd_c32_kernel(const float* __restrict__ g_cl, const float* __restrict__ x,
           accx[r][1] = fmaf(t.y, wj[p], accx[r][1]);
           accx[r][2] = fmaf(t.z, wj[p], accx[r][2]);
           accx[r][3] = fmaf(t.w, wj[p], accx[r][3]);
-          float dot = xr[r].x * t.x;
-          dot = fmaf(xr[r].y, t.y, dot);
-          dot = fmaf(xr[r].z, t.z, dot);
-          dot = fmaf(xr[r].w, t.w, dot);
-          d[p] += r < nb ? dot * scale[r] : 0.f;
+          if constexpr (WG) {
+            float dot = xr[r].x * t.x;
+            dot = fmaf(xr[r].y, t.y, dot);
+            dot = fmaf(xr[r].z, t.z, dot);
+            dot = fmaf(xr[r].w, t.w, dot);
+            d[p] += r < nb ? dot * scale[r] : 0.f;
+          }
         }
-      float tot = reduce_packed8<P2>(d, sl);
-      tot += __shfl_xor_sync(0xffffffffu, tot, 8);
-      tot += __shfl_xor_sync(0xffffffffu, tot, 16);
-      const int p = sl >> KSHIFT;
-      if (sub == 0 && (sl & ((1 << KSHIFT) - 1)) == 0 && p < P_)
-        part[((size_t)chunk * G + slotj) * P_ + p] = tot;   // one partial per (replica chunk, slot): the reduce adds `chunks`
+      if constexpr (WG) {
+        float tot = reduce_packed8<P2>(d, sl);
+        tot += __shfl_xor_sync(0xffffffffu, tot, 8);
+        tot += __shfl_xor_sync(0xffffffffu, tot, 16);
+        const int p = sl >> KSHIFT;
+        if (sub == 0 && (sl & ((1 << KSHIFT) - 1)) == 0 && p < P_)
+          part[((size_t)chunk * G + slotj) * P_ + p] = tot;   // one partial per (replica chunk, slot): the reduce adds `chunks`
+      }
+    }
+  }
+  if (g_vm) {   // dL/dvm = sum_c x * (the unscaled gradient row), summed over the 8 lanes of the group
+#pragma unroll
+    for (int r = 0; r < RBS; ++r) {
+      float dv = xr[r].x * accx[r][0];
+      dv = fmaf(xr[r].y, accx[r][1], dv);
+      dv = fmaf(xr[r].z, accx[r][2], dv);
+      dv = fmaf(xr[r].w, accx[r][3], dv);
+      dv += __shfl_xor_sync(0xffffffffu, dv, 1);
+      dv += __shfl_xor_sync(0xffffffffu, dv, 2);
+      dv += __shfl_xor_sync(0xffffffffu, dv, 4);
+      if (sl == 0 && r < nb) g_vm[(size_t)(b0 + r) * n_rows + row] = dv;
     }
   }
 #pragma unroll
@@ -840,12 +891,11 @@ extern "C" int mlg_pool_bwd(const float* g_out_cl, const float* x, const float* 
                              workspace, mask_input, mask_slope, w_mask, 0, stream);
 }
 
-extern "C" int mlg_pool_bwd_layout(const float* g_out_cl, const float* x, const float* vm, const float* w,
-                                   const int32_t* node_rowptr, const int32_t* node_slot, const int32_t* seg_of_slot,
-                                   int64_t B, int64_t N, int64_t C, int64_t G, int64_t S, int64_t P, int64_t replicas,
-                                   float* g_x, float* g_w, float* workspace, int mask_input, float mask_slope,
-                                   const float* w_mask, int gx_node_major, void* stream) {
-  MLG_CHECK_ARG(g_out_cl && x && w && node_rowptr && node_slot && seg_of_slot && g_x && g_w && workspace,
+static int pool_bwd_impl(const float* g_out_cl, const float* x, const float* vm, const float* w, const int32_t* node_rowptr,
+                         const int32_t* node_slot, const int32_t* seg_of_slot, int64_t B, int64_t N, int64_t C, int64_t G,
+                         int64_t S, int64_t P, int64_t replicas, float* g_x, float* g_w, float* workspace, int mask_input,
+                         float mask_slope, const float* w_mask, int gx_node_major, float* g_vm, void* stream) {
+  MLG_CHECK_ARG(g_out_cl && x && w && node_rowptr && node_slot && seg_of_slot && g_x && (!g_w || workspace),
                 "mlg_pool_bwd: null pointer");
   MLG_CHECK_ARG(!gx_node_major || (mlg_pool_bwd_node_major_supported(C, replicas) && (uintptr_t)g_out_cl % 16 == 0 &&
                                    (uintptr_t)x % 16 == 0 && (uintptr_t)g_x % 16 == 0),
@@ -856,6 +906,8 @@ extern "C" int mlg_pool_bwd_layout(const float* g_out_cl, const float* x, const 
   MLG_CHECK_ARG(C <= 128, "mlg_pool_bwd: fused backward supports C <= 128 (use mlg_pool_bwd_x / _w)");
   cudaStream_t st = (cudaStream_t)stream;
   const long long n_rows = replicas > 1 ? N : B * N;
+  // g_w == NULL: no weight gradient -- the kernels skip the partial dot products, nothing is reduced
+  const bool wg = g_w != nullptr;
   static const bool v1_only = getenv("MLG_POOL_BWD_V1") != nullptr;
   if (!v1_only && replicas > 1 && (C == 32 || C == 64 || C == 128) && (uintptr_t)g_out_cl % 16 == 0 && (uintptr_t)x % 16 == 0 &&
       (uintptr_t)g_x % 16 == 0) {
@@ -870,47 +922,84 @@ extern "C" int mlg_pool_bwd_layout(const float* g_out_cl, const float* x, const 
       const long long chunks = (replicas + rw - 1) / rw;
       const long long warps3 = n_rows * chunks;
       const int grid3 = mlg_ceil_div(warps3, kThreads / 32);
-      MLG_CUDA(cudaMemsetAsync(workspace, 0, (size_t)chunks * G * P * sizeof(float), st));   // slots without a node stay zero
-      MLG_P_SWITCH(P, (pool_bwd_c32_kernel<P_, 2><<<grid3, kThreads, 0, st>>>(
-                          g_out_cl, x, vm, w, node_rowptr, node_slot, seg_of_slot, (int)n_rows, (int)replicas, (int)S,
-                          (int)G, g_x, workspace, mask_input, mask_slope, gx_node_major)));
+      if (wg) {
+        MLG_CUDA(cudaMemsetAsync(workspace, 0, (size_t)chunks * G * P * sizeof(float), st));   // slots without a node stay zero
+        MLG_P_SWITCH(P, (pool_bwd_c32_kernel<P_, 2><<<grid3, kThreads, 0, st>>>(
+                            g_out_cl, x, vm, w, node_rowptr, node_slot, seg_of_slot, (int)n_rows, (int)replicas, (int)S,
+                            (int)G, g_x, workspace, mask_input, mask_slope, gx_node_major, g_vm)));
+      } else {
+        MLG_P_SWITCH(P, (pool_bwd_c32_kernel<P_, 2, false><<<grid3, kThreads, 0, st>>>(
+                            g_out_cl, x, vm, w, node_rowptr, node_slot, seg_of_slot, (int)n_rows, (int)replicas, (int)S,
+                            (int)G, g_x, nullptr, mask_input, mask_slope, gx_node_major, g_vm)));
+      }
       MLG_CHECK_LAUNCH("mlg_pool_bwd(c32)");
-      pool_wgrad_reduce_kernel<<<mlg_ceil_div(G * P, 256), 256, 0, st>>>(workspace, (int)chunks, G * P, (int)P, w_mask, g_w);
-      MLG_CHECK_LAUNCH("mlg_pool_bwd(reduce)");
+      if (wg) {
+        pool_wgrad_reduce_kernel<<<mlg_ceil_div(G * P, 256), 256, 0, st>>>(workspace, (int)chunks, G * P, (int)P, w_mask, g_w);
+        MLG_CHECK_LAUNCH("mlg_pool_bwd(reduce)");
+      }
       return MLG_OK;
     }
-    MLG_CUDA(cudaMemsetAsync(workspace, 0, (size_t)B * G * P * sizeof(float), st));   // slots without a node stay zero
+    if (wg) MLG_CUDA(cudaMemsetAsync(workspace, 0, (size_t)B * G * P * sizeof(float), st));   // slots without a node stay zero
     // C = 64 / 128: replicas per warp chosen so that RB2 * pow2(P) <= 32 packed dot products
     const int rb2 = P <= 4 ? 8 : 4;
     const long long warps2 = n_rows * ((replicas + rb2 - 1) / rb2);
     const int grid2 = mlg_ceil_div(warps2, kThreads / 32);
-#define MLG_POOL_F2(VV, RR)                                                                                           \
-  MLG_P_SWITCH(P, (pool_bwd_fused2_kernel<P_, VV, RR><<<grid2, kThreads, 0, st>>>(                                     \
+#define MLG_POOL_F2(VV, RR, WW)                                                                                       \
+  MLG_P_SWITCH(P, (pool_bwd_fused2_kernel<P_, VV, RR, WW><<<grid2, kThreads, 0, st>>>(                                 \
                       g_out_cl, x, vm, w, node_rowptr, node_slot, seg_of_slot, (int)n_rows, (int)replicas, (int)S,     \
-                      (int)G, g_x, workspace, mask_input, mask_slope)))
-    if (C == 64) { MLG_POOL_F2(2, (P_ <= 4 ? 8 : 4)); }
-    else { MLG_POOL_F2(4, (P_ <= 4 ? 8 : 4)); }
+                      (int)G, g_x, workspace, mask_input, mask_slope, g_vm)))
+    if (C == 64 && wg) { MLG_POOL_F2(2, (P_ <= 4 ? 8 : 4), true); }
+    else if (C == 64) { MLG_POOL_F2(2, (P_ <= 4 ? 8 : 4), false); }
+    else if (wg) { MLG_POOL_F2(4, (P_ <= 4 ? 8 : 4), true); }
+    else { MLG_POOL_F2(4, (P_ <= 4 ? 8 : 4), false); }
 #undef MLG_POOL_F2
     MLG_CHECK_LAUNCH("mlg_pool_bwd(fused2)");
-    pool_wgrad_reduce_kernel<<<mlg_ceil_div(G * P, 256), 256, 0, st>>>(workspace, (int)B, G * P, (int)P, w_mask, g_w);
-    MLG_CHECK_LAUNCH("mlg_pool_bwd(reduce)");
+    if (wg) {
+      pool_wgrad_reduce_kernel<<<mlg_ceil_div(G * P, 256), 256, 0, st>>>(workspace, (int)B, G * P, (int)P, w_mask, g_w);
+      MLG_CHECK_LAUNCH("mlg_pool_bwd(reduce)");
+    }
     return MLG_OK;
   }
-  MLG_CUDA(cudaMemsetAsync(workspace, 0, (size_t)B * G * P * sizeof(float), st));   // slots without a node stay zero
+  if (wg) MLG_CUDA(cudaMemsetAsync(workspace, 0, (size_t)B * G * P * sizeof(float), st));   // slots without a node stay zero
   const long long warps = n_rows * ((replicas + 3) / 4);
   const int grid = mlg_ceil_div(warps, kThreads / 32);
   const int cch = C <= 32 ? 1 : (C <= 64 ? 2 : 4);
-#define MLG_POOL_FUSED(CC)                                                                                          \
-  MLG_P_SWITCH(P, (pool_bwd_fused_kernel<P_, CC><<<grid, kThreads, 0, st>>>(g_out_cl, x, vm, w, node_rowptr, node_slot, \
-                                                                            seg_of_slot, (int)n_rows, (int)replicas,   \
-                                                                            (int)S, (int)C, (int)G, g_x, workspace,   \
-                                                                            mask_input, mask_slope)))
-  if (cch == 1) { MLG_POOL_FUSED(1); }
-  else if (cch == 2) { MLG_POOL_FUSED(2); }
-  else { MLG_POOL_FUSED(4); }
+#define MLG_POOL_FUSED(CC, WW)                                                                                         \
+  MLG_P_SWITCH(P, (pool_bwd_fused_kernel<P_, CC, WW><<<grid, kThreads, 0, st>>>(g_out_cl, x, vm, w, node_rowptr, node_slot, \
+                                                                                seg_of_slot, (int)n_rows, (int)replicas,   \
+                                                                                (int)S, (int)C, (int)G, g_x, workspace,   \
+                                                                                mask_input, mask_slope, g_vm)))
+  if (cch == 1 && wg) { MLG_POOL_FUSED(1, true); }
+  else if (cch == 1) { MLG_POOL_FUSED(1, false); }
+  else if (cch == 2 && wg) { MLG_POOL_FUSED(2, true); }
+  else if (cch == 2) { MLG_POOL_FUSED(2, false); }
+  else if (wg) { MLG_POOL_FUSED(4, true); }
+  else { MLG_POOL_FUSED(4, false); }
 #undef MLG_POOL_FUSED
   MLG_CHECK_LAUNCH("mlg_pool_bwd(fused)");
-  pool_wgrad_reduce_kernel<<<mlg_ceil_div(G * P, 256), 256, 0, st>>>(workspace, (int)B, G * P, (int)P, w_mask, g_w);
-  MLG_CHECK_LAUNCH("mlg_pool_bwd(reduce)");
+  if (wg) {
+    pool_wgrad_reduce_kernel<<<mlg_ceil_div(G * P, 256), 256, 0, st>>>(workspace, (int)B, G * P, (int)P, w_mask, g_w);
+    MLG_CHECK_LAUNCH("mlg_pool_bwd(reduce)");
+  }
   return MLG_OK;
+}
+
+extern "C" int mlg_pool_bwd_layout(const float* g_out_cl, const float* x, const float* vm, const float* w,
+                                   const int32_t* node_rowptr, const int32_t* node_slot, const int32_t* seg_of_slot,
+                                   int64_t B, int64_t N, int64_t C, int64_t G, int64_t S, int64_t P, int64_t replicas,
+                                   float* g_x, float* g_w, float* workspace, int mask_input, float mask_slope,
+                                   const float* w_mask, int gx_node_major, void* stream) {
+  MLG_CHECK_ARG(g_w && workspace, "mlg_pool_bwd: null pointer");
+  return pool_bwd_impl(g_out_cl, x, vm, w, node_rowptr, node_slot, seg_of_slot, B, N, C, G, S, P, replicas, g_x, g_w, workspace,
+                       mask_input, mask_slope, w_mask, gx_node_major, nullptr, stream);
+}
+
+extern "C" int mlg_pool_bwd_vm(const float* g_out_cl, const float* x, const float* vm, const float* w,
+                               const int32_t* node_rowptr, const int32_t* node_slot, const int32_t* seg_of_slot,
+                               int64_t B, int64_t N, int64_t C, int64_t G, int64_t S, int64_t P, int64_t replicas,
+                               float* g_x, float* g_w, float* workspace, int mask_input, float mask_slope,
+                               const float* w_mask, int gx_node_major, float* g_vm, void* stream) {
+  MLG_CHECK_ARG(vm && g_vm, "mlg_pool_bwd_vm: vm and g_vm are required");
+  return pool_bwd_impl(g_out_cl, x, vm, w, node_rowptr, node_slot, seg_of_slot, B, N, C, G, S, P, replicas, g_x, g_w, workspace,
+                       mask_input, mask_slope, w_mask, gx_node_major, g_vm, stream);
 }

@@ -718,6 +718,9 @@ class SageLayer(torch.autograd.Function):
             ctx.xs_t = xs_t
             ctx.mbits = mbits
             ctx.h1_nm = h1_nm
+            # the input gradient w.r.t. xs reads the per-gene tables again (7.9 MB at the gbm shape): kept only when asked for
+            ctx.e12 = e12 if ctx.needs_input_grad[1] else None
+            ctx.xs_shape = xs.shape
             if h1_nm:
                 link["h1_nm"] = True          # y (and the gradient this layer gets back) is node-major
             ctx.save_for_backward(xd, y, wst, w_r, w_nn, xs_d)
@@ -771,12 +774,37 @@ class SageLayer(torch.autograd.Function):
         ctx.save_for_backward(xcat, y, wbuf, w_r, w_nn, xs_d if rank1 else None)
         ctx.topo, ctx.relative, ctx.slope, ctx.cin, ctx.has_bias = topo, bool(relative), float(slope), cin, nn_b is not None
         ctx.rank1 = rank1
+        ctx.emb_d = xd if (rank1 and ctx.needs_input_grad[1]) else None
+        ctx.xs_shape = xs.shape if rank1 else None
         ctx.emb_param = x if (rank1 and isinstance(x, torch.nn.Parameter)) else None
         ctx.in_slope = None if (in_slope is None or relative or rank1) else float(in_slope)
         if in_slope is not None and ctx.in_slope is None:
             raise ValueError("SageLayer: in_slope needs a plain (non-relative, materialised) input")
         ctx.out_premasked = bool(out_premasked)
         return y
+
+    @staticmethod
+    def _rank1_input_grad(ctx, gz, bits, y):
+        """dL/dxs of the factored layer (mlg_sage_rank1_bwd_xs): gz is dL/dz, or dL/dy with the LeakyReLU derivative taken
+        from the forward's sign bits ``bits`` or from the output ``y``; rows node-major when the layer wrote its output so."""
+        L = _cabi.lib()
+        topo = ctx.topo
+        n1, B = topo.n_single, topo.replicas
+        e12 = ctx.e12
+        cout = e12.shape[1] // 2
+        fw, bw = topo.fwd, topo.bwd
+        g_xs = torch.empty(B * n1, dtype=torch.float32, device=gz.device)
+        ws_bytes = L.mlg_sage_rank1_bwd_xs_workspace_bytes(fw.cap, n1, B)
+        ws = torch.empty(max(ws_bytes // 4, 1), dtype=torch.float32, device=gz.device)
+        nbytes = 4 * cout * gz.shape[0] + 8 * fw.col.numel() + 3 * ws_bytes + 4 * g_xs.numel()
+        with torch.cuda.device(gz.device), _cabi.span("sage_rank1_bwd_xs", nbytes):
+            _cabi.check(L.mlg_sage_rank1_bwd_xs(
+                _cabi.fptr(gz), cout, 1 if getattr(ctx, "h1_nm", False) else 0, _cabi.fptr(y, True), _cabi.lptr(bits, True),
+                float(ctx.slope), _vptr(e12), 2 * cout, _vptr(e12[:, cout:]), 2 * cout, _cabi.iptr(fw.rowptr),
+                _cabi.iptr(fw.col), _cabi.fptr(topo.fwd_val, True), _cabi.iptr(topo.fwd_order, True), _cabi.iptr(bw.rowptr),
+                _cabi.iptr(topo.bwd2fwd), n1, fw.cap, cout, B, _cabi.fptr(g_xs), _cabi.fptr(ws), ws_bytes,
+                _cabi.stream_ptr()), "mlg_sage_rank1_bwd_xs")
+        return g_xs.view(ctx.xs_shape)
 
     @staticmethod
     def _backward_factored(ctx, gy):
@@ -786,6 +814,16 @@ class SageLayer(torch.autograd.Function):
         gy = _f32c(gy)
         L = _cabi.lib()
         n1, B = topo.n_single, topo.replicas
+        needs = ctx.needs_input_grad
+        want_w = needs[0] or needs[2] or needs[3] or needs[4]
+        g_xs = None
+        if not want_w:
+            # input gradient only (attribution): none of the table / weight-gradient work below
+            if ctx.out_premasked:
+                g_xs = SageLayer._rank1_input_grad(ctx, gy, None, None)
+            else:
+                g_xs = SageLayer._rank1_input_grad(ctx, gy, ctx.mbits, None if ctx.mbits is not None else y)
+            return None, g_xs, None, None, None, None, None, None, None, None, None, None
         by_rows = FACTORED_RANK1 != "gather" and bool(L.mlg_sage_rank1_bwd_rows_supported(cout))
         y_mask = bits = None
         if ctx.out_premasked:
@@ -796,6 +834,8 @@ class SageLayer(torch.autograd.Function):
         else:
             gz = torch.ops.aten.leaky_relu_backward(gy, y, ctx.slope, True) if ctx.slope != 0.0 \
                 else torch.ops.aten.threshold_backward(gy, y, 0.0)
+        if needs[1]:
+            g_xs = SageLayer._rank1_input_grad(ctx, gz, bits, None)
         if by_rows:
             # by target row: gz read once -> per-entry rows h (+ the self / bias reductions), then a segment sum by source
             fw, bw = topo.fwd, topo.bwd
@@ -853,7 +893,7 @@ class SageLayer(torch.autograd.Function):
             fk.hold(g_wst, g_wnn, g_wr)
         slot = grad_slot(ctx.emb_param, (n1, cin)) if ctx.emb_param is not None else None
         g_emb = tall_matmul(g12, wst.t(), tag="sage_rank1_demb", w_split=ctx.wst_t_split, out=slot)     # g12 @ Wst
-        return g_emb, None, g_wr, g_wnn, g_b, None, None, None, None, None, None, None
+        return g_emb, g_xs, g_wr, g_wnn, g_b, None, None, None, None, None, None, None
 
     @staticmethod
     def _backward_transform_first(ctx, gy):
@@ -943,12 +983,13 @@ class SageLayer(torch.autograd.Function):
                 _cabi.check(_cabi.lib().mlg_sage_fold_bwd(_cabi.fptr(g_wcat), _cabi.fptr(w_nn), _cabi.fptr(w_r), cout, cin,
                                                           w_r.shape[0], _cabi.fptr(g_wnn), _cabi.fptr(g_wr),
                                                           _cabi.stream_ptr()), "mlg_sage_fold_bwd")
-        if needs[0]:
+        g_xs = None
+        if needs[0] or (ctx.rank1 and needs[1]):
             wcat_t = wbuf[0].view(cout, 2 * cin).t()
             gxcat = tall_matmul(gz, wcat_t, tag="sage_dgrad_gemm",
                                 w_split=(wbuf[3].view(2 * cin, cout), wbuf[4].view(2 * cin, cout)))   # [N, 2cin]
             bw = topo.bwd
-            if ctx.rank1 and not ctx.relative and topo.replicas > 1 and cin % 4 == 0:
+            if ctx.rank1 and not ctx.relative and topo.replicas > 1 and cin % 4 == 0 and not needs[1]:
                 # first layer: only g_emb[n,:] = sum_b xs[b,n] * g_x0[b,n,:] is needed, so the backward aggregation reduces
                 # over the replicas in its epilogue (per replica slice; slices added here) and g_x0 is never written
                 n1 = topo.n_single
@@ -968,15 +1009,20 @@ class SageLayer(torch.autograd.Function):
             if ctx.relative:
                 gx = gx - gxcat[:, cin:]
             if ctx.rank1:
-                # gradient of the rank-1 input w.r.t. node_embedding: g_emb[n,:] = sum_b xs[b,n] * g_x0[b,n,:]
                 L = _cabi.lib()
                 n1 = topo.n_single
-                g_emb = torch.empty(n1, cin, dtype=torch.float32, device=gx.device)
-                with torch.cuda.device(gx.device), _cabi.span("embed_scale_bwd", 4 * gx.numel()):
-                    _cabi.check(L.mlg_embed_scale_bwd(_cabi.fptr(xs_d), _cabi.fptr(gx), topo.replicas, n1, cin,
-                                                      _cabi.fptr(g_emb), _cabi.stream_ptr()), "mlg_embed_scale_bwd")
+                if needs[1]:
+                    # gradient w.r.t. the node values: g_xs[b,n] = <g_x0[b,n,:], emb[n,:]>
+                    g_xs = _embed_scale_input_grad(gx, ctx.emb_d, topo.replicas, n1, cin).view(ctx.xs_shape)
+                g_emb = None
+                if needs[0]:
+                    # gradient of the rank-1 input w.r.t. node_embedding: g_emb[n,:] = sum_b xs[b,n] * g_x0[b,n,:]
+                    g_emb = torch.empty(n1, cin, dtype=torch.float32, device=gx.device)
+                    with torch.cuda.device(gx.device), _cabi.span("embed_scale_bwd", 4 * gx.numel()):
+                        _cabi.check(L.mlg_embed_scale_bwd(_cabi.fptr(xs_d), _cabi.fptr(gx), topo.replicas, n1, cin,
+                                                          _cabi.fptr(g_emb), _cabi.stream_ptr()), "mlg_embed_scale_bwd")
                 gx = g_emb
-        return gx, None, g_wr, g_wnn, (g_b if ctx.has_bias else None), None, None, None, None, None, None, None
+        return gx, g_xs, g_wr, g_wnn, (g_b if ctx.has_bias else None), None, None, None, None, None, None, None
 
 
 class RankOne:
@@ -1013,21 +1059,35 @@ class EmbedScale(torch.autograd.Function):
         with torch.cuda.device(emb.device):
             _cabi.check(L.mlg_embed_scale_fwd(_cabi.fptr(xs_d), _cabi.fptr(emb_d), B, N, C, _cabi.fptr(out),
                                               _cabi.stream_ptr()), "mlg_embed_scale_fwd")
-        ctx.save_for_backward(xs_d)
+        ctx.save_for_backward(xs_d, emb_d if ctx.needs_input_grad[0] else None)
         ctx.dims = (B, N, C)
+        ctx.xs_shape = xs.shape
         return out
 
     @staticmethod
     def backward(ctx, g):
         L = _cabi.lib()
-        (xs_d,) = ctx.saved_tensors
+        xs_d, emb_d = ctx.saved_tensors
         B, N, C = ctx.dims
         g = _f32c(g)
-        g_emb = torch.empty(N, C, dtype=torch.float32, device=g.device)
-        with torch.cuda.device(g.device):
-            _cabi.check(L.mlg_embed_scale_bwd(_cabi.fptr(xs_d), _cabi.fptr(g), B, N, C, _cabi.fptr(g_emb),
-                                              _cabi.stream_ptr()), "mlg_embed_scale_bwd")
-        return None, g_emb
+        g_xs = g_emb = None
+        if ctx.needs_input_grad[0]:
+            g_xs = _embed_scale_input_grad(g, emb_d, B, N, C).view(ctx.xs_shape)
+        if ctx.needs_input_grad[1] or not ctx.needs_input_grad[0]:
+            g_emb = torch.empty(N, C, dtype=torch.float32, device=g.device)
+            with torch.cuda.device(g.device):
+                _cabi.check(L.mlg_embed_scale_bwd(_cabi.fptr(xs_d), _cabi.fptr(g), B, N, C, _cabi.fptr(g_emb),
+                                                  _cabi.stream_ptr()), "mlg_embed_scale_bwd")
+        return g_xs, g_emb
+
+
+def _embed_scale_input_grad(g_x0, emb, B, N, C):
+    """g_xs [B*N] = <g_x0[b*N+n, :], emb[n, :]>: the gradient w.r.t. the node values of x0 = xs * emb (mlg_embed_scale_bwd_xs)."""
+    g_xs = torch.empty(B * N, dtype=torch.float32, device=g_x0.device)
+    with torch.cuda.device(g_x0.device), _cabi.span("embed_scale_bwd_xs", 4 * (g_x0.numel() + N * C + B * N)):
+        _cabi.check(_cabi.lib().mlg_embed_scale_bwd_xs(_cabi.fptr(_f32c(g_x0)), _cabi.fptr(_f32c(emb)), B, N, C,
+                                                       _cabi.fptr(g_xs), _cabi.stream_ptr()), "mlg_embed_scale_bwd_xs")
+    return g_xs
 
 
 class LayerNormFn(torch.autograd.Function):
@@ -1137,9 +1197,11 @@ class PathwayPool(torch.autograd.Function):
     def forward(ctx, x, w, vm, layout, in_slope=None, w_mask=None, link=None):
         """``in_slope``: x is the output of a (Leaky)ReLU with that slope whose producer expects dL/dz (see SageLayer).
         ``w_mask`` [G, 1] or [G]: the projection weights are w * w_mask (learnable_pca_params * info_mask,
-        multilevel_gnn.py:222); the product and its backward are folded in (the gradient returned for ``w`` is dL/dw)."""
+        multilevel_gnn.py:222); the product and its backward are folded in (the gradient returned for ``w`` is dL/dw).
+        ``vm`` is differentiable: when it requires grad, the backward returns dL/dvm from the same pass as dL/dx."""
         L = _cabi.lib()
         _cabi.require_cuda(x, w)
+        vm = None if vm is None else vm.detach()
         ctx.w_param = w
         ctx.w_mask = None
         if w_mask is not None:
@@ -1170,6 +1232,8 @@ class PathwayPool(torch.autograd.Function):
         C, P = xd.shape[1], wd.shape[1]
         g_cl = g.float().permute(0, 2, 3, 1).contiguous()     # [B,S,P,C]; no copy when g is already channel-last
         gx = gw = None
+        if ctx.needs_input_grad[2]:
+            return PathwayPool._backward_with_vm(ctx, g_cl)
         if ctx.needs_input_grad[0] and ctx.needs_input_grad[1] and C <= 128 and not lay.wrap_negative:
             slot = grad_slot(ctx.w_param, wd.shape)
             gx, gw = torch.empty_like(xd), (slot if slot is not None else torch.empty_like(wd))
@@ -1211,6 +1275,49 @@ class PathwayPool(torch.autograd.Function):
         if getattr(ctx, "link", None) is not None:
             ctx.link["gz_written_node_major"] = False
         return gx, gw, None, None, None, None, None
+
+    @staticmethod
+    def _backward_with_vm(ctx, g_cl):
+        """Backward when the value mask vm (batch.x) needs a gradient: g_x and g_vm in one pass (mlg_pool_bwd_vm), the weight
+        gradient in the same pass when it is needed too (or by mlg_pool_bwd_w where the fused pass does not apply); the
+        node-major hand-shake with the producing layer works as on the training path."""
+        L = _cabi.lib()
+        xd, wd = ctx.saved_tensors
+        lay, vm = ctx.layout, ctx.vm
+        B, N, G, S = lay.B, lay.N, lay.G, lay.S
+        C, P = xd.shape[1], wd.shape[1]
+        if C > 128:
+            raise NotImplementedError("PathwayPool: the gradient w.r.t. the value mask needs C <= 128 (got %d)" % C)
+        fused_w = ctx.needs_input_grad[1] and not lay.wrap_negative
+        gx, g_vm = torch.empty_like(xd), torch.empty_like(vm)
+        gw = ws = None
+        if fused_w:
+            slot = grad_slot(ctx.w_param, wd.shape)
+            gw = slot if slot is not None else torch.empty_like(wd)
+            ws = torch.empty(B * G * P, dtype=torch.float32, device=xd.device)
+        node = lay.node_csr
+        link = getattr(ctx, "link", None)
+        node_major = bool(link is not None and link.get("gz_node_major") and ctx.in_slope is not None
+                          and L.mlg_pool_bwd_node_major_supported(C, lay.replicas))
+        with torch.cuda.device(xd.device), _cabi.span("pool_bwd_vm", 2 * (4 * C * B * N) + 4 * B * C * S * P + 8 * B * N):
+            _cabi.check(L.mlg_pool_bwd_vm(_cabi.fptr(g_cl), _cabi.fptr(xd), _cabi.fptr(vm), _cabi.fptr(wd),
+                                          _cabi.iptr(node.rowptr), _cabi.iptr(node.col), _cabi.iptr(lay.seg_of_slot),
+                                          B, N, C, G, S, P, lay.replicas, _cabi.fptr(gx), _cabi.fptr(gw, True),
+                                          _cabi.fptr(ws, True), 0 if ctx.in_slope is None else 1,
+                                          0.0 if ctx.in_slope is None else ctx.in_slope, _cabi.fptr(ctx.w_mask, True),
+                                          1 if node_major else 0, _cabi.fptr(g_vm), _cabi.stream_ptr()), "mlg_pool_bwd_vm")
+            if ctx.needs_input_grad[1] and not fused_w:
+                gw = torch.empty_like(wd)
+                with _cabi.span("pool_bwd_w", 4 * C * B * N + 4 * B * C * S * P):
+                    _cabi.check(L.mlg_pool_bwd_w(_cabi.fptr(g_cl), _cabi.fptr(xd), _cabi.fptr(vm),
+                                                 _cabi.lptr(lay.match), _cabi.lptr(lay.raw_indice), B, N, C, G, S, P,
+                                                 int(lay.wrap_negative), lay.replicas, _cabi.fptr(gw), _cabi.stream_ptr()),
+                                "mlg_pool_bwd_w")
+                if ctx.w_mask is not None:
+                    gw = gw * ctx.w_mask.reshape(-1, 1)
+        if link is not None:
+            link["gz_written_node_major"] = node_major      # read (and cleared) by the producer layer's backward
+        return (gx if ctx.needs_input_grad[0] else None), gw, g_vm, None, None, None, None
 
 
 def _drop_bits(n, device):
@@ -1275,14 +1382,19 @@ class HeadConvPool(torch.autograd.Function):
             slot = grad_slot(param, param.shape)
             return slot if slot is not None else torch.empty(param.shape, dtype=torch.float32, device=dev)
 
-        gW1, gb1, gW2, gb2 = dest(W1), dest(b1), dest(W2), dest(b2)
-        ws_bytes = L.mlg_head_conv_pool_bwd_workspace_bytes(B, H, W, kh, kw)
-        ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=dev)
+        if any(ctx.needs_input_grad[1:5]):
+            gW1, gb1, gW2, gb2 = dest(W1), dest(b1), dest(W2), dest(b2)
+            ws_bytes = L.mlg_head_conv_pool_bwd_workspace_bytes(B, H, W, kh, kw)
+            ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=dev)
+        else:      # input gradient only: the kernel skips the weight-gradient partials and their reduce
+            gW1 = gb1 = gW2 = gb2 = ws = None
+            ws_bytes = 0
         with torch.cuda.device(dev), _cabi.span("head_conv_pool_bwd", 4 * (2 * x_cl.numel() + g.numel())):
             _cabi.check(L.mlg_head_conv_pool_bwd(_cabi.fptr(g), ld, _cabi.fptr(x_cl), _cabi.fptr(w1), _cabi.fptr(b1d),
                                                  _cabi.fptr(w2), _cabi.fptr(b2d), _cabi.iptr(bits, True), p, B, H, W, kh, kw,
-                                                 _cabi.fptr(gx), _cabi.fptr(gW1), _cabi.fptr(gb1), _cabi.fptr(gW2),
-                                                 _cabi.fptr(gb2), _cabi.fptr(ws), ws_bytes, _cabi.stream_ptr()),
+                                                 _cabi.fptr(gx), _cabi.fptr(gW1, True), _cabi.fptr(gb1, True),
+                                                 _cabi.fptr(gW2, True), _cabi.fptr(gb2, True), _cabi.fptr(ws, True), ws_bytes,
+                                                 _cabi.stream_ptr()),
                         "mlg_head_conv_pool_bwd")
         g_age = g[:, ld - 1] if (ctx.needs_input_grad[5]) else None
         return gx.permute(0, 3, 1, 2), gW1, gb1, gW2, gb2, g_age, None, None, None, None
@@ -1350,13 +1462,17 @@ class HeadMLP(torch.autograd.Function):
             slot = grad_slot(param, param.shape)
             return slot if slot is not None else torch.empty(param.shape, dtype=torch.float32, device=dev)
 
-        gW0, gb0, gW3, gb3 = dest(W0), dest(b0), dest(W3), dest(b3)
+        if any(ctx.needs_input_grad[1:5]):
+            gW0, gb0, gW3, gb3 = dest(W0), dest(b0), dest(W3), dest(b3)
+        else:      # input gradient only: one pass over W0, no weight-gradient slices
+            gW0 = gb0 = gW3 = gb3 = None
         g_a0 = torch.empty(R, K, dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
         with torch.cuda.device(dev), _cabi.span("head_mlp_bwd", 4 * (2 * D * K + 2 * R * K)):
             _cabi.check(L.mlg_head_mlp_bwd(_cabi.fptr(gp, True), _cabi.fptr(gl, True), _cabi.fptr(pred), _cabi.fptr(yd, True),
                                            _cabi.fptr(wd, True), _vptr(a0d), a0d.stride(0), _cabi.fptr(a1), _cabi.fptr(w0),
-                                           _cabi.fptr(w3), ctx.p, R, D, K, _cabi.fptr(g_a0, True), K, _cabi.fptr(gW0),
-                                           _cabi.fptr(gb0), _cabi.fptr(gW3), _cabi.fptr(gb3), _cabi.stream_ptr()),
+                                           _cabi.fptr(w3), ctx.p, R, D, K, _cabi.fptr(g_a0, True), K, _cabi.fptr(gW0, True),
+                                           _cabi.fptr(gb0, True), _cabi.fptr(gW3, True), _cabi.fptr(gb3, True),
+                                           _cabi.stream_ptr()),
                         "mlg_head_mlp_bwd")
         if AFTER_HEAD_BACKWARD is not None:
             AFTER_HEAD_BACKWARD()

@@ -195,7 +195,8 @@ class MultilevelGNN(nn.Module):
         vm = None
         if args.value_att_mask and value_mask:
             if args.merge_mode == 'mult':
-                vm = mask_x.reshape(-1).detach().float().contiguous()   # folded into the pool kernel
+                # folded into the pool kernel; differentiable: the pool returns dL/dvm when batch.x requires grad
+                vm = mask_x.reshape(-1).float().contiguous()
             else:
                 x = args.add_coef1 * x + args.add_coef2 * mask_col
 
