@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define MLG_ABI_VERSION 1
+#define MLG_ABI_VERSION 2
 
 /* aggregation modes of GenMessagePassing.aggregate (models/gcn_lib/sparse/torch_message.py:44-85) */
 #define MLG_AGGR_SOFTMAX 0 /* softmax, softmax_sg (learn_t=0), softmax_sum (y_dev != NULL) */
@@ -191,47 +191,33 @@ int mlg_sage_rank1_bwd_rows_nm(const float* gz, int64_t ld_g, const float* y, co
  *     out[b*n_rows+i,:] = LeakyReLU_slope( xs[b*n_rows+i] * e_self[i,:]
  *                                          + (1/cnt_i) * sum_{q in row i} val[q] * xs[b*n_rows+idx[q]] * e_nbr[idx[q],:] + bias )
  * (cnt_i = row length incl. the added self loop: PyG mean aggregation; bias NULL ok; slope 0 = ReLU).
- * Neither x0, the [x0 | agg] buffer nor the (replicas*n_rows)-row update GEMM are ever formed.  replicas >= 2, C % 4 == 0,
- * 16-byte aligned tables / out with leading dimensions that are multiples of 4; CSR / order as in mlg_gather_sum. */
-int mlg_sage_rank1_fwd(const float* xs, const float* e_self, int64_t ld_self, const float* e_nbr, int64_t ld_nbr,
-                       const int32_t* rowptr, const int32_t* idx, const float* val, const int32_t* order, int64_t n_rows,
-                       int64_t C, int64_t replicas, const float* bias, float slope, float* out, int64_t ld_out,
-                       uint64_t* mask_bits, void* stream);
-/* mask_bits (NULL ok; C == 64 only): [n_rows][replicas] 64-bit words, bit 16*(c % 4) + c / 4 = (out[b,i,c] > 0): lets the
+ * Neither x0, the [x0 | agg] buffer nor the (replicas*n_rows)-row update GEMM are ever formed.
+ * mlg_sage_rank1_fwd_rows runs it with one WARP per gene for all replicas (C == 32 or 64): the neighbour's table row and its
+ * replica values are loaded once per CSR entry.  xs_t [n_rows, replicas]: the node values TRANSPOSED (mlg_transpose_bn of
+ * xs [replicas, n_rows]); the same matrix serves mlg_sage_rank1_bwd_rows (xs_transposed = 1).  CSR / order as in
+ * mlg_gather_sum; tables / out 8-byte aligned with even leading dimensions.
+ * mask_bits (NULL ok; C == 64 only): [n_rows][replicas] 64-bit words, bit 16*(c % 4) + c / 4 = (out[b,i,c] > 0): lets the
  * backward pass apply LeakyReLU' from 8 bytes per (row, replica) instead of re-reading the activation. */
-/* Its backward w.r.t. the tables and the bias from gz = dL/dz [replicas*n_rows, C], one pass over the by-source CSR
- * (rowptr_t / idx_t / val_t / order_t; inv_cnt[i] = 1/cnt_i of the forward rows, NULL = 1):
- *     g_e12_parts[s*n_rows+j, 0:C]  = sum_{b in slice s} xs[b,j] * gz[b,j,:]                                       -> g_E_self
- *     g_e12_parts[s*n_rows+j, C:2C] = sum_{b in slice s} xs[b,j] * sum_{i: j in row i} val_ij * inv_cnt[i] * gz[b,i,:] -> g_E_nbr
- *     g_bias_parts[s*n_rows+j, :]   = sum_{b in slice s} gz[b,j,:]
- * for s < mlg_gather_sum_slices(n_rows, C, replicas); the caller adds the slices (fixed order: deterministic). */
-int mlg_sage_rank1_bwd(const float* gz, int64_t ld_g, const float* xs, const int32_t* rowptr_t, const int32_t* idx_t,
-                       const float* val_t, const float* inv_cnt, const int32_t* order_t, int64_t n_rows, int64_t C,
-                       int64_t replicas, float* g_e12_parts, float* g_bias_parts, void* stream);
-
-/* The same gradients organised by TARGET row so that gz is read exactly once (C == 32 or 64; forward CSR rowptr / idx /
- * val / order): per entry q of row i (source j = idx[q])  h[q,:] = (val[q] / cnt_i) * sum_b xs[b,j] * gz[b,i,:], and per row
- * g_self[i,:] = sum_b xs[b,i] * gz[b,i,:] (-> g_E_self, leading dimension ld_self), g_bias_rows[i,:] = sum_b gz[b,i,:].
- * g_E_nbr[j,:] = sum_{q: idx[q] == j} h[q,:] is a segment sum the caller runs over the by-source CSR with mlg_gather_sum
- * (single graph, idx = by-source position -> forward position).  h must hold rowptr[n_rows] rows of C floats.
- * y != NULL: gz is dL/dy of the layer's LeakyReLU(slope) output y (same layout as gz) and the kernel multiplies by the
- * activation derivative while loading (no separate activation-backward pass); mask_bits != NULL (C == 64): the same
- * from the sign bits mlg_sage_rank1_fwd wrote (y is then not read).  xs_transposed != 0: xs is [n_rows, replicas]. */
-int mlg_sage_rank1_bwd_rows_supported(int64_t C);
-int mlg_sage_rank1_bwd_rows(const float* gz, int64_t ld_g, const float* y, const uint64_t* mask_bits, float slope, const float* xs, int xs_transposed, const int32_t* rowptr, const int32_t* idx,
-                            const float* val, const int32_t* order, int64_t n_rows, int64_t C, int64_t replicas, float* h,
-                            float* g_self, int64_t ld_self, float* g_bias_rows, void* stream);
-
-/* The forward pass with one WARP per gene for all replicas (C == 32 or 64): the neighbour's table row and its replica values
- * are loaded once per CSR entry.  xs_t [n_rows, replicas]: the node values TRANSPOSED (mlg_transpose_bn of xs [replicas,
- * n_rows]); the same matrix serves mlg_sage_rank1_bwd_rows (xs_transposed = 1).  Other arguments as mlg_sage_rank1_fwd;
- * tables / out 8-byte aligned with even leading dimensions. */
 int mlg_transpose_bn(const float* xs, int64_t B, int64_t n, float* xs_t, void* stream);
 int mlg_sage_rank1_fwd_rows_supported(int64_t C);
 int mlg_sage_rank1_fwd_rows(const float* xs_t, const float* e_self, int64_t ld_self, const float* e_nbr, int64_t ld_nbr,
                             const int32_t* rowptr, const int32_t* idx, const float* val, const int32_t* order, int64_t n_rows,
                             int64_t C, int64_t replicas, const float* bias, float slope, float* out, int64_t ld_out,
                             uint64_t* mask_bits, void* stream);
+
+/* Its backward w.r.t. the tables and the bias from gz = dL/dz [replicas*n_rows, C], organised by TARGET row so that gz is
+ * read exactly once (C == 32 or 64; forward CSR rowptr / idx / val / order): per entry q of row i (source j = idx[q])
+ * h[q,:] = (val[q] / cnt_i) * sum_b xs[b,j] * gz[b,i,:], and per row g_self[i,:] = sum_b xs[b,i] * gz[b,i,:] (-> g_E_self,
+ * leading dimension ld_self), g_bias_rows[i,:] = sum_b gz[b,i,:].
+ * g_E_nbr[j,:] = sum_{q: idx[q] == j} h[q,:] is a segment sum the caller runs over the by-source CSR with mlg_gather_sum
+ * (single graph, idx = by-source position -> forward position).  h must hold rowptr[n_rows] rows of C floats.
+ * y != NULL: gz is dL/dy of the layer's LeakyReLU(slope) output y (same layout as gz) and the kernel multiplies by the
+ * activation derivative while loading (no separate activation-backward pass); mask_bits != NULL (C == 64): the same
+ * from the sign bits mlg_sage_rank1_fwd_rows wrote (y is then not read).  xs_transposed != 0: xs is [n_rows, replicas]. */
+int mlg_sage_rank1_bwd_rows_supported(int64_t C);
+int mlg_sage_rank1_bwd_rows(const float* gz, int64_t ld_g, const float* y, const uint64_t* mask_bits, float slope, const float* xs, int xs_transposed, const int32_t* rowptr, const int32_t* idx,
+                            const float* val, const int32_t* order, int64_t n_rows, int64_t C, int64_t replicas, float* h,
+                            float* g_self, int64_t ld_self, float* g_bias_rows, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Tall-skinny transposed product: out[M,K] = A[rows,M]^T * X[rows,K], colsum[M] = sum_r A[r,:] (NULL ok).
@@ -608,17 +594,14 @@ int mlg_adam_step(float* params, const float* grads, float* exp_avg, float* exp_
  * gradient bucket, flat parameter buffer and a flag block (mlg_peer_flag_bytes(), zero-initialised) in device memory
  * from mlg_peer_alloc (cudaMalloc, zeroed) that the other ranks of the box map with mlg_peer_export / mlg_peer_open
  * (CUDA IPC, 64-byte handle).  peer_grads / peer_params / peer_flags are HOST arrays of `world` device pointers indexed
- * by rank (entry `rank` = this rank's own buffers).  [lo, hi): the CHUNK of the flat buffers this call updates (lo a multiple
- * of 4, hi - lo a multiple of 4*world; one flag block, one step counter and one optimizer-state shard PER CHUNK); rank r owns
- * the r-th 1/world of the chunk, and exp_avg / exp_avg_sq hold only that shard.  Chunks let the trainer update parameters
- * whose gradients are final early (the classifier head) on a forked branch while backward still runs.  Gradients are summed
- * in rank order and scaled by 1/world, so every rank ends with bitwise identical parameters.  step_dev as in mlg_adam_step.
+ * by rank (entry `rank` = this rank's own buffers).  n: the length of the flat buffers (a multiple of 4*world); rank r
+ * owns the r-th 1/world of them, and exp_avg / exp_avg_sq hold only that shard.  Gradients are summed in rank order and
+ * scaled by 1/world, so every rank ends with bitwise identical parameters.  step_dev as in mlg_adam_step.
  * The kernel synchronises the ranks itself (system-scope flags): every rank must issue the same sequence of calls.  A wait
  * longer than timeout_s (<= 0: 5 s) is a hard failure: the update is skipped (parameters and optimizer state untouched), the
  * status word of this rank AND of every peer is set (sticky: later calls return immediately; mlg_peer_status, 0 = ok) and,
  * when host_status != NULL (a pinned host int32, device-addressable), 1 is stored there so that the host can poll without a
- * device synchronisation.  max_blocks > 0 caps the grid (default 96 blocks of 512 threads) for a chunk that runs next to
- * other kernels.  Graph-capturable. */
+ * device synchronisation.  Graph-capturable. */
 int64_t mlg_peer_flag_bytes(void);
 void* mlg_peer_alloc(int64_t bytes);
 int mlg_peer_free(void* ptr);
@@ -626,15 +609,15 @@ int mlg_peer_export(void* ptr, void* handle64);
 void* mlg_peer_open(const void* handle64);
 int mlg_peer_close(void* ptr);
 int mlg_peer_adam_step(const float* const* peer_grads, float* const* peer_params, void* const* peer_flags, int world,
-                       int rank, int64_t lo, int64_t hi, float* exp_avg, float* exp_avg_sq, float* step_dev, float lr,
+                       int rank, int64_t n, float* exp_avg, float* exp_avg_sq, float* step_dev, float lr,
                        float beta1, float beta2, float eps, float weight_decay, double timeout_s, int32_t* host_status,
-                       int max_blocks, void* stream);
+                       void* stream);
 /* Test support (one GPU): `world` ranks whose arenas all live on this device, stepped by ONE cooperative launch (blocks that
  * wait on one another must be co-resident).  exp_avg / exp_avg_sq / step_dev: HOST arrays of one device pointer per rank;
  * ranks_dev: device scratch of mlg_peer_emulated_bytes(world) bytes.  Synchronises the stream once (argument upload). */
 int64_t mlg_peer_emulated_bytes(int world);
 int mlg_peer_adam_step_emulated(const float* const* peer_grads, float* const* peer_params, void* const* peer_flags, int world,
-                                int64_t lo, int64_t hi, float* const* exp_avg, float* const* exp_avg_sq, float* const* step_dev,
+                                int64_t n, float* const* exp_avg, float* const* exp_avg_sq, float* const* step_dev,
                                 float lr, float beta1, float beta2, float eps, float weight_decay, double timeout_s,
                                 void* ranks_dev, void* stream);
 int mlg_peer_status(const void* flags, int* status_out);

@@ -39,12 +39,6 @@ _SIGNATURES = {
                                     _c_i64, _c_i64, _c_int, _c_int, _c_vp, _c_i64, _c_vp, _c_i64, _c_vp, _c_i64, _c_vp, _c_i64,
                                     _c_f32, _c_vp, _c_int, _c_f32, _c_vp]),
     "mlg_gather_sum_slices": (_c_i64, [_c_i64, _c_i64, _c_i64]),
-    # (xs, e_self, ld_self, e_nbr, ld_nbr, rowptr, idx, val, order, n_rows, C, replicas, bias, slope, out, ld_out, mask_bits, stream)
-    "mlg_sage_rank1_fwd": (_c_int, [_c_vp, _c_vp, _c_i64, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64,
-                                    _c_vp, _c_f32, _c_vp, _c_i64, _c_vp, _c_vp]),
-    # (gz, ld_g, xs, rowptr_t, idx_t, val_t, inv_cnt, order_t, n_rows, C, replicas, g_e12_parts, g_bias_parts, stream)
-    "mlg_sage_rank1_bwd": (_c_int, [_c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_vp,
-                                    _c_vp, _c_vp]),
     "mlg_sage_rank1_bwd_rows_supported": (_c_int, [_c_i64]),
     # (gz, ld_g, y, mask_bits, slope, xs, rowptr, idx, val, order, n_rows, C, replicas, h, g_self, ld_self, g_bias_rows, stream)
     "mlg_sage_rank1_bwd_rows": (_c_int, [_c_vp, _c_i64, _c_vp, _c_vp, _c_f32, _c_vp, _c_int, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64,
@@ -163,10 +157,10 @@ _SIGNATURES = {
     "mlg_peer_export": (_c_int, [_c_vp, _c_vp]),
     "mlg_peer_open": (_c_vp, [_c_vp]),
     "mlg_peer_close": (_c_int, [_c_vp]),
-    "mlg_peer_adam_step": (_c_int, [_c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_f32, _c_f32,
-                                    _c_f32, _c_f32, _c_f32, ctypes.c_double, _c_vp, _c_int, _c_vp]),
+    "mlg_peer_adam_step": (_c_int, [_c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_i64, _c_vp, _c_vp, _c_vp, _c_f32, _c_f32,
+                                    _c_f32, _c_f32, _c_f32, ctypes.c_double, _c_vp, _c_vp]),
     "mlg_peer_emulated_bytes": (_c_i64, [_c_int]),
-    "mlg_peer_adam_step_emulated": (_c_int, [_c_vp, _c_vp, _c_vp, _c_int, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_f32, _c_f32,
+    "mlg_peer_adam_step_emulated": (_c_int, [_c_vp, _c_vp, _c_vp, _c_int, _c_i64, _c_vp, _c_vp, _c_vp, _c_f32, _c_f32,
                                              _c_f32, _c_f32, _c_f32, ctypes.c_double, _c_vp, _c_vp]),
     "mlg_peer_status": (_c_int, [_c_vp, _c_vp]),
     "mlg_adam_step": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_f32, _c_f32, _c_f32, _c_f32, _c_f32, _c_vp]),
@@ -198,7 +192,7 @@ def lib():
         for name, (res, args) in _SIGNATURES.items():
             fn = getattr(handle, name)
             fn.restype, fn.argtypes = res, args
-        if handle.mlg_abi_version() != 1:
+        if handle.mlg_abi_version() != 2:
             raise NativeLibraryError("libmlg_b200.so ABI version mismatch")
         _lib = handle
     return _lib

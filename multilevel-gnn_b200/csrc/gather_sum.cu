@@ -16,9 +16,8 @@
 // Also here, because they share the row / lane-group / replica-slice geometry and the helpers:
 //   * the fast replicated epilogue's extras -- the row's own src rows copied alongside (self_out: left half of cat(x, agg)),
 //     addend, activation-derivative mask, fused output activation (mlg_gather_sum_act: transform-first SAGE layer);
-//   * the fully factored first SAGE layer of MultilevelGNN: sage_rank1_fwd_kernel (mlg_sage_rank1_fwd),
-//     sage_rank1_bwd_rows_kernel (mlg_sage_rank1_bwd_rows, by target row) and the by-source gather variant
-//     (gather_sum_rep_kernel<.., RED, AUX>, mlg_sage_rank1_bwd) for widths the by-row kernel does not cover.
+//   * the backward of the fully factored first SAGE layer of MultilevelGNN: sage_rank1_bwd_rows_kernel
+//     (mlg_sage_rank1_bwd_rows, by target row; its forward is in sage_rank1.cu).
 #include <cstdlib>
 
 #include "common.cuh"
@@ -71,15 +70,8 @@ struct GsP {
   int replicas;
   unsigned rep_rows_src;   // 0: every replica reads the SAME src rows (rank-1 source, pre is per replica)
   unsigned rep_rows_pre;   // rows per replica of `pre` (0: shared)
-  // fully factored rank-1 SAGE layer (mlg_sage_rank1_fwd / _bwd below)
-  const float* e_self;     // fwd: out = act(pre[b,row] * e_self[row] + post * sum + bias)
-  const float* bias;
   float act_slope;
-  unsigned long long* mbits;   // sage_rank1_fwd_kernel<16> (C == 64): sign bits of the output, [n][replicas] x 64 bits
   int act;                 // fast replicated epilogue: out = LeakyReLU_act_slope(out) after addend / mask
-  float* aux1;             // bwd (RED): aux1[slice*n + row] = sum_b red_scale[b,row] * addend[b,row]   (NOT added to out)
-  float* auxb;             //            auxb[slice*n + row] = sum_b addend[b,row]
-  unsigned ld_aux1, ld_auxb;
 };
 
 __device__ __forceinline__ const float* rowp(const float* b, unsigned r, unsigned ld) { return b + (size_t)r * ld; }
@@ -263,7 +255,7 @@ __global__ void __launch_bounds__(kThreads) gather_sum_kernel(const GsP P) {
 // RANK1: every replica reads the SAME src rows and differs only by the per-(replica,row) scalar `pre`
 //        (MultilevelGNN layer 0: x0[b,n,:] = x[b,n] * node_embedding[n,:] is never materialised).
 // ---------------------------------------------------------------------------------------------
-template <int LANES, int VEC, bool RANK1, bool RED = false, bool AUX = false>
+template <int LANES, int VEC, bool RANK1, bool RED = false>
 __global__ void __launch_bounds__(kThreads, MLG_GS_MINB) gather_sum_rep_kernel(const GsP P, int gy) {
   constexpr int RPW = 32 / LANES;
   constexpr int CW = LANES * VEC;
@@ -303,11 +295,9 @@ __global__ void __launch_bounds__(kThreads, MLG_GS_MINB) gather_sum_rep_kernel(c
     const bool cok = c < (unsigned)C;
     const float* sc = P.src + (cok ? c : 0u);   // lanes past C read (and discard) the row start: no predicated loads
     const size_t rep_stride = (size_t)P.rep_rows_src * P.ld_src;
-    float red[VEC], red1[AUX ? VEC : 1], redb[AUX ? VEC : 1];
+    float red[VEC];
 #pragma unroll
     for (int k = 0; k < VEC; ++k) red[k] = 0.f;
-#pragma unroll
-    for (int k = 0; k < (AUX ? VEC : 1); ++k) red1[k] = redb[k] = 0.f;
     for (int b0 = b_lo; b0 < b_hi; b0 += RB) {
       const int nb = min(RB, b_hi - b0);
       float acc[RB][VEC];
@@ -392,27 +382,7 @@ __global__ void __launch_bounds__(kThreads, MLG_GS_MINB) gather_sum_rep_kernel(c
           for (int r = 0; r < RB; ++r)
             if (b0 + r < b_hi) stv<VEC>(rowp(P.self_out, (unsigned)(b0 + r) * (unsigned)P.n + row, P.ld_self) + c, t[r], cok);
         }
-        if (AUX) {
-          // factored first layer: the row's own gradient rows feed two SEPARATE replica reductions (weighted -> aux1,
-          // plain -> auxb) instead of being added to the gathered sum
-          float w[RB];
-#pragma unroll
-          for (int r = 0; r < RB; ++r) {
-            const unsigned brow = (unsigned)min(b0 + r, b_hi - 1) * (unsigned)P.n + row;
-            ldv<VEC>(t[r], rowp(P.addend, brow, P.ld_add) + c, cok);
-            w[r] = __ldg(P.red_scale + brow);
-          }
-#pragma unroll
-          for (int r = 0; r < RB; ++r) {
-            const bool live = b0 + r < b_hi;
-#pragma unroll
-            for (int k = 0; k < (AUX ? VEC : 1); ++k) {
-              red1[k] = fmaf(live ? w[r] : 0.f, t[r][k], red1[k]);
-              redb[k] += live ? t[r][k] : 0.f;
-              red[k] = fmaf(live ? w[r] * postf : 0.f, acc[r][k], red[k]);
-            }
-          }
-        } else if (P.addend) {
+        if (P.addend) {
 #pragma unroll
           for (int r = 0; r < RB; ++r)
             ldv<VEC>(t[r], rowp(P.addend, (unsigned)min(b0 + r, b_hi - 1) * (unsigned)P.n + row, P.ld_add) + c, cok);
@@ -441,9 +411,7 @@ __global__ void __launch_bounds__(kThreads, MLG_GS_MINB) gather_sum_rep_kernel(c
 #pragma unroll
             for (int k = 0; k < VEC; ++k) acc[r][k] = acc[r][k] > 0.f ? acc[r][k] : acc[r][k] * P.act_slope;
         }
-        if (AUX) {
-          // reductions done above
-        } else if (RED) {   // weighted reduction over the replicas instead of one output row per replica
+        if (RED) {   // weighted reduction over the replicas instead of one output row per replica
 #pragma unroll
           for (int r = 0; r < RB; ++r) {
             const float w = (b0 + r < b_hi) ? __ldg(P.red_scale + (size_t)(b0 + r) * P.n + row) : 0.f;
@@ -489,137 +457,12 @@ __global__ void __launch_bounds__(kThreads, MLG_GS_MINB) gather_sum_rep_kernel(c
       }
     }
     if (RED) stv<VEC>(rowp(P.out, (unsigned)ychunk * (unsigned)P.n + row, P.ld_out) + c, red, cok);
-    if (AUX) {
-      float a1[VEC], ab[VEC];
-#pragma unroll
-      for (int k = 0; k < VEC; ++k) {
-        a1[k] = red1[AUX ? k : 0];
-        ab[k] = redb[AUX ? k : 0];
-      }
-      stv<VEC>(rowp(P.aux1, (unsigned)ychunk * (unsigned)P.n + row, P.ld_aux1) + c, a1, cok);
-      stv<VEC>(rowp(P.auxb, (unsigned)ychunk * (unsigned)P.n + row, P.ld_auxb) + c, ab, cok);
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Fully factored first SAGE layer, forward (mlg_sage_rank1_fwd):
-//     out[b,i,:] = act( x[b,i] E_self[i,:] + (1/cnt_i) sum_q val_q x[b,idx_q] E_nbr[idx_q,:] + bias )
-// Same row / lane-group / replica-slice geometry as gather_sum_rep_kernel<.., RANK1>, but that kernel (2 entries and 4
-// replicas per step under an 80-register budget) measured latency bound here: 8 dependent load round trips per row and
-// slice, 110 us for a 126 MB output.  This one keeps F_JU = 4 entries x F_RB = 8 replicas in flight (table rows + the
-// per-replica scalars of all four entries are requested before the first FMA), 2 blocks/SM.
-// ---------------------------------------------------------------------------------------------
-constexpr int F_RB = 8, F_JU = 4;
-
-template <int LANES>
-__global__ void __launch_bounds__(kThreads, 2) sage_rank1_fwd_kernel(const GsP P, int gy) {
-  constexpr int VEC = 4;
-  constexpr int RPW = 32 / LANES;
-  constexpr int CW = LANES * VEC;
-  const int lane = threadIdx.x & 31;
-  const int sub = lane / LANES, sl = lane % LANES;
-  const unsigned gmask = (LANES == 32) ? 0xffffffffu : (((1u << LANES) - 1u) << (sub * LANES));
-  const int ychunk = blockIdx.x % gy;
-  const long long rowblock = blockIdx.x / gy;
-  const long long warp = (rowblock * (long long)blockDim.x + threadIdx.x) >> 5;
-  const int rep_per_y = (P.replicas + gy - 1) / gy;
-  const int b_lo = ychunk * rep_per_y, b_hi = min(P.replicas, b_lo + rep_per_y);
-  const long long slot = warp * RPW + sub;
-  if (slot >= P.n || b_lo >= b_hi) return;
-  const unsigned row = P.order ? (unsigned)__ldg(P.order + slot) : (unsigned)slot;
-  const int beg = __ldg(P.rowptr + row), end = __ldg(P.rowptr + row + 1);
-  const int cnt_row = end - beg;
-  const float postf = cnt_row > 0 ? 1.f / (float)cnt_row : 0.f;
-  unsigned idx0 = 0;
-  float w0 = 0.f;
-  if (cnt_row > 0) {
-    const int q = min(beg + sl, end - 1);
-    idx0 = (unsigned)__ldg(P.idx + q);
-    w0 = P.val ? __ldg(P.val + q) : 1.f;
-  }
-  const int nchunks = (P.C + CW - 1) / CW;
-  for (int ch = 0; ch < nchunks; ++ch) {
-    const unsigned c = ch * CW + sl * VEC;
-    const bool cok = c < (unsigned)P.C;
-    const float* sc = P.src + (cok ? c : 0u);
-    for (int b0 = b_lo; b0 < b_hi; b0 += F_RB) {
-      float acc[F_RB][VEC];
-#pragma unroll
-      for (int r = 0; r < F_RB; ++r)
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) acc[r][k] = 0.f;
-      const float* pre0 = P.pre + (size_t)b0 * P.rep_rows_pre;
-      const int nb = min(F_RB, b_hi - b0);
-      for (int base = beg; base < end; base += LANES) {
-        unsigned my_idx = idx0;
-        float my_w = w0;
-        if (base != beg) {
-          const int q = min(base + sl, end - 1);
-          my_idx = (unsigned)__ldg(P.idx + q);
-          my_w = P.val ? __ldg(P.val + q) : 1.f;
-        }
-        const int cnt = min(LANES, end - base);
-        for (int j = 0; j < cnt; j += F_JU) {
-          unsigned s[F_JU];
-          float w[F_JU], xv[F_JU][VEC], pw[F_JU][F_RB];
-#pragma unroll
-          for (int u = 0; u < F_JU; ++u) {
-            const int jj = min(j + u, cnt - 1);
-            s[u] = __shfl_sync(gmask, my_idx, jj, LANES);
-            w[u] = __shfl_sync(gmask, my_w, jj, LANES);
-            if (j + u >= cnt) w[u] = 0.f;
-            ldv<VEC>(xv[u], rowp(sc, s[u], P.ld_src), true);
-#pragma unroll
-            for (int r = 0; r < F_RB; ++r)
-              pw[u][r] = __ldg(pre0 + (size_t)min(r, nb - 1) * P.rep_rows_pre + s[u]);
-          }
-#pragma unroll
-          for (int u = 0; u < F_JU; ++u)
-#pragma unroll
-            for (int r = 0; r < F_RB; ++r) {
-              const float f = w[u] * pw[u][r];
-#pragma unroll
-              for (int k = 0; k < VEC; ++k) acc[r][k] = fmaf(f, xv[u][k], acc[r][k]);
-            }
-        }
-      }
-      // epilogue operands requested together (one exposed latency): self table row, bias, the row's own scalars
-      float es[VEC], bs[VEC], xself[F_RB];
-      ldv<VEC>(es, rowp(P.e_self, row, P.ld_self) + c, cok);
-#pragma unroll
-      for (int k = 0; k < VEC; ++k) bs[k] = (cok && P.bias) ? __ldg(P.bias + c + k) : 0.f;   // parameter view: 4-byte aligned only
-#pragma unroll
-      for (int r = 0; r < F_RB; ++r) xself[r] = __ldg(pre0 + (size_t)min(r, nb - 1) * P.rep_rows_pre + row);
-#pragma unroll
-      for (int r = 0; r < F_RB; ++r) {
-        if (r < nb) {
-          float y[VEC];
-#pragma unroll
-          for (int k = 0; k < VEC; ++k) {
-            const float z = fmaf(es[k], xself[r], fmaf(acc[r][k], postf, bs[k]));
-            y[k] = z > 0.f ? z : z * P.act_slope;
-          }
-          stv<VEC>(rowp(P.out, (unsigned)(b0 + r) * (unsigned)P.n + row, P.ld_out) + c, y, cok);
-          if (LANES == 16 && P.mbits) {
-            // sign bits of this (replica, row): 64 channels -> bit 16*(c % 4) + c / 4; the backward pass reads 8 bytes
-            // per (row, replica) instead of the 256-byte activation row to apply LeakyReLU'
-            unsigned f[VEC];
-#pragma unroll
-            for (int k = 0; k < VEC; ++k) f[k] = (__ballot_sync(gmask, y[k] > 0.f) >> (sub * LANES)) & 0xffffu;
-            if (sl == 0)
-              P.mbits[(size_t)row * P.replicas + (b0 + r)] =
-                  (unsigned long long)(f[0] | (f[1] << 16)) | ((unsigned long long)(f[2] | (f[3] << 16)) << 32);
-          }
-        }
-      }
-    }
   }
 }
 
 // ---------------------------------------------------------------------------------------------
 // Fully factored first SAGE layer, backward w.r.t. the tables (mlg_sage_rank1_bwd_rows), organised by TARGET row so
-// that gz is read exactly once (the by-source gather of mlg_sage_rank1_bwd re-reads every gz row once per edge):
+// that gz is read exactly once:
 // one warp per row i; lane l owns channels l, l+32, ... and keeps gz[b,i,channel] of 32 replicas in registers
 // (coalesced 128-byte loads, all in flight together); then for every entry q of the row (source j)
 //     h[q,:] = (val_q / cnt_i) * sum_b x[b,j] gz[b,i,:]
@@ -630,7 +473,7 @@ __global__ void __launch_bounds__(kThreads, 2) sage_rank1_fwd_kernel(const GsP P
 // ---------------------------------------------------------------------------------------------
 struct R1B {
   const float* gz;
-  const unsigned long long* mbits;   // optional (C == 64): sign bits of y written by sage_rank1_fwd_kernel, [n][B]
+  const unsigned long long* mbits;   // optional (C == 64): sign bits of y written by sage_rank1_fwd_rows_kernel, [n][B]
   const float* y;      // optional: gz is dL/dy of this layer's LeakyReLU output y; the kernel applies the derivative
   float slope;
   const float* xs;
@@ -1071,7 +914,7 @@ extern "C" int mlg_gather_sum_act(const float* src, int64_t ld_src, const int32_
   P.ld_src = (unsigned)ld_src; P.ld_out = (unsigned)ld_out; P.ld_add = (unsigned)ld_add; P.ld_self = (unsigned)ld_self;
   P.n = (int)n_rows; P.C = (int)C; P.post_mode = post_mode; P.relative = relative;
   P.replicas = (int)replicas; P.rep_rows_src = (unsigned)rep_rows_src; P.rep_rows_pre = (unsigned)rep_rows_pre;
-  P.e_self = nullptr; P.bias = nullptr; P.act_slope = act_slope; P.act = act; P.aux1 = nullptr; P.auxb = nullptr; P.ld_aux1 = P.ld_auxb = 0;
+  P.act_slope = act_slope; P.act = act;
   MLG_CHECK_ARG(!act || (replicas > 1 && rep_rows_src > 0 && !relative && !reduce_scale),
                 "mlg_gather_sum_act: the fused activation needs the replicated path (replicas > 1, per-replica src), no "
                 "relative / reduce_scale");
@@ -1108,85 +951,6 @@ extern "C" int mlg_gather_sum_act(const float* src, int64_t ld_src, const int32_
     else gather_sum_kernel<32, 4><<<(unsigned)gx, kThreads, 0, st>>>(P);
   }
   MLG_CHECK_LAUNCH("mlg_gather_sum");
-  return MLG_OK;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Fully factored first SAGE layer of MultilevelGNN (multilevel_gnn.py:150-151 + torch_vertex.py:269-294).  The layer
-// input x0[b,n,:] = x[b,n] * node_embedding[n,:] is rank-1 per node, so BOTH halves of the update
-//     z = [x0 | mean_j(w_ij x0_j)] * [W1 | W2 W_r]^T + bias
-// factor through two small per-gene tables  E_self = emb W1^T,  E_nbr = emb (W2 W_r)^T  ([N, Cout], a 15 405-row GEMM):
-//     z[b,i,:] = x[b,i] E_self[i,:] + (1/cnt_i) sum_q val_q x[b,idx_q] E_nbr[idx_q,:] + bias.
-// Neither x0, the [x0 | agg] buffer (252 MB at the gbm shape) nor the 492 960-row update GEMM exist any more; the kernel
-// reads the two tables (L2-resident) and x, and writes the activation once.
-// ---------------------------------------------------------------------------------------------
-extern "C" int mlg_sage_rank1_fwd(const float* xs, const float* e_self, int64_t ld_self, const float* e_nbr,
-                                  int64_t ld_nbr, const int32_t* rowptr, const int32_t* idx, const float* val,
-                                  const int32_t* order, int64_t n_rows, int64_t C, int64_t replicas, const float* bias,
-                                  float slope, float* out, int64_t ld_out, uint64_t* mask_bits, void* stream) {
-  MLG_CHECK_ARG(xs && e_self && e_nbr && rowptr && idx && out, "mlg_sage_rank1_fwd: null pointer");
-  MLG_CHECK_ARG(n_rows >= 0 && replicas >= 2 && replicas * n_rows < (1ll << 31) && C > 0 && C % 4 == 0 && C < (1ll << 20),
-                "mlg_sage_rank1_fwd: bad sizes (needs replicas >= 2, C %% 4 == 0)");
-  MLG_CHECK_ARG(ld_self >= C && ld_nbr >= C && ld_out >= C && ld_self % 4 == 0 && ld_nbr % 4 == 0 && ld_out % 4 == 0,
-                "mlg_sage_rank1_fwd: leading dimensions must be >= C and multiples of 4");
-  MLG_CHECK_ARG(((uintptr_t)e_self | (uintptr_t)e_nbr | (uintptr_t)out) % 16 == 0,
-                "mlg_sage_rank1_fwd: 16-byte alignment");
-  if (n_rows == 0) return MLG_OK;
-  GsP P;
-  memset(&P, 0, sizeof(P));
-  P.src = e_nbr; P.ld_src = (unsigned)ld_nbr; P.rowptr = rowptr; P.idx = idx; P.val = val; P.pre = xs; P.order = order;
-  P.out = out; P.ld_out = (unsigned)ld_out; P.e_self = e_self; P.ld_self = (unsigned)ld_self; P.bias = bias;
-  P.act_slope = slope; P.n = (int)n_rows; P.C = (int)C; P.post_mode = 1; P.replicas = (int)replicas;
-  P.rep_rows_src = 0; P.rep_rows_pre = (unsigned)n_rows;
-  MLG_CHECK_ARG(!mask_bits || C == 64, "mlg_sage_rank1_fwd: mask_bits needs C == 64");
-  P.mbits = reinterpret_cast<unsigned long long*>(mask_bits);
-  int lanes, rpb;
-  rep_geometry(C, true, &lanes, &rpb);
-  const long long gx = mlg_ceil_div(n_rows, rpb);
-  const int gy = rep_slices(gx, replicas);
-  const unsigned grid = (unsigned)(gx * gy);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (lanes == 8) sage_rank1_fwd_kernel<8><<<grid, kThreads, 0, st>>>(P, gy);
-  else if (lanes == 16) sage_rank1_fwd_kernel<16><<<grid, kThreads, 0, st>>>(P, gy);
-  else sage_rank1_fwd_kernel<32><<<grid, kThreads, 0, st>>>(P, gy);
-  MLG_CHECK_LAUNCH("mlg_sage_rank1_fwd");
-  return MLG_OK;
-}
-
-// Backward of the above w.r.t. the two tables and the bias, from gz = dL/dz [replicas*n_rows, C] (one pass, by-source CSR):
-//   g_e12_parts[s*n + j, 0:C]  = sum_{b in slice s} x[b,j] gz[b,j,:]                                  (-> g_E_self)
-//   g_e12_parts[s*n + j, C:2C] = sum_{b in slice s} x[b,j] sum_{i: j in row i} val_ij/cnt_i gz[b,i,:]  (-> g_E_nbr)
-//   g_bias_parts[s*n + j, :]   = sum_{b in slice s} gz[b,j,:]
-// The caller adds the mlg_gather_sum_slices(n_rows, C, replicas) slices (fixed order: deterministic).
-extern "C" int mlg_sage_rank1_bwd(const float* gz, int64_t ld_g, const float* xs, const int32_t* rowptr_t,
-                                  const int32_t* idx_t, const float* val_t, const float* inv_cnt, const int32_t* order_t,
-                                  int64_t n_rows, int64_t C, int64_t replicas, float* g_e12_parts, float* g_bias_parts,
-                                  void* stream) {
-  MLG_CHECK_ARG(gz && xs && rowptr_t && idx_t && g_e12_parts && g_bias_parts, "mlg_sage_rank1_bwd: null pointer");
-  MLG_CHECK_ARG(n_rows >= 0 && replicas >= 2 && replicas * n_rows < (1ll << 31) && C > 0 && C % 4 == 0 && C < (1ll << 20),
-                "mlg_sage_rank1_bwd: bad sizes (needs replicas >= 2, C %% 4 == 0)");
-  MLG_CHECK_ARG(ld_g >= C && ld_g % 4 == 0, "mlg_sage_rank1_bwd: ld_g must be >= C and a multiple of 4");
-  MLG_CHECK_ARG(((uintptr_t)gz | (uintptr_t)g_e12_parts | (uintptr_t)g_bias_parts) % 16 == 0,
-                "mlg_sage_rank1_bwd: 16-byte alignment");
-  if (n_rows == 0) return MLG_OK;
-  GsP P;
-  memset(&P, 0, sizeof(P));
-  P.src = gz; P.ld_src = (unsigned)ld_g; P.rowptr = rowptr_t; P.idx = idx_t; P.val = val_t; P.pre = inv_cnt;
-  P.order = order_t; P.addend = gz; P.ld_add = (unsigned)ld_g; P.red_scale = xs;
-  P.out = g_e12_parts + C; P.ld_out = (unsigned)(2 * C); P.aux1 = g_e12_parts; P.ld_aux1 = (unsigned)(2 * C);
-  P.auxb = g_bias_parts; P.ld_auxb = (unsigned)C;
-  P.n = (int)n_rows; P.C = (int)C; P.post_mode = 0; P.replicas = (int)replicas;
-  P.rep_rows_src = (unsigned)n_rows; P.rep_rows_pre = 0;
-  int lanes, rpb;
-  rep_geometry(C, true, &lanes, &rpb);
-  const long long gx = mlg_ceil_div(n_rows, rpb);
-  const int gy = rep_slices(gx, replicas);
-  const unsigned grid = (unsigned)(gx * gy);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (lanes == 8) gather_sum_rep_kernel<8, 4, false, true, true><<<grid, kThreads, 0, st>>>(P, gy);
-  else if (lanes == 16) gather_sum_rep_kernel<16, 4, false, true, true><<<grid, kThreads, 0, st>>>(P, gy);
-  else gather_sum_rep_kernel<32, 4, false, true, true><<<grid, kThreads, 0, st>>>(P, gy);
-  MLG_CHECK_LAUNCH("mlg_sage_rank1_bwd");
   return MLG_OK;
 }
 

@@ -13,11 +13,7 @@
 // with fixed pointers the whole training step (forward, loss, backward, this kernel) is ONE CUDA graph per rank.
 // Per-GPU traffic: (world-1)/world * 4n bytes read and the same written over NVLink + 16 B/parameter of local state.
 //
-// The bucket may be updated in CHUNKS (mlg_peer_adam_step's [lo, hi) range + a flag block per chunk): the trainer launches the
-// chunk holding the classifier head -- 62 % of the gbm parameters, final right after the head's backward kernel -- on a forked
-// graph branch while the rest of backward still runs, so only the last chunk's exchange sits on the critical path.
-//
-// Flag block (uint32, one per rank and chunk, peer-writable):  [0..7] ready[src]   [8..15] done[src]   [16] epoch   [17] block
+// Flag block (uint32, one per rank, peer-writable):  [0..7] ready[src]   [8..15] done[src]   [16] epoch   [17] block
 // counter   [18] status.  A wait that exceeds the timeout is a HARD failure: the rank sets its own status word, the status
 // word of EVERY peer and the host-visible status word (pinned memory), skips the update (parameters and optimizer state stay
 // untouched, so the replicas do not silently diverge) and every later launch returns immediately; the host (Trainer.step)
@@ -39,7 +35,7 @@ struct PeerP {
   unsigned* flags[kMaxWorld];
   float* m;          // exp_avg of the owned shard      [hi - lo]
   float* v;          // exp_avg_sq of the owned shard   [hi - lo]
-  float* step_dev;   // Adam step counter of this chunk (float, as mlg_adam_step)
+  float* step_dev;   // Adam step counter (float, as mlg_adam_step)
   int* host_status;  // pinned host word (or NULL)
   long long lo, hi;  // owned shard, multiples of 4
   int world, rank;
@@ -182,12 +178,11 @@ __global__ void __launch_bounds__(kThreads) peer_adam_emulated_kernel(const Peer
 }
 
 int fill_peer(PeerP& P, const float* const* peer_grads, float* const* peer_params, void* const* peer_flags, int world, int rank,
-              int64_t lo, int64_t hi, float* exp_avg, float* exp_avg_sq, float* step_dev, float lr, float beta1, float beta2,
+              int64_t n, float* exp_avg, float* exp_avg_sq, float* step_dev, float lr, float beta1, float beta2,
               float eps, float weight_decay, double timeout_s, int* host_status) {
   MLG_CHECK_ARG(peer_grads && peer_params && peer_flags && exp_avg && exp_avg_sq && step_dev, "mlg_peer_adam_step: null pointer");
   MLG_CHECK_ARG(world >= 1 && world <= kMaxWorld && rank >= 0 && rank < world, "mlg_peer_adam_step: world must be 1..8");
-  MLG_CHECK_ARG(lo >= 0 && hi >= lo && lo % 4 == 0 && (hi - lo) % (4 * world) == 0,
-                "mlg_peer_adam_step: chunk [lo, hi) must start at a multiple of 4 and hold a multiple of 4*world elements");
+  MLG_CHECK_ARG(n >= 0 && n % (4 * world) == 0, "mlg_peer_adam_step: the bucket must hold a multiple of 4*world elements");
   memset(&P, 0, sizeof(P));
   for (int r = 0; r < world; ++r) {
     MLG_CHECK_ARG(peer_grads[r] && peer_params[r] && peer_flags[r], "mlg_peer_adam_step: null peer pointer");
@@ -197,9 +192,9 @@ int fill_peer(PeerP& P, const float* const* peer_grads, float* const* peer_param
     P.flags[r] = (unsigned*)peer_flags[r];
   }
   MLG_CHECK_ARG(((uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) % 16 == 0, "mlg_peer_adam_step: 16-byte alignment");
-  const long long shard = (hi - lo) / world;
+  const long long shard = n / world;
   P.m = exp_avg; P.v = exp_avg_sq; P.step_dev = step_dev; P.host_status = host_status;
-  P.lo = lo + shard * rank; P.hi = P.lo + shard;
+  P.lo = shard * rank; P.hi = P.lo + shard;
   P.world = world; P.rank = rank;
   P.lr = lr; P.b1 = beta1; P.b2 = beta2; P.eps = eps; P.wd = weight_decay;
   P.timeout_clocks = (long long)((timeout_s > 0 ? timeout_s : 5.0) * 1.9e9);
@@ -269,20 +264,18 @@ extern "C" int mlg_peer_close(void* ptr) {
 }
 
 extern "C" int mlg_peer_adam_step(const float* const* peer_grads, float* const* peer_params, void* const* peer_flags,
-                                  int world, int rank, int64_t lo, int64_t hi, float* exp_avg, float* exp_avg_sq,
+                                  int world, int rank, int64_t n, float* exp_avg, float* exp_avg_sq,
                                   float* step_dev, float lr, float beta1, float beta2, float eps, float weight_decay,
-                                  double timeout_s, int32_t* host_status, int max_blocks, void* stream) {
-  if (hi == lo) return MLG_OK;
+                                  double timeout_s, int32_t* host_status, void* stream) {
+  if (n == 0) return MLG_OK;
   PeerP P;
-  if (int rc = fill_peer(P, peer_grads, peer_params, peer_flags, world, rank, lo, hi, exp_avg, exp_avg_sq, step_dev, lr, beta1,
+  if (int rc = fill_peer(P, peer_grads, peer_params, peer_flags, world, rank, n, exp_avg, exp_avg_sq, step_dev, lr, beta1,
                          beta2, eps, weight_decay, timeout_s, host_status))
     return rc;
   // enough blocks to keep ~world float4 loads per thread in flight on every NVLink, few enough that the whole grid is
   // resident next to whatever else the stream overlaps
-  // (max_blocks > 0: a chunk that runs NEXT TO other kernels -- the early head chunk -- takes fewer SMs away from them)
   long long blocks = ((P.hi - P.lo) / 4 + kThreads - 1) / kThreads;
-  const long long cap = max_blocks > 0 ? max_blocks : 96;
-  if (blocks > cap) blocks = cap;
+  if (blocks > 96) blocks = 96;
   if (blocks < 1) blocks = 1;
   peer_adam_kernel<<<(unsigned)blocks, kThreads, 0, (cudaStream_t)stream>>>(P);
   MLG_CHECK_LAUNCH("mlg_peer_adam_step");
@@ -295,14 +288,14 @@ extern "C" int mlg_peer_adam_step(const float* const* peer_grads, float* const* 
 extern "C" int64_t mlg_peer_emulated_bytes(int world) { return (int64_t)world * (int64_t)sizeof(PeerP); }
 
 extern "C" int mlg_peer_adam_step_emulated(const float* const* peer_grads, float* const* peer_params, void* const* peer_flags,
-                                           int world, int64_t lo, int64_t hi, float* const* exp_avg, float* const* exp_avg_sq,
+                                           int world, int64_t n, float* const* exp_avg, float* const* exp_avg_sq,
                                            float* const* step_dev, float lr, float beta1, float beta2, float eps,
                                            float weight_decay, double timeout_s, void* ranks_dev, void* stream) {
   MLG_CHECK_ARG(exp_avg && exp_avg_sq && step_dev && ranks_dev, "mlg_peer_adam_step_emulated: null pointer");
-  if (hi == lo) return MLG_OK;
+  if (n == 0) return MLG_OK;
   PeerP host[kMaxWorld];
   for (int r = 0; r < world; ++r)
-    if (int rc = fill_peer(host[r], peer_grads, peer_params, peer_flags, world, r, lo, hi, exp_avg[r], exp_avg_sq[r], step_dev[r],
+    if (int rc = fill_peer(host[r], peer_grads, peer_params, peer_flags, world, r, n, exp_avg[r], exp_avg_sq[r], step_dev[r],
                            lr, beta1, beta2, eps, weight_decay, timeout_s, nullptr))
       return rc;
   cudaStream_t st = (cudaStream_t)stream;

@@ -3,8 +3,6 @@
 Each Function cites the reference lines whose autograd graph it replaces.  Tensors are allocated by
 torch, the kernels only fill them (include/mlg_b200.h conventions).
 """
-import os
-
 import torch
 
 from . import _cabi
@@ -519,90 +517,14 @@ class SageAggregate(torch.autograd.Function):
         return gx, None, None
 
 
-def _flag(name, default):
-    """Tuning switches that are worth flipping from the shell for an A/B run (tools/): everything else is a module constant."""
-    return os.environ.get(name, "1" if default else "0") == "1"
-
-
 # Evaluation order of a SAGE layer (same algebra, torch_vertex.py:269-294; DESIGN.md section 4).  Module constants -- the parity
 # tests flip them to compare each order with the buffered one -- not environment switches.
-# first layer of MultilevelGNN through mlg_sage_rank1_fwd_rows / mlg_sage_rank1_bwd_rows; "gather": backward through the
-# by-source gather mlg_sage_rank1_bwd (any width); False: [x0 | agg] buffer + GEMMs
+# first layer of MultilevelGNN through mlg_sage_rank1_fwd_rows / mlg_sage_rank1_bwd_rows (widths 32 and 64); False: [x0 | agg]
+# buffer + GEMMs
 FACTORED_RANK1 = True
 # SAGE layers with out_channels < in_channels evaluated transform-first (gather on the narrower rows); False: [x | agg] + GEMM
 TRANSFORM_FIRST = True
 H1_NODE_MAJOR = True     # the factored first layer writes its output node-major for a transform-first consumer (and takes its gradient so)
-GZ_NODE_MAJOR = True     # the pool writes the last layer's output gradient node-major for the transform-first backward aggregation
-# The factored first layer applies LeakyReLU'(y) to its output gradient INSIDE mlg_sage_rank1_bwd_rows, from 64 sign bits per
-# (gene, replica) its forward kernel wrote (B200: 66 us vs 61 us unmasked; re-reading the 126 MB activation instead costs
-# 175 us, profiles/r02_rank1_bwd_probe.jsonl).  Widths without sign words (!= 64): one library leaky_relu_backward pass.
-RANK1_SIGN_BITS = True
-# forward of the factored first layer with one warp per gene for all replicas (mlg_sage_rank1_fwd_rows); False: r01's kernel
-RANK1_FWD_ROWS = True
-
-# Independent branches of the backward pass on forked streams (captured by the trainer's CUDA graph as parallel branches):
-# a layer's weight gradient does not feed the input-gradient chain, so it runs next to it instead of in front of it.
-# Both branches are HBM streams, so the win is the latency / tail overlap, not 2x.  The fork is joined back into the
-# launching stream at the END of the backward pass (autograd engine callback); tensors the side branch reads stay
-# referenced until then (no cross-stream reuse by the caching allocator).
-# measured on B200 (gpurun_out r02_bench_quick: 0.8455 ms forked vs 0.8463 ms serial): no gain today -- the big backward kernels
-# (gemm_tf32x3, xty_tc) are persistent one-CTA-per-SM kernels that cannot co-reside, so the branches serialise anyway; off by default
-PARALLEL_BACKWARD = _flag("MLG_PARALLEL_BACKWARD", False)     # A/B switch (tools/gpu_quick.sh)
-# Set by train.Trainer around its own autograd.grad call only: the gradients a forked branch produces may not be touched
-# before the end-of-backward join, which holds for the trainer (it stores them after the pass) but not for an arbitrary
-# loss.backward(), whose AccumulateGrad nodes run on the launching stream as soon as a Function returns.
-PARALLEL_ACTIVE = False
-# set by train.Trainer (data parallel, fused peer update): called at the end of HeadMLP.backward, when the classifier head's
-# gradients are final, to start that chunk's reduce-scatter / Adam / all-gather while the rest of backward runs
-AFTER_HEAD_BACKWARD = None
-_SIDE_STREAMS = {}
-
-
-def _side_stream(device, idx):
-    key = (device.index if device.index is not None else torch.cuda.current_device(), idx)
-    if key not in _SIDE_STREAMS:
-        _SIDE_STREAMS[key] = torch.cuda.Stream(device=device)
-    return _SIDE_STREAMS[key]
-
-
-class _Forked:
-    """with _Forked(device, idx, keep=[tensors the branch reads]) as f: ... enqueue the branch ...
-    Inside the block the current stream is a side stream that waits for everything enqueued so far; leaving the block
-    registers the join for the end of the backward pass.  Outside a backward pass, or with PARALLEL_BACKWARD off, the
-    block simply runs on the current stream."""
-
-    def __init__(self, device, idx, keep=(), force=False):
-        self.device, self.idx, self.keep, self.force = device, idx, list(keep), force
-        self.active = False
-
-    def __enter__(self):
-        if not ((PARALLEL_BACKWARD or self.force) and PARALLEL_ACTIVE and self.device.type == "cuda"):
-            return self
-        self.main = torch.cuda.current_stream(self.device)
-        self.side = _side_stream(self.device, self.idx)
-        self.side.wait_stream(self.main)
-        self.ctx = torch.cuda.stream(self.side)
-        self.ctx.__enter__()
-        self.active = True
-        return self
-
-    def hold(self, *tensors):
-        self.keep.extend(t for t in tensors if t is not None)
-
-    def __exit__(self, *exc):
-        if not self.active:
-            return False
-        self.ctx.__exit__(*exc)
-        main, side, keep = self.main, self.side, self.keep
-
-        def join(_keep=keep):
-            main.wait_stream(side)
-
-        try:
-            torch.autograd.Variable._execution_engine.queue_callback(join)
-        except RuntimeError:          # not inside a backward pass: join right away
-            join()
-        return False
 
 
 class SageLayer(torch.autograd.Function):
@@ -638,7 +560,8 @@ class SageLayer(torch.autograd.Function):
         w_r, w_nn = lin_r_w.detach(), nn_w.detach()
         w_r, w_nn = _f32c(w_r), _f32c(w_nn)
         cout = w_nn.shape[0]
-        factored_ok = (FACTORED_RANK1 and rank1 and not relative and topo.replicas > 1 and cout % 4 == 0
+        factored_ok = (FACTORED_RANK1 and rank1 and not relative and topo.replicas > 1
+                       and bool(_cabi.lib().mlg_sage_rank1_fwd_rows_supported(cout))
                        and xd.shape[0] == topo.n_single and n == topo.n_single * topo.replicas)
         tfirst_ok = (not factored_ok and TRANSFORM_FIRST and not rank1 and not relative and in_slope is None
                      and topo.replicas > 1 and cout < cin and cout % 4 == 0 and cin % 4 == 0
@@ -685,36 +608,26 @@ class SageLayer(torch.autograd.Function):
             bias = None if nn_b is None else _f32c(nn_b.detach())
             nbytes = 4 * cout * n + 4 * n + 8 * csr.col.numel() + 8 * cout * n1
             # the consumer does not pre-mask our output gradient: keep the sign bits of y (8 bytes per row and replica) so that
-            # the backward kernel applies LeakyReLU' without re-reading y
+            # mlg_sage_rank1_bwd_rows applies LeakyReLU' without re-reading y (B200: 66 us vs 61 us unmasked; re-reading the
+            # 126 MB activation instead costs 175 us, profiles/r02_rank1_bwd_probe.jsonl).  Width 32 has no sign words: its
+            # backward takes one library leaky_relu_backward pass.
             mbits = None
-            if RANK1_SIGN_BITS and cout == 64 and not out_premasked and any(ctx.needs_input_grad):
+            if cout == 64 and not out_premasked and any(ctx.needs_input_grad):
                 mbits = torch.empty(n1 * topo.replicas, dtype=torch.int64, device=xd.device)
-            rows_ok = RANK1_FWD_ROWS and bool(L.mlg_sage_rank1_fwd_rows_supported(cout))
-            xs_t = None
-            h1_nm = bool(H1_NODE_MAJOR and rows_ok and link is not None and link.get("want_h1_nm")
-                         and bool(L.mlg_sage_rank1_bwd_rows_supported(cout)) and FACTORED_RANK1 != "gather")
+            h1_nm = bool(H1_NODE_MAJOR and link is not None and link.get("want_h1_nm"))
             fwd_rows = L.mlg_sage_rank1_fwd_rows_nm if h1_nm else L.mlg_sage_rank1_fwd_rows
             with torch.cuda.device(xd.device):
-                if rows_ok:
-                    # node values transposed to [n1, B]: one coalesced load per CSR entry in the forward AND the backward kernel
-                    xs_t = torch.empty(n1 * topo.replicas, dtype=torch.float32, device=xd.device)
-                    _cabi.check(L.mlg_transpose_bn(_cabi.fptr(xs_d), topo.replicas, n1, _cabi.fptr(xs_t), _cabi.stream_ptr()),
-                                "mlg_transpose_bn")
+                # node values transposed to [n1, B]: one coalesced load per CSR entry in the forward AND the backward kernel
+                xs_t = torch.empty(n1 * topo.replicas, dtype=torch.float32, device=xd.device)
+                _cabi.check(L.mlg_transpose_bn(_cabi.fptr(xs_d), topo.replicas, n1, _cabi.fptr(xs_t), _cabi.stream_ptr()),
+                            "mlg_transpose_bn")
                 with _cabi.span("sage_rank1_fwd", nbytes):
-                    if rows_ok:
-                        _cabi.check(fwd_rows(
-                            _cabi.fptr(xs_t), _vptr(e12), 2 * cout, _vptr(e12[:, cout:]), 2 * cout, _cabi.iptr(csr.rowptr),
-                            _cabi.iptr(csr.col), _cabi.fptr(topo.fwd_val, True),
-                            _cabi.iptr(topo.fwd_order, True), n1, cout, topo.replicas,
-                            _cabi.fptr(bias, True), float(slope), _cabi.fptr(y), cout, _cabi.lptr(mbits, True),
-                            _cabi.stream_ptr()), "mlg_sage_rank1_fwd_rows")
-                    else:
-                        _cabi.check(L.mlg_sage_rank1_fwd(
-                            _cabi.fptr(xs_d), _vptr(e12), 2 * cout, _vptr(e12[:, cout:]), 2 * cout, _cabi.iptr(csr.rowptr),
-                            _cabi.iptr(csr.col), _cabi.fptr(topo.fwd_val, True),
-                            _cabi.iptr(topo.fwd_order, True), n1, cout, topo.replicas,
-                            _cabi.fptr(bias, True), float(slope), _cabi.fptr(y), cout, _cabi.lptr(mbits, True),
-                            _cabi.stream_ptr()), "mlg_sage_rank1_fwd")
+                    _cabi.check(fwd_rows(
+                        _cabi.fptr(xs_t), _vptr(e12), 2 * cout, _vptr(e12[:, cout:]), 2 * cout, _cabi.iptr(csr.rowptr),
+                        _cabi.iptr(csr.col), _cabi.fptr(topo.fwd_val, True),
+                        _cabi.iptr(topo.fwd_order, True), n1, cout, topo.replicas,
+                        _cabi.fptr(bias, True), float(slope), _cabi.fptr(y), cout, _cabi.lptr(mbits, True),
+                        _cabi.stream_ptr()), "mlg_sage_rank1_fwd_rows")
             ctx.xs_t = xs_t
             ctx.mbits = mbits
             ctx.h1_nm = h1_nm
@@ -723,7 +636,7 @@ class SageLayer(torch.autograd.Function):
             ctx.xs_shape = xs.shape
             if h1_nm:
                 link["h1_nm"] = True          # y (and the gradient this layer gets back) is node-major
-            ctx.save_for_backward(xd, y, wst, w_r, w_nn, xs_d)
+            ctx.save_for_backward(xd, y, wst, w_r, w_nn, None)
             ctx.topo, ctx.relative, ctx.slope, ctx.cin, ctx.has_bias = topo, False, float(slope), cin, nn_b is not None
             ctx.rank1, ctx.factored, ctx.transform_first = True, True, False
             ctx.emb_param = x if isinstance(x, torch.nn.Parameter) else None
@@ -757,7 +670,7 @@ class SageLayer(torch.autograd.Function):
             # ``link``: shared with the PathwayPool that consumes y and pre-masks its gradient (out_premasked).  gy then IS dL/dz
             # and its only reader is this layer's backward aggregation, so the pool may write it NODE-MAJOR (row i * B + b: the B
             # replica rows a CSR entry gathers are one contiguous block) -- requested here, confirmed by the pool's backward.
-            ctx.link = link if (GZ_NODE_MAJOR and link is not None and out_premasked and cout == 32 and topo.replicas > 1) else None
+            ctx.link = link if (link is not None and out_premasked and cout == 32 and topo.replicas > 1) else None
             if ctx.link is not None:
                 ctx.link["gz_node_major"] = True
             return y
@@ -799,7 +712,7 @@ class SageLayer(torch.autograd.Function):
         nbytes = 4 * cout * gz.shape[0] + 8 * fw.col.numel() + 3 * ws_bytes + 4 * g_xs.numel()
         with torch.cuda.device(gz.device), _cabi.span("sage_rank1_bwd_xs", nbytes):
             _cabi.check(L.mlg_sage_rank1_bwd_xs(
-                _cabi.fptr(gz), cout, 1 if getattr(ctx, "h1_nm", False) else 0, _cabi.fptr(y, True), _cabi.lptr(bits, True),
+                _cabi.fptr(gz), cout, 1 if ctx.h1_nm else 0, _cabi.fptr(y, True), _cabi.lptr(bits, True),
                 float(ctx.slope), _vptr(e12), 2 * cout, _vptr(e12[:, cout:]), 2 * cout, _cabi.iptr(fw.rowptr),
                 _cabi.iptr(fw.col), _cabi.fptr(topo.fwd_val, True), _cabi.iptr(topo.fwd_order, True), _cabi.iptr(bw.rowptr),
                 _cabi.iptr(topo.bwd2fwd), n1, fw.cap, cout, B, _cabi.fptr(g_xs), _cabi.fptr(ws), ws_bytes,
@@ -808,7 +721,7 @@ class SageLayer(torch.autograd.Function):
 
     @staticmethod
     def _backward_factored(ctx, gy):
-        emb, y, wst, w_r, w_nn, xs_d = ctx.saved_tensors
+        emb, y, wst, w_r, w_nn, _ = ctx.saved_tensors
         topo, cin = ctx.topo, ctx.cin
         cout = w_nn.shape[0]
         gy = _f32c(gy)
@@ -824,11 +737,10 @@ class SageLayer(torch.autograd.Function):
             else:
                 g_xs = SageLayer._rank1_input_grad(ctx, gy, ctx.mbits, None if ctx.mbits is not None else y)
             return None, g_xs, None, None, None, None, None, None, None, None, None, None
-        by_rows = FACTORED_RANK1 != "gather" and bool(L.mlg_sage_rank1_bwd_rows_supported(cout))
-        y_mask = bits = None
+        bits = None
         if ctx.out_premasked:
             gz = gy
-        elif by_rows and ctx.mbits is not None:
+        elif ctx.mbits is not None:
             # the kernel applies LeakyReLU'(y) while it loads the gradient rows, from the forward kernel's sign bits
             gz, bits = gy, ctx.mbits
         else:
@@ -836,61 +748,40 @@ class SageLayer(torch.autograd.Function):
                 else torch.ops.aten.threshold_backward(gy, y, 0.0)
         if needs[1]:
             g_xs = SageLayer._rank1_input_grad(ctx, gz, bits, None)
-        if by_rows:
-            # by target row: gz read once -> per-entry rows h (+ the self / bias reductions), then a segment sum by source
-            fw, bw = topo.fwd, topo.bwd
-            g12 = torch.empty(n1, 2 * cout, dtype=torch.float32, device=gz.device)      # [g_E_self | g_E_nbr]
-            gbr = torch.empty(n1, cout, dtype=torch.float32, device=gz.device)
-            h = torch.empty(fw.cap, cout, dtype=torch.float32, device=gz.device)
-            nbytes = 4 * cout * gz.shape[0] + 4 * gz.shape[0] + 8 * fw.col.numel() + 4 * (h.numel() + 2 * gbr.numel())
-            with torch.cuda.device(gz.device), _cabi.span("sage_rank1_bwd", nbytes):
-                xs_t = getattr(ctx, "xs_t", None)
-                bwd_rows = L.mlg_sage_rank1_bwd_rows_nm if getattr(ctx, "h1_nm", False) else L.mlg_sage_rank1_bwd_rows
-                _cabi.check(bwd_rows(
-                    _cabi.fptr(gz), cout, _cabi.fptr(y_mask, True),
-                    _cabi.lptr(bits, True), float(ctx.slope),
-                    _cabi.fptr(xs_d if xs_t is None else xs_t), 0 if xs_t is None else 1, _cabi.iptr(fw.rowptr),
-                    _cabi.iptr(fw.col),
-                    _cabi.fptr(topo.fwd_val, True), _cabi.iptr(topo.fwd_order, True), n1, cout, B,
-                    _cabi.fptr(h),
-                    _cabi.fptr(g12), 2 * cout, _cabi.fptr(gbr), _cabi.stream_ptr()), "mlg_sage_rank1_bwd_rows")
-            g_b = None
-            if ctx.has_bias:       # column sums of the per-row partials: one streaming pass, fixed order (mlg_wcolsum)
-                with _Forked(gz.device, 1, keep=(gbr,)) as fk:      # independent of the segment sum below
-                    g_b = grad_slot(ctx.wparams[2], (cout,))
-                    if g_b is None:
-                        g_b = torch.empty(cout, dtype=torch.float32, device=gz.device)
-                    ws_bytes = L.mlg_wcolsum_workspace_bytes(n1, cout)
-                    ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=gz.device)
-                    with torch.cuda.device(gz.device):
-                        _cabi.check(L.mlg_wcolsum(_cabi.fptr(gbr), cout, None, n1, cout, None, _cabi.fptr(g_b), _cabi.fptr(ws),
-                                                  ws_bytes, _cabi.stream_ptr()), "mlg_wcolsum")
-                    fk.hold(g_b, ws)
-            gather_sum(h, bw.rowptr, topo.bwd2fwd, n1, out=g12[:, cout:], order=topo.bwd_order, tag="sage_rank1_bwd_seg")
-        else:
-            slices = L.mlg_gather_sum_slices(n1, cout, B)
-            parts = torch.empty(slices * n1 * 3 * cout, dtype=torch.float32, device=gz.device)
-            p12 = parts[:slices * n1 * 2 * cout].view(slices, n1, 2 * cout)
-            pb = parts[slices * n1 * 2 * cout:].view(slices * n1, cout)
-            bw = topo.bwd
-            nbytes = 4 * cout * gz.shape[0] + 4 * gz.shape[0] + 8 * bw.col.numel() + 4 * parts.numel()
-            with torch.cuda.device(gz.device), _cabi.span("sage_rank1_bwd", nbytes):
-                _cabi.check(L.mlg_sage_rank1_bwd(
-                    _cabi.fptr(gz), cout, _cabi.fptr(xs_d), _cabi.iptr(bw.rowptr), _cabi.iptr(bw.col),
-                    _cabi.fptr(topo.bwd_val, True), _cabi.fptr(topo.inv_cnt, True), _cabi.iptr(topo.bwd_order, True), n1, cout, B,
-                    _cabi.fptr(p12), _cabi.fptr(pb), _cabi.stream_ptr()), "mlg_sage_rank1_bwd")
-            g12 = p12.sum(0) if slices > 1 else p12[0]                 # [n1, 2cout] = [g_E_self | g_E_nbr]
-            g_b = pb.sum(0) if ctx.has_bias else None
-        # [2cout, cin] = [g_W1 ; g_(W2 W_r)] = g12^T emb (a 15 405-deep reduction) + the weight un-folding: on a forked stream
-        # next to the table -> embedding product
-        with _Forked(gz.device, 2, keep=(g12, emb, w_nn, w_r)) as fk:
-            g_wst, _ = xty(g12, emb, tag="sage_rank1_wgrad")                       # [2cout, cin], stacked like Wst
-            g_wnn, g_wr = _slot_or_empty(ctx.wparams[1], w_nn), _slot_or_empty(ctx.wparams[0], w_r)
+        # by target row: gz read once -> per-entry rows h (+ the self / bias reductions), then a segment sum by source
+        fw, bw = topo.fwd, topo.bwd
+        g12 = torch.empty(n1, 2 * cout, dtype=torch.float32, device=gz.device)      # [g_E_self | g_E_nbr]
+        gbr = torch.empty(n1, cout, dtype=torch.float32, device=gz.device)
+        h = torch.empty(fw.cap, cout, dtype=torch.float32, device=gz.device)
+        nbytes = 4 * cout * gz.shape[0] + 4 * gz.shape[0] + 8 * fw.col.numel() + 4 * (h.numel() + 2 * gbr.numel())
+        with torch.cuda.device(gz.device), _cabi.span("sage_rank1_bwd", nbytes):
+            bwd_rows = L.mlg_sage_rank1_bwd_rows_nm if ctx.h1_nm else L.mlg_sage_rank1_bwd_rows
+            _cabi.check(bwd_rows(
+                _cabi.fptr(gz), cout, None,
+                _cabi.lptr(bits, True), float(ctx.slope),
+                _cabi.fptr(ctx.xs_t), 1, _cabi.iptr(fw.rowptr),
+                _cabi.iptr(fw.col),
+                _cabi.fptr(topo.fwd_val, True), _cabi.iptr(topo.fwd_order, True), n1, cout, B,
+                _cabi.fptr(h),
+                _cabi.fptr(g12), 2 * cout, _cabi.fptr(gbr), _cabi.stream_ptr()), "mlg_sage_rank1_bwd_rows")
+        g_b = None
+        if ctx.has_bias:       # column sums of the per-row partials: one streaming pass, fixed order (mlg_wcolsum)
+            g_b = grad_slot(ctx.wparams[2], (cout,))
+            if g_b is None:
+                g_b = torch.empty(cout, dtype=torch.float32, device=gz.device)
+            ws_bytes = L.mlg_wcolsum_workspace_bytes(n1, cout)
+            ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=gz.device)
             with torch.cuda.device(gz.device):
-                _cabi.check(L.mlg_sage_fold_stacked_bwd(_cabi.fptr(g_wst), None, cin, _cabi.fptr(w_nn), _cabi.fptr(w_r), cout,
-                                                        cin, w_r.shape[0], _cabi.fptr(g_wnn), _cabi.fptr(g_wr),
-                                                        _cabi.stream_ptr()), "mlg_sage_fold_stacked_bwd")
-            fk.hold(g_wst, g_wnn, g_wr)
+                _cabi.check(L.mlg_wcolsum(_cabi.fptr(gbr), cout, None, n1, cout, None, _cabi.fptr(g_b), _cabi.fptr(ws),
+                                          ws_bytes, _cabi.stream_ptr()), "mlg_wcolsum")
+        gather_sum(h, bw.rowptr, topo.bwd2fwd, n1, out=g12[:, cout:], order=topo.bwd_order, tag="sage_rank1_bwd_seg")
+        # [2cout, cin] = [g_W1 ; g_(W2 W_r)] = g12^T emb (a 15 405-deep reduction) + the weight un-folding
+        g_wst, _ = xty(g12, emb, tag="sage_rank1_wgrad")                       # [2cout, cin], stacked like Wst
+        g_wnn, g_wr = _slot_or_empty(ctx.wparams[1], w_nn), _slot_or_empty(ctx.wparams[0], w_r)
+        with torch.cuda.device(gz.device):
+            _cabi.check(L.mlg_sage_fold_stacked_bwd(_cabi.fptr(g_wst), None, cin, _cabi.fptr(w_nn), _cabi.fptr(w_r), cout,
+                                                    cin, w_r.shape[0], _cabi.fptr(g_wnn), _cabi.fptr(g_wr),
+                                                    _cabi.stream_ptr()), "mlg_sage_fold_stacked_bwd")
         slot = grad_slot(ctx.emb_param, (n1, cin)) if ctx.emb_param is not None else None
         g_emb = tall_matmul(g12, wst.t(), tag="sage_rank1_demb", w_split=ctx.wst_t_split, out=slot)     # g12 @ Wst
         return g_emb, g_xs, g_wr, g_wnn, g_b, None, None, None, None, None, None, None
@@ -911,9 +802,9 @@ class SageLayer(torch.autograd.Function):
         bw = topo.bwd
         # G = [g_U | g_V] = [gz | A^T gz]: the by-source aggregation runs on the cout-wide gz rows and copies them alongside
         g_uv = torch.empty(n, 2 * cout, dtype=torch.float32, device=gz.device)
-        link = getattr(ctx, "link", None)
+        link = ctx.link
         gz_nm = bool(link is not None and link.pop("gz_written_node_major", False))
-        x_nm = bool(getattr(ctx, "x_nm", False))
+        x_nm = ctx.x_nm
         if x_nm and not gz_nm:      # x (and so g_uv) node-major but the gradient arrived graph-major: one transposing copy
             gz = gz.view(topo.replicas, topo.n_single, cout).transpose(0, 1).contiguous().view(n, cout)
             gz_nm = True
@@ -932,29 +823,25 @@ class SageLayer(torch.autograd.Function):
                        tag="sage_aggr_bwd")
         needs = ctx.needs_input_grad
         gx = g_wr = g_wnn = g_b = None
-        # the weight gradient (tensor-core x^T G over the row pairs + fold) on a forked stream next to the input-gradient GEMM
-        # and everything autograd runs after it (the first layer's backward); joined at the end of the backward pass
         if needs[2] or needs[3] or needs[4]:
-            with _Forked(gz.device, 0, keep=(g_uv, x, w_nn, w_r)) as fk:
-                if n % 2 == 0 and 4 * cout == 128 and 2 * cin == 128:
-                    # tensor-core weight gradient on ROW PAIRS: [G_even | G_odd]^T [x_even | x_odd] is 128 x 128; its two
-                    # diagonal blocks are the even- and odd-row halves of G^T x (the off-diagonal blocks are discarded)
-                    # (the two diagonal blocks are added inside the un-folding kernel)
-                    o2, cs2 = xty(g_uv.view(n // 2, 4 * cout), x.view(n // 2, 2 * cin), want_colsum=ctx.has_bias, tag="sage_wgrad")
-                    ga, gb, ld = o2, o2[2 * cout:, cin:], 2 * cin
-                    if ctx.has_bias:
-                        g_b = torch.add(cs2[:cout], cs2[2 * cout:3 * cout], out=grad_slot(ctx.wparams[2], (cout,)))
-                else:
-                    o2, cs = xty(g_uv, x, want_colsum=ctx.has_bias, tag="sage_wgrad")
-                    ga, gb, ld = o2, None, cin
-                    if ctx.has_bias:
-                        g_b = cs[:cout]
-                g_wnn, g_wr = _slot_or_empty(ctx.wparams[1], w_nn), _slot_or_empty(ctx.wparams[0], w_r)
-                with torch.cuda.device(gz.device):
-                    _cabi.check(L.mlg_sage_fold_stacked_bwd(_vptr(ga), None if gb is None else _vptr(gb), ld, _cabi.fptr(w_nn),
-                                                            _cabi.fptr(w_r), cout, cin, w_r.shape[0], _cabi.fptr(g_wnn),
-                                                            _cabi.fptr(g_wr), _cabi.stream_ptr()), "mlg_sage_fold_stacked_bwd")
-                fk.hold(o2, g_wnn, g_wr, g_b)
+            if n % 2 == 0 and 4 * cout == 128 and 2 * cin == 128:
+                # tensor-core weight gradient on ROW PAIRS: [G_even | G_odd]^T [x_even | x_odd] is 128 x 128; its two
+                # diagonal blocks are the even- and odd-row halves of G^T x (the off-diagonal blocks are discarded)
+                # (the two diagonal blocks are added inside the un-folding kernel)
+                o2, cs2 = xty(g_uv.view(n // 2, 4 * cout), x.view(n // 2, 2 * cin), want_colsum=ctx.has_bias, tag="sage_wgrad")
+                ga, gb, ld = o2, o2[2 * cout:, cin:], 2 * cin
+                if ctx.has_bias:
+                    g_b = torch.add(cs2[:cout], cs2[2 * cout:3 * cout], out=grad_slot(ctx.wparams[2], (cout,)))
+            else:
+                o2, cs = xty(g_uv, x, want_colsum=ctx.has_bias, tag="sage_wgrad")
+                ga, gb, ld = o2, None, cin
+                if ctx.has_bias:
+                    g_b = cs[:cout]
+            g_wnn, g_wr = _slot_or_empty(ctx.wparams[1], w_nn), _slot_or_empty(ctx.wparams[0], w_r)
+            with torch.cuda.device(gz.device):
+                _cabi.check(L.mlg_sage_fold_stacked_bwd(_vptr(ga), None if gb is None else _vptr(gb), ld, _cabi.fptr(w_nn),
+                                                        _cabi.fptr(w_r), cout, cin, w_r.shape[0], _cabi.fptr(g_wnn),
+                                                        _cabi.fptr(g_wr), _cabi.stream_ptr()), "mlg_sage_fold_stacked_bwd")
         if needs[0]:
             gx = tall_matmul(g_uv, wst.t(), tag="sage_dgrad_gemm", w_split=ctx.wst_t_split)     # dL/dx (the producer masks it itself)
         return gx, None, g_wr, g_wnn, (g_b if ctx.has_bias else None), None, None, None, None, None, None, None
@@ -1474,8 +1361,6 @@ class HeadMLP(torch.autograd.Function):
                                            _cabi.fptr(gb0, True), _cabi.fptr(gW3, True), _cabi.fptr(gb3, True),
                                            _cabi.stream_ptr()),
                         "mlg_head_mlp_bwd")
-        if AFTER_HEAD_BACKWARD is not None:
-            AFTER_HEAD_BACKWARD()
         return g_a0, gW0, gb0, gW3, gb3, None, None, None, None
 
 

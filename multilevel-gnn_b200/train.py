@@ -1,24 +1,17 @@
 """The caller of the hot path: one training step as the reference's ``train()`` runs it
 (train.py:38-68; optimizer / criterion set-up train.py:112-125), plus the data-parallel wrapper the
 reference lacks (SURVEY.md section 8e): patient graphs are independent, so every rank steps on its own
-batch and the replicas are synchronised by ONE fused kernel per parameter chunk over NVLink peer memory
-(gradient reduce-scatter -> Adam on the owned shard -> parameter all-gather, csrc/peer_adam.cu; the
-classifier-head chunk is launched from inside backward) -- or, selectably, one NCCL all-reduce (op=AVG)
+batch and the replicas are synchronised by ONE fused kernel after backward over NVLink peer memory
+(gradient reduce-scatter -> Adam on the owned shard -> parameter all-gather, csrc/peer_adam.cu) -- or,
+selectably, one NCCL all-reduce (op=AVG)
 over the flat fp32 gradient bucket followed by a replicated flat Adam.  Parameters that never receive a
 gradient (``lin_l.weight`` of every SAGEConv, ``info_mask``) are left out of the bucket and of the
 optimizer state.
 """
-import os
 from typing import NamedTuple, Optional
 
 import torch
 import torch.distributed as dist
-
-# Chunks of the fused peer update.  2 = the classifier-head chunk is exchanged from inside backward (VERDICT r01 item 6); it
-# was built, is tested, and measured SLOWER than one kernel after backward: N=2 on one box, 20-step windows, 0.8755 ms with
-# two chunks against 0.8613 ms with one (single GPU 0.833 ms; 8 / 24 / 64 early blocks alike) -- the early kernel's blocks
-# share SMs with the persistent backward kernels, whose duration is set by their slowest CTA.  MLG_PEER_CHUNKS=2 selects it.
-PEER_CHUNKS = int(os.environ.get("MLG_PEER_CHUNKS", "1"))
 
 
 def shard_indices(n_items, rank, world, per_rank_batch, epoch_seed=0, drop_last=True):
@@ -41,22 +34,17 @@ class GradBucket:
     """Flat fp32 gradient bucket: every ``p.grad`` is a view into one contiguous buffer, so the data-parallel
     synchronisation is ONE all-reduce with no packing/unpacking (NCCL: op=AVG folds the 1/world scale in;
     gloo has no AVG, so SUM + scale).  Parameters that never get a gradient are not in the bucket.
-    ``segments``: the parameters in groups that start at offsets aligned to ``align`` elements (the chunks of the fused
-    peer update: each chunk's length must divide by 4 * world); ``bounds`` = the (lo, hi) element range of every group."""
+    ``align``: the bucket length is rounded up to a multiple of it (the fused peer update needs a multiple of 4 * world);
+    the padding elements stay zero."""
 
-    def __init__(self, params, flat=None, segments=None, align=1):
-        segments = [list(params)] if segments is None else [list(g) for g in segments]
-        self.params = [p for g in segments for p in g]
+    def __init__(self, params, flat=None, align=1):
+        self.params = list(params)
         dev = self.params[0].device
-        self.offsets, self.bounds, off = {}, [], 0
-        for g in segments:
-            lo = off
-            for p in g:
-                self.offsets[id(p)] = off
-                off += p.numel()
-            off = -(-off // align) * align          # group end rounded up: padding elements stay zero
-            self.bounds.append((lo, off))
-        n = off
+        self.offsets, off = {}, 0
+        for p in self.params:
+            self.offsets[id(p)] = off
+            off += p.numel()
+        n = GradBucket.padded_size(self.params, align)
         self.n = n
         # ``flat``: caller-provided storage (PeerArena: peer-mapped device memory, padded past n)
         self.flat = torch.zeros(n, dtype=torch.float32, device=dev) if flat is None else flat
@@ -68,12 +56,8 @@ class GradBucket:
             p._mlg_grad_slot = {"view": p.grad, "claimed": False}
 
     @staticmethod
-    def padded_size(segments, align):
-        off = 0
-        for g in segments:
-            off += sum(p.numel() for p in g)
-            off = -(-off // align) * align
-        return off
+    def padded_size(params, align):
+        return -(-sum(p.numel() for p in params) // align) * align
 
     def zero(self):
         self.flat.zero_()
@@ -143,17 +127,16 @@ class _DeviceSpan:
 
 
 class PeerArena:
-    """This rank's peer-visible device memory [gradient bucket | parameters | one flag block per chunk] (mlg_peer_alloc) and
-    the mappings of every other rank's arena (CUDA IPC handles exchanged once through torch.distributed)."""
+    """This rank's peer-visible device memory [gradient bucket | parameters | flag block] (mlg_peer_alloc) and the mappings
+    of every other rank's arena (CUDA IPC handles exchanged once through torch.distributed)."""
 
-    def __init__(self, n_padded, world, rank, device, exchange=True, n_chunks=1):
+    def __init__(self, n_padded, world, rank, device, exchange=True):
         from . import _cabi
         L = _cabi.lib()
-        self.world, self.rank, self.device, self.n_chunks = world, rank, device, n_chunks
+        self.world, self.rank, self.device = world, rank, device
         assert n_padded % 4 == 0
         self.n_padded = n_padded
-        self.flag_bytes = int(L.mlg_peer_flag_bytes())
-        self.bytes = 2 * 4 * self.n_padded + self.flag_bytes * n_chunks
+        self.bytes = 2 * 4 * self.n_padded + int(L.mlg_peer_flag_bytes())
         with torch.cuda.device(device):
             self.base = L.mlg_peer_alloc(self.bytes)
         if not self.base:
@@ -186,26 +169,22 @@ class PeerArena:
                 self._opened.append(ptr)
                 self.peer_base[r] = ptr
 
-    def pointer_tables(self, chunk=0):
-        """(grads, params, flags): ctypes arrays of ``world`` device pointers, indexed by rank (flags: of ``chunk``)."""
+    def pointer_tables(self):
+        """(grads, params, flags): ctypes arrays of ``world`` device pointers, indexed by rank."""
         import ctypes
         arr = ctypes.c_void_p * self.world
         g = arr(*[b for b in self.peer_base])
         p = arr(*[b + 4 * self.n_padded for b in self.peer_base])
-        f = arr(*[b + 8 * self.n_padded + chunk * self.flag_bytes for b in self.peer_base])
+        f = arr(*[b + 8 * self.n_padded for b in self.peer_base])
         return g, p, f
 
     def status(self):
-        """Non-zero when a wait of any chunk's update kernel gave up on this rank (device read: synchronises)."""
+        """Non-zero when a wait of the update kernel gave up on this rank (device read: synchronises)."""
         import ctypes
         from . import _cabi
-        worst = 0
-        for c in range(self.n_chunks):
-            out = ctypes.c_int(0)
-            _cabi.check(_cabi.lib().mlg_peer_status(self.base + 8 * self.n_padded + c * self.flag_bytes, ctypes.byref(out)),
-                        "mlg_peer_status")
-            worst = max(worst, out.value)
-        return worst
+        out = ctypes.c_int(0)
+        _cabi.check(_cabi.lib().mlg_peer_status(self.base + 8 * self.n_padded, ctypes.byref(out)), "mlg_peer_status")
+        return out.value
 
     def close(self):
         from . import _cabi
@@ -217,12 +196,11 @@ class PeerArena:
 
 
 class PeerAdam:
-    """Data-parallel optimizer step as ONE kernel per chunk over NVLink peer memory (mlg_peer_adam_step): reduce-scatter of
-    the gradient buckets, torch.optim.Adam on the owned 1/world shard (ZeRO-1: the moment buffers exist once per box),
+    """Data-parallel optimizer step as ONE kernel over NVLink peer memory (mlg_peer_adam_step): reduce-scatter of the
+    gradient buckets, torch.optim.Adam on the owned 1/world shard (ZeRO-1: the moment buffers exist once per box),
     all-gather of the updated parameters -- no NCCL call, no second graph, every rank bitwise in step.  Parameters are
-    re-homed as views of the arena's parameter buffer (like FlatAdam).  ``bucket.bounds`` are the chunks: ``step(c)`` updates
-    chunk c only (the trainer launches the classifier-head chunk from inside backward), ``step()`` whatever has not run yet
-    this round, ``finish_round()`` re-arms.  A wait that times out is a hard failure on every rank (``failed()``)."""
+    re-homed as views of the arena's parameter buffer (like FlatAdam).  A wait that times out is a hard failure on every
+    rank (``failed()``)."""
 
     def __init__(self, bucket, arena, lr, betas, eps=1e-8, weight_decay=0.0, timeout_s=5.0):
         self.bucket, self.arena = bucket, arena
@@ -232,42 +210,28 @@ class PeerAdam:
             n, off = p.numel(), bucket.offsets[id(p)]
             self.flat_p[off:off + n].copy_(p.data.reshape(-1))
             p.data = self.flat_p[off:off + n].view_as(p)
-        self.chunks = list(bucket.bounds)
-        assert len(self.chunks) <= arena.n_chunks
         dev = arena.device
-        self.exp_avg = [torch.zeros((hi - lo) // arena.world, dtype=torch.float32, device=dev) for lo, hi in self.chunks]
-        self.exp_avg_sq = [torch.zeros_like(t) for t in self.exp_avg]
-        self.step_dev = [torch.zeros(1, dtype=torch.float32, device=dev) for _ in self.chunks]
-        self._tables = [arena.pointer_tables(c) for c in range(len(self.chunks))]
-        # pinned host word the kernels set on a failed wait: read by the host without synchronising the device
+        self.exp_avg = torch.zeros(bucket.n // arena.world, dtype=torch.float32, device=dev)
+        self.exp_avg_sq = torch.zeros_like(self.exp_avg)
+        self.step_dev = torch.zeros(1, dtype=torch.float32, device=dev)
+        self._tables = arena.pointer_tables()
+        # pinned host word the kernel sets on a failed wait: read by the host without synchronising the device
         self.host_status = torch.zeros(1, dtype=torch.int32).pin_memory()
-        self._done = [False] * len(self.chunks)
 
     def failed(self):
         return int(self.host_status[0]) != 0
 
-    EARLY_BLOCKS = int(os.environ.get("MLG_PEER_EARLY_BLOCKS", "24"))      # grid cap of a chunk launched next to the backward kernels
-
-    def step(self, chunk=None):
+    def step(self):
         import ctypes
         from . import _cabi
-        L = _cabi.lib()
         a = self.arena
-        todo = [c for c in range(len(self.chunks)) if not self._done[c]] if chunk is None else [chunk]
+        g, p, f = self._tables
         with torch.cuda.device(a.device):
-            for c in todo:
-                g, p, f = self._tables[c]
-                lo, hi = self.chunks[c]
-                _cabi.check(L.mlg_peer_adam_step(g, p, f, a.world, a.rank, lo, hi, _cabi.fptr(self.exp_avg[c]),
-                                                 _cabi.fptr(self.exp_avg_sq[c]), _cabi.fptr(self.step_dev[c]), float(self.lr),
-                                                 float(self.betas[0]), float(self.betas[1]), float(self.eps), float(self.wd),
-                                                 float(self.timeout_s), ctypes.c_void_p(self.host_status.data_ptr()),
-                                                 self.EARLY_BLOCKS if chunk is not None else 0, _cabi.stream_ptr()),
-                            "mlg_peer_adam_step")
-                self._done[c] = True
-
-    def finish_round(self):
-        self._done = [False] * len(self.chunks)
+            _cabi.check(_cabi.lib().mlg_peer_adam_step(
+                g, p, f, a.world, a.rank, self.bucket.n, _cabi.fptr(self.exp_avg), _cabi.fptr(self.exp_avg_sq),
+                _cabi.fptr(self.step_dev), float(self.lr), float(self.betas[0]), float(self.betas[1]), float(self.eps),
+                float(self.wd), float(self.timeout_s), ctypes.c_void_p(self.host_status.data_ptr()), _cabi.stream_ptr()),
+                "mlg_peer_adam_step")
 
 
 def peer_update_available(world, device):
@@ -426,22 +390,11 @@ class Trainer(StaticBatchFeed):
                 raise RuntimeError("peer_update=True but the ranks do not all have CUDA peer access on one box")
             want_peer = False
         if want_peer:
-            # PEER_CHUNKS = 2: two chunks of the fused update: [classifier head] -- 62 % of the gbm parameters, gradients final
-            # right after the head's backward kernel, updated on a forked branch while the rest of backward runs -- and
-            # [everything else].  Default 1: see PEER_CHUNKS.
-            head_ids = {id(p) for n, p in model.named_parameters() if n.startswith("head.")}
-            early = [p for p in self.params if id(p) in head_ids]
-            late = [p for p in self.params if id(p) not in head_ids]
-            segments = [early, late] if (early and late and PEER_CHUNKS >= 2) else [self.params]
             align = 4 * world_size
-            self.early_params = early if len(segments) == 2 else []
-            self.peer = PeerArena(GradBucket.padded_size(segments, align), world_size, dist.get_rank(), dev,
-                                  n_chunks=len(segments))
-            self.bucket = GradBucket(self.params, flat=self.peer.grad, segments=segments, align=align)
+            self.peer = PeerArena(GradBucket.padded_size(self.params, align), world_size, dist.get_rank(), dev)
+            self.bucket = GradBucket(self.params, flat=self.peer.grad, align=align)
         else:
-            self.early_params = []
             self.bucket = GradBucket(self.params)
-        self.params = self.bucket.params          # bucket order (chunks of the fused update first): autograd.grad / store use it
         self.flat = self.bucket.flat
         if self.peer is not None:
             self.opt = PeerAdam(self.bucket, self.peer, lr=args.lr, betas=(args.beta1, args.beta2), weight_decay=args.wd)
@@ -473,32 +426,18 @@ class Trainer(StaticBatchFeed):
         loss = self.loss(batch)
         # == optimizer.zero_grad(); loss.backward() with the gradients landing in the bucket views (p.grad)
         from . import functional as Fn
-        Fn.GRAD_SLOTS_ENABLED = Fn.PARALLEL_ACTIVE = loss.is_cuda
-        Fn.AFTER_HEAD_BACKWARD = self._early_update if (self.peer is not None and self.early_params) else None
+        Fn.GRAD_SLOTS_ENABLED = loss.is_cuda
         try:
             grads = torch.autograd.grad(loss, self.params, allow_unused=True)
         finally:
-            Fn.GRAD_SLOTS_ENABLED = Fn.PARALLEL_ACTIVE = False
-            Fn.AFTER_HEAD_BACKWARD = None
+            Fn.GRAD_SLOTS_ENABLED = False
         self.bucket.store(grads)
         return loss.detach()
-
-    def _early_update(self):
-        """Called by functional.HeadMLP.backward once the classifier head's gradients sit in their bucket slots: launch the
-        head chunk of the fused peer update on a forked stream (joined at the end of the backward pass).  The head's weights
-        are not read again in this step on any rank: every rank signals 'ready' only after its own head backward."""
-        from . import functional as Fn
-        if not all(p._mlg_grad_slot["claimed"] for p in self.early_params):
-            return          # a gradient took the copy path (bucket.store): the chunk runs with the rest, after backward
-        with Fn._Forked(self.flat.device, 3, keep=(), force=True):
-            self.opt.step(0)
 
     def _update(self):
         if self.args.clip_grad:
             torch.nn.utils.clip_grad_norm_(self.params, max_norm=20, norm_type=2)
         self.opt.step()
-        if self.peer is not None:
-            self.opt.finish_round()
 
     def _step_eager(self, batch):
         loss = self._fwd_bwd(batch)

@@ -72,7 +72,7 @@ def test_ctypes_signatures_match_header():
 
 def test_abi_version_and_errors(lib):
     from multilevel_gnn_b200 import _cabi
-    assert lib.mlg_abi_version() == 1
+    assert lib.mlg_abi_version() == 2
     rc = lib.mlg_gen_aggr_fwd(None, None, None, None, None, 4, 8, 0, 1.0, None, 1.0, None, None, 1e-7, 0, None,
                               None, None, None, None)
     assert rc < 0 and "null" in _cabi.last_error()

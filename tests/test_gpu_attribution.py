@@ -96,9 +96,8 @@ def test_input_gradients_full_size_vs_oracle(mlg, cfg, bsz):
         _check(a, c, tag + " g_" + name, rtol=2e-4, atol=1e-5, l2=1e-3, outliers=1e-3)
 
 
-ROUTES = [("factored_off", dict(FACTORED_RANK1=False)), ("factored_gather", dict(FACTORED_RANK1="gather")),
-          ("transform_first_off", dict(TRANSFORM_FIRST=False)), ("act_fusion_off", dict(FUSE_ACT_BACKWARD=False)),
-          ("explicit_x", {})]
+ROUTES = [("factored_off", dict(FACTORED_RANK1=False)), ("transform_first_off", dict(TRANSFORM_FIRST=False)),
+          ("act_fusion_off", dict(FUSE_ACT_BACKWARD=False)), ("explicit_x", {})]
 
 
 @pytest.mark.parametrize("name,flags", ROUTES, ids=[r[0] for r in ROUTES])
@@ -311,9 +310,8 @@ def test_zz_attribution_structure(mlg, monkeypatch):
         torch.cuda.synchronize()
     names = [c[0] for c in rec.calls]
     banned = ("mlg_xty", "mlg_sage_fold_stacked_bwd", "mlg_sage_fold_bwd", "mlg_wcolsum", "mlg_pool_bwd_w",
-              "mlg_pool_bwd_layout", "mlg_sage_rank1_bwd_rows", "mlg_sage_rank1_bwd")
-    assert not [n for n in names if n.startswith(banned) and not n.startswith("mlg_sage_rank1_bwd_xs")
-                and not n.endswith("_supported")], names
+              "mlg_pool_bwd_layout", "mlg_sage_rank1_bwd_rows")
+    assert not [n for n in names if n.startswith(banned) and not n.endswith("_supported")], names
     assert "mlg_sage_rank1_bwd_xs" in names and "mlg_pool_bwd_vm" in names
     for n, a in rec.calls:
         if n == "mlg_head_mlp_bwd":

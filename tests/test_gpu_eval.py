@@ -238,7 +238,7 @@ def test_predict_structure(mlg, monkeypatch):
     called = [c for c, _ in rec.calls]
     assert "mlg_sage_rank1_fwd_rows_nm" in called and "mlg_gather_sum_nm_ex" in called, called
     for name, a in rec.calls:
-        if name in ("mlg_sage_rank1_fwd", "mlg_sage_rank1_fwd_rows", "mlg_sage_rank1_fwd_rows_nm"):
+        if name in ("mlg_sage_rank1_fwd_rows", "mlg_sage_rank1_fwd_rows_nm"):
             assert a[16] is None, "predict asked the first layer for sign-bit words"
     # nothing outlives the call but pred and the pooled buffer pca_feature views
     def block(nbytes):

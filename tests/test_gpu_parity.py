@@ -789,12 +789,13 @@ def test_activation_backward_fusion_is_equivalent(mlg):
 
 
 def test_factored_first_layer_is_equivalent(mlg):
-    """mlg_sage_rank1_fwd/_bwd (first SAGE layer factored through the per-gene tables E_self / E_nbr) against the
-    [x0 | agg] buffer + GEMM path it replaces: prediction, pooled features and every parameter gradient, on the plain
-    and on the activation-unfused chain; and the factored path must be the one that ran."""
+    """mlg_sage_rank1_fwd_rows / _bwd_rows (first SAGE layer factored through the per-gene tables E_self / E_nbr) against
+    the [x0 | agg] buffer + GEMM path it replaces: prediction, pooled features and every parameter gradient, on the plain
+    and on the activation-unfused chain; and the factored path must be the one that ran.  The 32-wide first layer with
+    activation fusion off is the one route that applies LeakyReLU' in a library pass (no sign words at width 32)."""
     from multilevel_gnn_b200 import _cabi, configs, functional as Fn, synth
-    for cfg, fuse in (("gbm", True), ("gbm", False), ("kirc", True)):
-        args = configs.make_args(cfg)
+    for cfg, over, fuse in (("gbm", {}, True), ("gbm", {}, False), ("kirc", {}, True), ("gbm", dict(hidden_channels=32), False)):
+        args = configs.make_args(cfg, **over)
         torch.manual_seed(3)
         model = mlg.MultilevelGNN(args)
         synth.multilevel_params(model)
@@ -803,13 +804,11 @@ def test_factored_first_layer_is_equivalent(mlg):
         b = synth.multilevel_batch(batch_size=5, seed=6).to(DEV)
         params = [p for n, p in model.named_parameters() if p.requires_grad and not n.endswith("lin_l.weight")]
 
-        defaults = (Fn.FACTORED_RANK1, Fn.TRANSFORM_FIRST, Fn.RANK1_SIGN_BITS, Fn.RANK1_FWD_ROWS)
+        defaults = (Fn.FACTORED_RANK1, Fn.TRANSFORM_FIRST)
 
-        def run(factored, tfirst=True, sign_bits=True, fwd_rows=True):
+        def run(factored, tfirst=True):
             Fn.FACTORED_RANK1 = factored
             Fn.TRANSFORM_FIRST = tfirst
-            Fn.RANK1_SIGN_BITS = sign_bits
-            Fn.RANK1_FWD_ROWS = fwd_rows
             type(model).FUSE_ACT_BACKWARD = fuse
             torch.manual_seed(11)                     # same dropout masks
             timer = _cabi.KernelTimer()
@@ -821,23 +820,19 @@ def test_factored_first_layer_is_equivalent(mlg):
                 torch.cuda.synchronize()
             finally:
                 _cabi.TIMER = None
-                Fn.FACTORED_RANK1, Fn.TRANSFORM_FIRST, Fn.RANK1_SIGN_BITS, Fn.RANK1_FWD_ROWS = defaults
+                Fn.FACTORED_RANK1, Fn.TRANSFORM_FIRST = defaults
                 type(model).FUSE_ACT_BACKWARD = True
             return pred.detach(), feat.detach(), g, set(timer.summary())
 
         p0, f0, g0, tags0 = run(False, False)      # [x | agg] buffer + GEMM in both layers
         assert not ({"sage_rank1_fwd", "sage_rank1_bwd"} & tags0), tags0
         names = [n for n, p in model.named_parameters() if p.requires_grad and not n.endswith("lin_l.weight")]
-        # first flag True: backward by target row (mlg_sage_rank1_bwd_rows + segment sum); "gather": by-source gather
-        # (mlg_sage_rank1_bwd).  second: layer 2 (64 -> 32) transform-first (layer 1 then masks its own output gradient).
-        # third: from the forward kernel's sign bits (False: one library activation-backward pass).  fourth: forward with one
-        # warp per gene (False: r01's lane-group kernel)
-        for mode, tfirst, bits, rows in ((True, True, True, True), (True, True, False, True), (True, True, True, False),
-                                         ("gather", True, True, True), (True, False, True, True), (False, True, True, True)):
-            p1, f1, g1, tags1 = run(mode, tfirst, bits, rows)
-            if mode is not False:
-                assert {"sage_rank1_fwd", "sage_rank1_bwd"} <= tags1, tags1
-                assert ("sage_rank1_bwd_seg" in tags1) == (mode is True), (mode, tags1)
+        # first flag: the factored first layer (backward by target row: mlg_sage_rank1_bwd_rows + segment sum).  second:
+        # layer 2 (64 -> 32) transform-first (layer 1 then masks its own output gradient)
+        for mode, tfirst in ((True, True), (True, False), (False, True)):
+            p1, f1, g1, tags1 = run(mode, tfirst)
+            if mode:
+                assert {"sage_rank1_fwd", "sage_rank1_bwd", "sage_rank1_bwd_seg"} <= tags1, tags1
             assert_close(p1, p0, rtol=1e-5, atol=1e-6, what="factored vs buffered pred")
             assert_close(f1, f0, rtol=1e-4, atol=1e-6, what="factored vs buffered pooled features")
             for n, a, c in zip(names, g1, g0):

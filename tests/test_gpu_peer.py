@@ -19,52 +19,47 @@ def mlg():
     return m
 
 
-def _virtual_ranks(mlg, seg_shapes, world, seed, wd):
-    """seg_shapes: list of chunks, each a list of parameter shapes."""
+def _virtual_ranks(mlg, shapes, world, seed, wd):
     from multilevel_gnn_b200.train import GradBucket, PeerAdam, PeerArena
     g = torch.Generator().manual_seed(seed)
-    init = [[torch.randn(s, generator=g) for s in seg] for seg in seg_shapes]
+    init = [torch.randn(s, generator=g) for s in shapes]
     align = 4 * world
     ranks = []
     for r in range(world):
-        segs = [[torch.nn.Parameter(t.clone().to(DEV)) for t in seg] for seg in init]
-        n_pad = GradBucket.padded_size(segs, align)
-        arena = PeerArena(n_pad, world, r, DEV, exchange=False, n_chunks=len(segs))
-        ranks.append([segs, arena])
-    for segs, arena in ranks:
+        params = [torch.nn.Parameter(t.clone().to(DEV)) for t in init]
+        arena = PeerArena(GradBucket.padded_size(params, align), world, r, DEV, exchange=False)
+        ranks.append([params, arena])
+    for params, arena in ranks:
         arena.peer_base = [a.base for _, a in ranks]
     out = []
-    for segs, arena in ranks:
-        params = [p for seg in segs for p in seg]
-        bucket = GradBucket(params, flat=arena.grad, segments=segs, align=align)
+    for params, arena in ranks:
+        bucket = GradBucket(params, flat=arena.grad, align=align)
         opt = PeerAdam(bucket, arena, lr=1e-2, betas=(0.9, 0.999), weight_decay=wd, timeout_s=2.0)
         out.append((params, bucket, opt))
-    return [t for seg in init for t in seg], out, g
+    return init, out, g
 
 
-def _step_all(mlg, ranks, chunk, scratch):
-    """All ranks' update kernels of ``chunk`` as one cooperative launch."""
+def _step_all(mlg, ranks, scratch):
+    """All ranks' update kernels as one cooperative launch."""
     from multilevel_gnn_b200 import _cabi
     L = _cabi.lib()
     opt0 = ranks[0][2]
     world = len(ranks)
-    g, p, f = opt0.arena.pointer_tables(chunk)
-    lo, hi = opt0.chunks[chunk]
+    g, p, f = opt0.arena.pointer_tables()
     arr = ctypes.c_void_p * world
-    m = arr(*[o.exp_avg[chunk].data_ptr() for _, _, o in ranks])
-    v = arr(*[o.exp_avg_sq[chunk].data_ptr() for _, _, o in ranks])
-    t = arr(*[o.step_dev[chunk].data_ptr() for _, _, o in ranks])
-    _cabi.check(L.mlg_peer_adam_step_emulated(g, p, f, world, lo, hi, m, v, t, 1e-2, 0.9, 0.999, 1e-8, float(opt0.wd), 2.0,
-                                              ctypes.c_void_p(scratch.data_ptr()), _cabi.stream_ptr()),
+    m = arr(*[o.exp_avg.data_ptr() for _, _, o in ranks])
+    v = arr(*[o.exp_avg_sq.data_ptr() for _, _, o in ranks])
+    t = arr(*[o.step_dev.data_ptr() for _, _, o in ranks])
+    _cabi.check(L.mlg_peer_adam_step_emulated(g, p, f, world, opt0.bucket.n, m, v, t, 1e-2, 0.9, 0.999, 1e-8, float(opt0.wd),
+                                              2.0, ctypes.c_void_p(scratch.data_ptr()), _cabi.stream_ptr()),
                 "mlg_peer_adam_step_emulated")
 
 
-@pytest.mark.parametrize("world,wd,chunks", [(1, 0.0, 1), (2, 0.0, 1), (3, 0.0, 2), (4, 1e-2, 2)])
-def test_peer_adam_matches_torch_adam(mlg, world, wd, chunks):
+@pytest.mark.parametrize("world,wd", [(1, 0.0), (2, 0.0), (3, 0.0), (4, 1e-2)])
+def test_peer_adam_matches_torch_adam(mlg, world, wd):
     from multilevel_gnn_b200 import _cabi
     shapes = [(257, 33), (1000,), (64, 64), (3,), (50001,)]
-    segs = [shapes] if chunks == 1 else [shapes[:2], shapes[2:]]
-    init, ranks, g = _virtual_ranks(mlg, segs, world, 7 + world, wd)
+    init, ranks, g = _virtual_ranks(mlg, shapes, world, 7 + world, wd)
     ref = [torch.nn.Parameter(t.clone().double()) for t in init]
     ref_opt = torch.optim.Adam(ref, lr=1e-2, betas=(0.9, 0.999), weight_decay=wd)
     scratch = torch.empty(int(_cabi.lib().mlg_peer_emulated_bytes(world)), dtype=torch.uint8, device=DEV)
@@ -75,21 +70,20 @@ def test_peer_adam_matches_torch_adam(mlg, world, wd, chunks):
         ref_opt.step()
         for (params, bucket, opt), gr in zip(ranks, grads):
             bucket.store([x.to(DEV) for x in gr])
-        for c in range(chunks):
-            _step_all(mlg, ranks, c, scratch)
+        _step_all(mlg, ranks, scratch)
         torch.cuda.synchronize()
         assert all(o.arena.status() == 0 for _, _, o in ranks), "a rank timed out waiting for its peers"
     for params, bucket, opt in ranks:
         for p, q, p0 in zip(params, ref, ranks[0][0]):
             assert torch.equal(p.data, p0.data), "replicas must stay bitwise identical"
             torch.testing.assert_close(p.data.cpu().double(), q.data, rtol=2e-5, atol=2e-6)
-        assert all(float(t.item()) == 4.0 for t in opt.step_dev)
+        assert float(opt.step_dev.item()) == 4.0
 
 
 def test_peer_adam_timeout_is_a_hard_failure(mlg):
     """One rank of two never shows up: the waiting rank must give up, leave parameters and optimizer state untouched, set the
     device status of BOTH arenas and the pinned host word, and refuse to run again."""
-    init, ranks, g = _virtual_ranks(mlg, [[(1000,), (77, 3)]], 2, 3, 0.0)
+    init, ranks, g = _virtual_ranks(mlg, [(1000,), (77, 3)], 2, 3, 0.0)
     params, bucket, opt = ranks[0]
     opt.timeout_s = 0.05
     before = [p.data.clone() for p in params]
@@ -99,8 +93,7 @@ def test_peer_adam_timeout_is_a_hard_failure(mlg):
     assert opt.failed() and opt.arena.status() == 1
     assert ranks[1][2].arena.status() == 1, "the failure must be visible in the peer's status word too"
     assert all(torch.equal(p.data, b) for p, b in zip(params, before)), "a failed step must not touch the parameters"
-    assert float(opt.step_dev[0].item()) == 0.0 and float(opt.exp_avg[0].abs().sum()) == 0.0
-    opt.finish_round()
+    assert float(opt.step_dev.item()) == 0.0 and float(opt.exp_avg.abs().sum()) == 0.0
     opt.step()                     # sticky: returns immediately
     torch.cuda.synchronize()
     assert all(torch.equal(p.data, b) for p, b in zip(params, before))
@@ -108,7 +101,7 @@ def test_peer_adam_timeout_is_a_hard_failure(mlg):
 
 def test_peer_adam_in_cuda_graph(mlg):
     """The update kernel replays inside a CUDA graph (device-side step counter and epoch), world = 1."""
-    init, ranks, g = _virtual_ranks(mlg, [[(4096,), (31, 7)]], 1, 3, 0.0)
+    init, ranks, g = _virtual_ranks(mlg, [(4096,), (31, 7)], 1, 3, 0.0)
     params, bucket, opt = ranks[0]
     ref = [torch.nn.Parameter(t.clone().double()) for t in init]
     ref_opt = torch.optim.Adam(ref, lr=1e-2, betas=(0.9, 0.999))
@@ -123,7 +116,6 @@ def test_peer_adam_in_cuda_graph(mlg):
     with torch.cuda.graph(graph):
         bucket.store(static)
         opt.step()
-        opt.finish_round()
     # the capture itself does not run the kernel: three replays = three steps
     for step in range(3):
         gr = [torch.randn(t.shape, generator=g) for t in init]

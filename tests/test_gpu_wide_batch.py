@@ -19,8 +19,8 @@ def mlg():
 
 
 def test_reformulated_layers_with_more_than_32_graphs(mlg):
-    """B = 40 graphs: replica blocks of 32 + 8 in mlg_sage_rank1_bwd_rows, 8-replica chunks with a ragged tail in
-    mlg_sage_rank1_fwd, odd slice sizes in the aggregations -- against the buffered [x | agg] + GEMM path."""
+    """B = 40 graphs: replica blocks of 32 + 8 in mlg_sage_rank1_fwd_rows and mlg_sage_rank1_bwd_rows, odd slice sizes
+    in the aggregations -- against the buffered [x | agg] + GEMM path."""
     from multilevel_gnn_b200 import configs, functional as Fn, synth
     args = configs.make_args("gbm")
     torch.manual_seed(5)

@@ -1,7 +1,7 @@
 """The algebra behind the reformulated SAGE layers, pinned on CPU in fp64 against the oracle restatement of
 SAGEConv.forward (oracle/restated.py::sage_forward, torch_vertex.py:269-294) and its autograd gradients:
 
- * factored first layer (mlg_sage_rank1_fwd / mlg_sage_rank1_bwd_rows): x0[b,n,:] = x[b,n] * emb[n,:] lets the layer run
+ * factored first layer (mlg_sage_rank1_fwd_rows / mlg_sage_rank1_bwd_rows): x0[b,n,:] = x[b,n] * emb[n,:] lets the layer run
    through the per-gene tables E_self = emb W1^T, E_nbr = emb (W2 W_r)^T; backward by TARGET row emits per-entry rows h and
    the self / bias reductions, then a segment sum by source;
  * transform-first layer (mlg_gather_sum_act + one dX GEMM): z = U + mean_j(w_ij V_j), [U | V] = x [W1 ; W2 W_r]^T + [b | 0],

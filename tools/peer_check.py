@@ -32,9 +32,8 @@ def flat_check(dev, world, rank):
     g0 = torch.Generator().manual_seed(5)
     init = [torch.randn(s, generator=g0) for s in shapes]
     params = [torch.nn.Parameter(t.clone().to(dev)) for t in init]
-    segs = [params[:2], params[2:]]                       # two chunks, as the trainer splits head / rest
-    arena = PeerArena(GradBucket.padded_size(segs, 4 * world), world, rank, dev, n_chunks=2)
-    bucket = GradBucket(params, flat=arena.grad, segments=segs, align=4 * world)
+    arena = PeerArena(GradBucket.padded_size(params, 4 * world), world, rank, dev)
+    bucket = GradBucket(params, flat=arena.grad, align=4 * world)
     opt = PeerAdam(bucket, arena, lr=1e-2, betas=(0.9, 0.999), weight_decay=1e-2)
     ref = [torch.nn.Parameter(t.clone().to(dev)) for t in init]
     ref_opt = torch.optim.Adam(ref, lr=1e-2, betas=(0.9, 0.999), weight_decay=1e-2)
@@ -47,9 +46,7 @@ def flat_check(dev, world, rank):
             dist.all_reduce(p.grad, op=dist.ReduceOp.AVG)
         ref_opt.step()
         bucket.store(grads)
-        opt.step(0)               # chunk by chunk, like the trainer's early head chunk
         opt.step()
-        opt.finish_round()
     torch.cuda.synchronize()
     assert arena.status() == 0, "rank %d: a peer wait timed out" % rank
     err = 0.0
@@ -57,7 +54,7 @@ def flat_check(dev, world, rank):
         assert same_on_all_ranks(p.data, world), "replicas differ across ranks"
         torch.testing.assert_close(p.data, q.data, rtol=2e-5, atol=2e-6)
         err = max(err, float((p.data - q.data).abs().max()))
-    assert all(float(t.item()) == 6.0 for t in opt.step_dev) and not opt.failed()
+    assert float(opt.step_dev.item()) == 6.0 and not opt.failed()
     return err
 
 
@@ -89,7 +86,7 @@ def trainer_check(dev, world, rank, graph):
         torch.cuda.synchronize()
         if tr.peer is not None:
             assert tr.peer.status() == 0, "rank %d: a peer wait timed out" % rank
-        ids = {id(p) for p in tr.params}          # model order: the two trainers order their buckets differently
+        ids = {id(p) for p in tr.params}
         flat = torch.cat([p.data.reshape(-1) for p in model.parameters() if id(p) in ids])
         assert same_on_all_ranks(flat, world), "%s: parameters differ across ranks" % mode
         out[mode] = (losses, flat.clone())
