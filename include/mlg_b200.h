@@ -472,6 +472,36 @@ int mlg_attr_accumulate(const float* g, int64_t ld_g, const float* w, const int3
                         int accumulate, float* acc, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Knockout screen, incremental trunk (csrc/knockout.cu).  Work item r = (patient b = item_b[r], group k = item_k[r]) sets
+ * the values of the nodes of group k (g_nodes[g_ptr[k] .. g_ptr[k+1])) to baseline[node] and writes the pooled features
+ * of that input to out[r] [S, P, 32] (channel-last, mlg_pool_fwd's layout); k < 0 copies patient b's base row.  Only the
+ * rows the group reaches are recomputed, each with the base AND the knocked-out values in the same thread:
+ *   T1 (t1_nodes, sorted): the first-layer rows whose CSR entries read a node of the group, the group included;
+ *     z1 = xs_i E_self[i] + inv_cnt_i sum_j w_ij xs_j E_nbr[j] + b1, LeakyReLU(slope1), [U | V] = y1 Wst2^T + b2;
+ *   T2 (t2_nodes, sorted): the second-layer rows that read a T1 row; y2 = LeakyReLU(slope2)(U_i + inv_cnt_i sum_j w_ij V_j),
+ *     U / V from the T1 rows where the node is in T1, else the forward's base row uv[i * B + b] (node-major [N*B, 64]);
+ *   pool: out = pooled[b] + sum over the slots of T2 nodes, per touched segment s_seg (sorted, per group s_ptr), of
+ *     (y2' x'_i - y2 x_i) w_pool[slot, p], entries e_ptr[q] .. e_ptr[q+1] in slot order: (e_slot = slot, e_t2 = the
+ *     node's position in the group's T2 list).  Missing slots (no node) are not listed: they add nothing.
+ * xs [B, N] node values (graph-major); e12 [N, ld_e12] = [E_self | E_nbr] (64 + 64 columns, the factored first layer's
+ * per-gene tables); b1 [64] or NULL; wst2 [64, 64] the second layer's stacked weight [W1 ; W2 W_r] from
+ * mlg_sage_fold_stacked_fwd, b2 [64] = [b | 0] or NULL; rowptr / col / val the forward CSR with the rewritten self loops
+ * (val NULL: weight 1); w_pool [G, P] = learnable_pca_params * info_mask; pooled [B, S, P, 32] the forward's pooled
+ * tensor.  Widths are fixed at 64 -> 32 (the shipped configs), 1 <= P <= 8, rows <= 65535.  The workspace holds
+ * rows * max_t1 [U | V] row pairs and rows * max_t2 value-mask differences (mlg_knockout_workspace_bytes).  No atomics;
+ * every sum has a fixed order: an item's output has the same bits whatever its row and the other items, a group whose
+ * values equal the baseline reproduces pooled[b] bitwise, and untouched segments are copies. */
+int64_t mlg_knockout_workspace_bytes(int64_t rows, int64_t max_t1, int64_t max_t2);
+int mlg_knockout_trunk(const float* xs, const float* baseline, int64_t N, int64_t B, const float* e12, int64_t ld_e12,
+                       const float* b1, float slope1, const float* wst2, const float* b2, const float* uv, float slope2,
+                       const int32_t* rowptr, const int32_t* col, const float* val, const float* w_pool, const float* pooled,
+                       int64_t S, int64_t P, const int32_t* g_ptr, const int32_t* g_nodes, const int32_t* t1_ptr,
+                       const int32_t* t1_nodes, const int32_t* t2_ptr, const int32_t* t2_nodes, const int32_t* s_ptr,
+                       const int32_t* s_seg, const int32_t* e_ptr, const int32_t* e_slot, const int32_t* e_t2,
+                       const int64_t* item_b, const int64_t* item_k, int64_t rows, int64_t max_t1, int64_t max_t2,
+                       void* workspace, int64_t workspace_bytes, float* out, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Gene -> pathway pool (models/multilevel_gnn.py:205-239): value mask, gather by gene_pca_match,
  * missing-gene mask, per-gene projection, segment sum -- without materialising [B,C,G,P].
  *     out[b,c,s,p] = sum_{g in seg(b,s)} vm[node] * x[node, c] * w[g,p],  node = b*N + match[b,g] (skipped if < 0)

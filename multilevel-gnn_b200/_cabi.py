@@ -126,6 +126,14 @@ _SIGNATURES = {
     "mlg_sage_rank1_bwd_xs": (_c_int, [_c_vp, _c_i64, _c_int, _c_vp, _c_vp, _c_f32, _c_vp, _c_i64, _c_vp, _c_i64, _c_vp, _c_vp,
                                        _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_vp, _c_vp, _c_i64, _c_vp]),
     "mlg_attr_accumulate": (_c_int, [_c_vp, _c_i64, _c_vp, _c_vp, _c_i64, _c_i64, _c_int, _c_vp, _c_vp]),
+    "mlg_knockout_workspace_bytes": (_c_i64, [_c_i64, _c_i64, _c_i64]),
+    # (xs, baseline, N, B, e12, ld_e12, b1, slope1, wst2, b2, uv, slope2, rowptr, col, val, w_pool, pooled, S, P, g_ptr, g_nodes,
+    #  t1_ptr, t1_nodes, t2_ptr, t2_nodes, s_ptr, s_seg, e_ptr, e_slot, e_t2, item_b, item_k, rows, max_t1, max_t2, workspace,
+    #  workspace_bytes, out, stream)
+    "mlg_knockout_trunk": (_c_int, [_c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_i64, _c_vp, _c_f32, _c_vp, _c_vp, _c_vp, _c_f32,
+                                    _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp,
+                                    _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_vp, _c_i64,
+                                    _c_vp, _c_vp]),
     "mlg_pool_fwd": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64,
                               _c_i64, _c_int, _c_vp, _c_vp]),
     "mlg_pool_bwd_x": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64,
@@ -204,7 +212,8 @@ def last_error():
 
 # kernels launched per C call (own kernels only; CUB's sort passes inside mlg_csr_build are not counted)
 _LAUNCHES_PER_CALL = {"mlg_csr_build": 2, "mlg_knn_graph": 2, "mlg_xty": 2, "mlg_xty_tc": 2, "mlg_skinny_linear": 2, "mlg_wcolsum": 2, "mlg_gen_aggr_bwd_affine": 3, "mlg_gen_aggr_bwd_affine_src": 3, "mlg_layernorm_bwd": 2, "mlg_layernorm_relu_bwd": 2, "mlg_pool_bwd": 2, "mlg_pool_bwd_layout": 2, "mlg_adam_step": 2,
-                      "mlg_head_conv_pool_bwd": 2, "mlg_head_mlp_fwd": 2, "mlg_diffpool_bwd": 2, "mlg_pca_indep_loss": 2}
+                      "mlg_head_conv_pool_bwd": 2, "mlg_head_mlp_fwd": 2, "mlg_diffpool_bwd": 2, "mlg_pca_indep_loss": 2,
+                      "mlg_knockout_trunk": 4}
 LAUNCH_COUNT = 0
 TIMER = None        # a KernelTimer while bench.py measures per-kernel device time
 

@@ -13,13 +13,12 @@ batch), with one host synchronisation per call.
     res = attr.attribute(dataset, topo)        # records with x / y / age, as Evaluator.evaluate
     res.nodes [n, N]; res.genes [n, 5135, 3]; res.pathways [n, 146, 3]; res.pred [n, 2]; res.delta [n]
 """
-import contextlib
 from collections import namedtuple
 
 import torch
 
 from . import _cabi
-from .train import StaticBatchFeed
+from .train import StaticBatchFeed, frozen_parameters
 
 METHODS = ("saliency", "input_x_gradient", "integrated_gradients")
 
@@ -153,7 +152,7 @@ class Attributor(StaticBatchFeed):
         self.alpha = torch.ones(B, dtype=torch.float32, device=dev)
         self._base = (torch.zeros(n_nodes, dtype=torch.float32, device=dev) if self.baseline is None
                       else self.baseline.to(dev).reshape(n_nodes).clone())
-        with self._frozen():
+        with frozen_parameters(self.model, grad_enabled=True):
             cur = torch.cuda.current_stream()
             side = torch.cuda.Stream()
             side.wait_stream(cur)
@@ -168,28 +167,10 @@ class Attributor(StaticBatchFeed):
         self._ptrs = self._param_ptrs()
         return self
 
-    @contextlib.contextmanager
-    def _frozen(self):
-        """Eval mode, grad mode on, every parameter frozen (no weight-gradient work, no .grad); all restored on exit."""
-        params = list(self.model.parameters())
-        flags = [p.requires_grad for p in params]
-        was_training, was_grad = self.model.training, torch.is_grad_enabled()
-        try:
-            for p in params:
-                p.requires_grad_(False)
-            self.model.train(False)
-            torch.set_grad_enabled(True)
-            yield
-        finally:
-            for p, f in zip(params, flags):
-                p.requires_grad_(f)
-            self.model.train(was_training)
-            torch.set_grad_enabled(was_grad)
-
     def eager(self):
         """One uncaptured pass of what a replay runs, on the static buffers (same kernels, launched from the host); the
         outputs land in ``out_g`` / ``out_pw`` / ``out_pred`` as after a replay."""
-        with self._frozen():
+        with frozen_parameters(self.model, grad_enabled=True):
             self._replay_body()
 
     def _step_fields(self, host_batch):

@@ -525,6 +525,10 @@ FACTORED_RANK1 = True
 # SAGE layers with out_channels < in_channels evaluated transform-first (gather on the narrower rows); False: [x | agg] + GEMM
 TRANSFORM_FIRST = True
 H1_NODE_MAJOR = True     # the factored first layer writes its output node-major for a transform-first consumer (and takes its gradient so)
+# None, or a dict into which SageLayer.forward puts the tensors of its factored / transform-first route that a knockout screen
+# starts from ("rank1": topology, [E_self | E_nbr], bias, slope; "tfirst": topology, [U | V], Wst, [b | 0], slope, node-major
+# flag).  Set by knockout.Knockout around its own forward only; nothing is computed or launched for it.
+KEEP_STATE = None
 
 
 class SageLayer(torch.autograd.Function):
@@ -628,6 +632,8 @@ class SageLayer(torch.autograd.Function):
                         _cabi.iptr(topo.fwd_order, True), n1, cout, topo.replicas,
                         _cabi.fptr(bias, True), float(slope), _cabi.fptr(y), cout, _cabi.lptr(mbits, True),
                         _cabi.stream_ptr()), "mlg_sage_rank1_fwd_rows")
+            if KEEP_STATE is not None:
+                KEEP_STATE["rank1"] = (topo, e12, bias, float(slope))
             ctx.xs_t = xs_t
             ctx.mbits = mbits
             ctx.h1_nm = h1_nm
@@ -649,6 +655,8 @@ class SageLayer(torch.autograd.Function):
             # [U | V] = x [W1 ; W2 W_r]^T + [b | 0]: the gather (the L2-bandwidth-bound step) runs on cout-wide rows instead of
             # cin-wide ones, forward and backward, and no [x | agg] buffer is written.
             uv = tall_matmul(xd, wst, bias2, tag="sage_update_gemm", w_split=wst_split)     # [n, 2cout] = [U | V]
+            if KEEP_STATE is not None:
+                KEEP_STATE["tfirst"] = (topo, uv, wst, bias2, float(slope), x_nm)
             csr = topo.fwd
             if x_nm:
                 # x came node-major, so [U | V] is: one contiguous block of V rows per CSR entry; y goes out graph-major

@@ -225,12 +225,19 @@ class MultilevelGNN(nn.Module):
 
     def forward(self, input_batch, x=None, gene_pca_match=None, raw_indice=None, age=None, require_grad=True,
                 _loss_args=None, _fused=False):
-        args = self.args
-        loss_args = _loss_args
         with torch.enable_grad() if require_grad else torch.no_grad():
             if x is None:
                 age = input_batch.age
             x = self.pool_genes(input_batch, x, gene_pca_match, raw_indice, value_mask=True, fused=_fused)     # [B, C, 438, P]
+        return self.post_pool(x, age, require_grad, _loss_args)
+
+    def post_pool(self, x, age, require_grad=True, _loss_args=None):
+        """The part of ``forward`` after the gene -> pathway pool: ``x`` the pooled tensor [B, C, 438, P] (as ``pool_genes``
+        returns it), ``age`` [B] -> ``(pred, pca_feature)``.  The reshape to [B, C, 146, 3P] and the pathway reorder run under
+        the grad mode ``require_grad`` selects, the head under the caller's."""
+        args = self.args
+        loss_args = _loss_args
+        with torch.enable_grad() if require_grad else torch.no_grad():
             x = x.reshape(x.shape[0], x.shape[1], 146, self.pca_dim * 3)
             if args.reorder_pathway and self.reorder_idxs is not None:
                 x = x[:, :, self.reorder_idxs.to(x.device), :]

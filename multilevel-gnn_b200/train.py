@@ -8,6 +8,7 @@ over the flat fp32 gradient bucket followed by a replicated flat Adam.  Paramete
 gradient (``lin_l.weight`` of every SAGEConv, ``info_mask``) are left out of the bucket and of the
 optimizer state.
 """
+import contextlib
 from typing import NamedTuple, Optional
 
 import torch
@@ -261,6 +262,26 @@ class _PendingLoss:
         if float(self.slot[1]) != 0.0:
             raise RuntimeError("Trainer: a batch uploaded after capture() carried a different topology than the captured graph")
         return float(self.slot[0])
+
+
+@contextlib.contextmanager
+def frozen_parameters(model, grad_enabled):
+    """Eval mode, every parameter frozen (no weight-gradient work, no .grad) and the grad mode set to ``grad_enabled``; all
+    restored on exit.  The attribution and knockout graphs are recorded under it: they read the parameters in place."""
+    params = list(model.parameters())
+    flags = [p.requires_grad for p in params]
+    was_training, was_grad = model.training, torch.is_grad_enabled()
+    try:
+        for p in params:
+            p.requires_grad_(False)
+        model.train(False)
+        torch.set_grad_enabled(grad_enabled)
+        yield
+    finally:
+        for p, f in zip(params, flags):
+            p.requires_grad_(f)
+        model.train(was_training)
+        torch.set_grad_enabled(was_grad)
 
 
 class StaticBatchFeed:
