@@ -471,6 +471,23 @@ int mlg_sage_rank1_bwd_xs(const float* gz, int64_t ld_g, int gz_node_major, cons
 int mlg_attr_accumulate(const float* g, int64_t ld_g, const float* w, const int32_t* slot_ptr, int64_t n_out, int64_t N,
                         int accumulate, float* acc, void* stream);
 
+/* Expected gradients against a background bank [M, N] (csrc/expected_grad.cu).  Slot s of a replay holds one draw: a bank
+ * row j[s] (int32 [B]) and alpha[s] (fp32 [B]).  x [B, N] is the static batch of node values (graph-major).
+ * mlg_attr_eg_interp: the interpolant the forward reads,
+ *     out[s, c] = fmaf(alpha[s], x[s, c], (1 - alpha[s]) * bank[j[s], c])     (fp32, in this order)
+ *   alpha = 1 gives x and alpha = 0 the bank row, bitwise.  Capturable, no allocation.
+ * mlg_attr_eg_accumulate: acc[p, c] = (accumulate ? acc[p, c] : 0) +
+ *       sum_{s = slot_ptr[p]}^{slot_ptr[p+1]-1} w[s] * (x[s, c] - bank[j[s], c]) * g[s, c]      (slots in order)
+ *   g [slots, N] the per-slot gradients, acc [n_out, N], slot_ptr int32 [n_out + 1]; one fixed-order sum per element, no
+ *   atomics.  As mlg_attr_accumulate with the difference x - x' formed in the same pass.
+ * B and n_out <= 65535.  A j[s] outside [0, M) is never read: the affected elements become NaN and *bad (int32, device) is set to 1, never
+ * cleared by these calls -- the caller zeroes it and reads it back at its next synchronisation. */
+int mlg_attr_eg_interp(const float* x, const float* bank, int64_t M, const int32_t* j, const float* alpha, int64_t B,
+                       int64_t N, float* out, int32_t* bad, void* stream);
+int mlg_attr_eg_accumulate(const float* g, const float* x, const float* bank, int64_t M, const int32_t* j, const float* w,
+                           const int32_t* slot_ptr, int64_t n_out, int64_t N, int accumulate, float* acc, int32_t* bad,
+                           void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Knockout screen, incremental trunk (csrc/knockout.cu).  Work item r = (patient b = item_b[r], group k = item_k[r]) sets
  * the values of the nodes of group k (g_nodes[g_ptr[k] .. g_ptr[k+1])) to baseline[node] and writes the pooled features

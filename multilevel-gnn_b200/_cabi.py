@@ -126,6 +126,11 @@ _SIGNATURES = {
     "mlg_sage_rank1_bwd_xs": (_c_int, [_c_vp, _c_i64, _c_int, _c_vp, _c_vp, _c_f32, _c_vp, _c_i64, _c_vp, _c_i64, _c_vp, _c_vp,
                                        _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_vp, _c_vp, _c_i64, _c_vp]),
     "mlg_attr_accumulate": (_c_int, [_c_vp, _c_i64, _c_vp, _c_vp, _c_i64, _c_i64, _c_int, _c_vp, _c_vp]),
+    # (x, bank, M, j, alpha, B, N, out, bad, stream)
+    "mlg_attr_eg_interp": (_c_int, [_c_vp, _c_vp, _c_i64, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp]),
+    # (g, x, bank, M, j, w, slot_ptr, n_out, N, accumulate, acc, bad, stream)
+    "mlg_attr_eg_accumulate": (_c_int, [_c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_int, _c_vp, _c_vp,
+                                        _c_vp]),
     "mlg_knockout_workspace_bytes": (_c_i64, [_c_i64, _c_i64, _c_i64]),
     # (xs, baseline, N, B, e12, ld_e12, b1, slope1, wst2, b2, uv, slope2, rowptr, col, val, w_pool, pooled, S, P, g_ptr, g_nodes,
     #  t1_ptr, t1_nodes, t2_ptr, t2_nodes, s_ptr, s_seg, e_ptr, e_slot, e_t2, item_b, item_k, rows, max_t1, max_t2, workspace,

@@ -1,9 +1,9 @@
 """Gene and pathway attribution for MultilevelGNN on the B200 kernels.
 
 ``Attributor`` answers "which genes and pathways drove this patient's prediction" with the gradient of the predicted class
-probability with respect to the patient's omics values (``batch.x``): saliency, input x gradient, or integrated gradients
-(IG).  IG for one patient evaluates ``points`` interpolants of that patient, all on the same gene network: one
-replicated-topology batch.  ``capture`` records the forward and the input-only backward (no weight-gradient kernel runs) as
+probability with respect to the patient's omics values (``batch.x``): saliency, input x gradient, integrated gradients
+(IG), or expected gradients (IG averaged over a background cohort: SHAP-style values).  IG for one patient evaluates
+``points`` interpolants of that patient, all on the same gene network: one replicated-topology batch.  ``capture`` records the forward and the input-only backward (no weight-gradient kernel runs) as
 ONE CUDA graph with its own memory pool; ``attribute`` replays it over a plan of patient slots and accumulates per-patient
 results on the device (mlg_attr_accumulate: slot order fixed, so a patient's result has the same bits in any slot and any
 batch), with one host synchronisation per call.
@@ -12,6 +12,8 @@ batch), with one host synchronisation per call.
     attr.capture(device_batch)                 # keyed batch, as Evaluator.capture
     res = attr.attribute(dataset, topo)        # records with x / y / age, as Evaluator.evaluate
     res.nodes [n, N]; res.genes [n, 5135, 3]; res.pathways [n, 146, 3]; res.pred [n, 2]; res.delta [n]
+
+    attr = Attributor(model, args, batch_size=32, method="expected_gradients", background=train_x, samples=32, seed=0)
 """
 from collections import namedtuple
 
@@ -20,7 +22,7 @@ import torch
 from . import _cabi
 from .train import StaticBatchFeed, frozen_parameters
 
-METHODS = ("saliency", "input_x_gradient", "integrated_gradients")
+METHODS = ("saliency", "input_x_gradient", "integrated_gradients", "expected_gradients")
 
 AttributionResult = namedtuple("AttributionResult", "nodes genes pathways pred delta")
 
@@ -61,6 +63,50 @@ def slot_plan(n, batch_size, per_patient):
     return plan
 
 
+_M64 = (1 << 64) - 1
+_GOLDEN = 0x9E3779B97F4A7C15
+
+
+def _mix64(z):
+    """splitmix64's output function (Steele, Lea and Flood, OOPSLA 2014) of a 64-bit state."""
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & _M64
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & _M64
+    return z ^ (z >> 31)
+
+
+def eg_draws(seed, index, S, M):
+    """Expected gradients' draws for the patient at position ``index`` of the dataset: (j [S] int64 in [0, M), alpha [S]
+    float64 in (0, 1)).  A pure function of (seed, index, S, M), so a patient's draws do not depend on batch_size, on the
+    other patients or on call order.  Draw k is the k-th output of a splitmix64 stream keyed by (seed, index): counter
+    based, computed directly.  j = (high 32 bits * M) >> 32; alpha = (u + 0.5) * 2^-23 with u the low 23 bits: the midpoints
+    of 2^23 equal bins, each exact in fp32."""
+    if S < 1 or M < 1 or index < 0:
+        raise ValueError("eg_draws: needs S >= 1, M >= 1 and index >= 0")
+    key = _mix64(((_mix64((seed + _GOLDEN) & _M64) ^ index) + _GOLDEN) & _M64)
+    j, alpha = [], []
+    for k in range(S):
+        h = _mix64((key + (k + 1) * _GOLDEN) & _M64)
+        j.append(((h >> 32) * M) >> 32)
+        alpha.append(((h & 0x7FFFFF) + 0.5) * 2.0 ** -23)
+    return torch.tensor(j, dtype=torch.int64), torch.tensor(alpha, dtype=torch.float64)
+
+
+def eg_plan(j, alpha, batch_size, completeness):
+    """Sample pass of expected gradients for n patients with draws j, alpha [n, S]: slot_plan over S slots per patient (2S
+    with ``completeness``).  Slot k < S holds draw k with weight 1 / S; slot S + k holds draw k at alpha = 0 with weight 0,
+    and its prediction F(x'_{j_k}) (at the patient's age) is kept at position patient * S + k (-1: not kept).  Returns per
+    replay (slots [s, 2] of (patient, k), j [s], alpha [s], w [s], f0 position [s])."""
+    n, S = j.shape
+    out = []
+    for slots in slot_plan(n, batch_size, 2 * S if completeness else S):
+        p, k = slots[:, 0], slots[:, 1]
+        draw = k % S
+        sample = k < S
+        out.append((slots, j[p, draw], torch.where(sample, alpha[p, draw], torch.zeros((), dtype=alpha.dtype)),
+                    sample.double() / S, torch.where(sample, torch.full_like(k, -1), p * S + draw)))
+    return out
+
+
 def gene_view(nodes):
     """[n, N] per-node values -> [n, N // 3, 3] per (gene, omic): gene g owns nodes 3g, 3g + 1, 3g + 2."""
     return nodes.reshape(nodes.shape[0], -1, 3)
@@ -89,14 +135,45 @@ class Attributor(StaticBatchFeed):
     the patient's value and not attributed.  Pathway attributions are gradient x activation at the pooled features at
     alpha = 1, per (pathway, omic) in the reference's pathway order.
 
+    "expected_gradients" measures the patient against a cohort instead of one reference profile:
+        phi_i(x) = E_{x' ~ background, alpha ~ U(0,1)} [(x_i - x'_i) dF/dx_i (x' + alpha (x - x'))],
+        sum_i phi_i(x) = F(x) - E_{x'} F(x')   (in expectation),
+    estimated from ``samples`` = S draws (j_k, alpha_k) per patient (``eg_draws``: a function of ``seed`` and the patient's
+    position in the dataset only, so a patient's result has the same bits in any batch or slot).  background: [M, N]
+    reference profiles, e.g. the training split's x.  A sample pass replays S interpolants per patient (x' = background[j_k])
+    and sums (x - x'_{j_k}) * g_k / S on the device (mlg_attr_eg_accumulate); a pass at alpha = 1 supplies ``pred`` and the
+    pathway attributions.  The pathway attributions are the same gradient x activation at alpha = 1 as for the other methods,
+    not a cohort-relative SHAP value of the pathway.  With ``completeness`` each patient also gets S slots at alpha = 0
+    (F(x'_{j_k}) at the patient's own age), and ``delta`` = F(x) - mean_k F(x'_{j_k}) - sum_i phi_i, the sampled
+    completeness gap: zero in expectation over alpha given the drawn j.  Without it, ``delta`` is None.
+
     Eval semantics (no dropout) on the fused training-forward route.  The parameters are read in place and receive no
     gradient: they are frozen while the graph is captured (requires_grad, the model's mode and the grad mode are restored
     afterwards), so the graph holds no weight-gradient kernel and writes no ``.grad``; if their storage moved since capture
     (e.g. a Trainer re-homed them), ``attribute`` re-captures first."""
 
-    def __init__(self, model, args, batch_size=32, method="integrated_gradients", points=32, target=1, baseline=None):
+    def __init__(self, model, args, batch_size=32, method="integrated_gradients", points=32, target=1, baseline=None,
+                 background=None, samples=32, seed=0, completeness=False):
         if method not in METHODS:
             raise ValueError("Attributor: method must be one of %s (got %r)" % (METHODS, method))
+        self.background = None
+        if method == "expected_gradients":
+            if background is None:
+                raise ValueError("Attributor: expected_gradients needs a background [M, N] of reference profiles")
+            if baseline is not None:
+                raise ValueError("Attributor: expected_gradients takes a background, not a baseline")
+            bg = torch.as_tensor(background).detach().to("cpu", torch.float32, copy=True)
+            n_nodes = 3 * model.node_num
+            if bg.dim() != 2 or bg.shape[0] < 1 or bg.shape[1] != n_nodes:
+                raise ValueError("Attributor: background must be [M >= 1, %d] (got %s)" % (n_nodes, tuple(bg.shape)))
+            if not bool(torch.isfinite(bg).all()):
+                raise ValueError("Attributor: background values must be finite")
+            if int(samples) < 1:
+                raise ValueError("Attributor: samples must be >= 1 (got %d)" % int(samples))
+            self.background = bg.contiguous()
+        elif background is not None:
+            raise ValueError("Attributor: background is only used by expected_gradients (method %r)" % method)
+        self.samples, self.seed, self.completeness = int(samples), int(seed), bool(completeness)
         self.model, self.args = model, args
         self.batch_size = int(batch_size)
         if not 1 <= self.batch_size <= 64:
@@ -122,6 +199,12 @@ class Attributor(StaticBatchFeed):
         if self.method == "integrated_gradients":
             a = self.alpha.view(B, 1)
             xin = torch.addcmul(self._base * (1.0 - a), a, xs)      # alpha * x + (1 - alpha) * x': exact at both ends
+        elif self.method == "expected_gradients":
+            xin = torch.empty_like(xs)
+            _cabi.check(_cabi.lib().mlg_attr_eg_interp(_cabi.fptr(xs), _cabi.fptr(self._bank), self._bank.shape[0],
+                                                       _cabi.iptr(self.j), _cabi.fptr(self.alpha), B, xs.shape[1],
+                                                       _cabi.fptr(xin), _cabi.iptr(self._bad), _cabi.stream_ptr()),
+                        "mlg_attr_eg_interp")
         else:
             xin = xs.clone()
         xin.requires_grad_(True)
@@ -152,6 +235,13 @@ class Attributor(StaticBatchFeed):
         self.alpha = torch.ones(B, dtype=torch.float32, device=dev)
         self._base = (torch.zeros(n_nodes, dtype=torch.float32, device=dev) if self.baseline is None
                       else self.baseline.to(dev).reshape(n_nodes).clone())
+        if self.method == "expected_gradients":
+            if self.background.shape[1] != n_nodes:
+                raise ValueError("Attributor.capture: the background has %d nodes, the batch %d"
+                                 % (self.background.shape[1], n_nodes))
+            self._bank = self.background.to(dev, copy=True)
+            self.j = torch.zeros(B, dtype=torch.int32, device=dev)
+            self._bad = torch.zeros(1, dtype=torch.int32, device=dev)
         with frozen_parameters(self.model, grad_enabled=True):
             cur = torch.cuda.current_stream()
             side = torch.cuda.Stream()
@@ -214,10 +304,38 @@ class Attributor(StaticBatchFeed):
                                                     _cabi.iptr(ptr), n_out, N, 0 if fresh else 1, _cabi.fptr(acc),
                                                     _cabi.stream_ptr()), "mlg_attr_accumulate")
 
+    def _replays(self, dataset, topo, plan, before, after):
+        """One replay per entry of ``plan`` on its slots' records, collated on the host and staged on a side stream while
+        the device works; ``before(s)`` sets replay s's per-slot inputs, ``after(s)`` consumes its outputs."""
+        from .data import collate
+
+        def host(s):
+            return collate([dataset[int(p)] for p in plan[s][:, 0]], topo)
+
+        nxt = host(0)
+        self.prefetch(nxt)
+        for s in range(len(plan)):
+            nxt_s = host(s + 1) if s + 1 < len(plan) else None      # collated on the host while the device works
+            self._take_staged()
+            before(s)
+            self.graph.replay()
+            after(s)
+            if nxt_s is not None:
+                self.prefetch(nxt_s)
+
+    def _pathways(self, host_pw, n):
+        """[n, S3] summed pooled contributions -> [n, 146, 3] in the reference's pathway order."""
+        reorder = self.model.reorder_idxs if (self.args.reorder_pathway and self.model.reorder_idxs is not None) else None
+        pathways = host_pw.view(n, host_pw.shape[1] // 3, 3)
+        if reorder is not None:
+            out = torch.empty_like(pathways)
+            out[:, reorder] = pathways
+            pathways = out
+        return pathways
+
     def attribute(self, dataset, topo):
         """Attributions of every record of ``dataset`` (records with x / y / age, as data.collate takes them; ``topo`` the
         dataset's FoldTopology) -> AttributionResult of host tensors, in dataset order."""
-        from .data import collate
         if self.graph is None:
             raise RuntimeError("Attributor: call capture(batch) first")
         want = "%s-b%d" % (topo.key, self.batch_size)
@@ -229,6 +347,8 @@ class Attributor(StaticBatchFeed):
         n = len(dataset)
         if n == 0:
             raise ValueError("Attributor: empty dataset")
+        if self.method == "expected_gradients":
+            return self._expected_gradients(dataset, topo)
         B = self.batch_size
         plan = slot_plan(n, B, self.points)
         dev = self.out_g.device
@@ -241,25 +361,19 @@ class Attributor(StaticBatchFeed):
         f0 = torch.empty(n, 1, dtype=torch.float32, device=dev)
         xs = torch.empty(n, N, dtype=torch.float32, device=dev)
 
-        def host(s):
-            return collate([dataset[int(p)] for p in plan[s][:, 0]], topo)
-
-        nxt = host(0)
-        self.prefetch(nxt)
-        for s in range(len(plan)):
-            nxt_s = host(s + 1) if s + 1 < len(plan) else None      # collated on the host while the device works
-            self._take_staged()
-            first, cnt, fresh = meta[s]
+        def before(s):
             self.alpha.copy_(tab[s, 0])
-            self.graph.replay()
+
+        def after(s):
+            first, cnt, fresh = meta[s]
             L = slice(first, first + cnt)
             self._accumulate(self.out_g, N, tab[s, 1], ptrs[s], cnt, N, fresh, acc[L])
             self._accumulate(self.out_pw, S3, tab[s, 2], ptrs[s], cnt, S3, fresh, pw[L])
             self._accumulate(self.out_pred, 2, tab[s, 2], ptrs[s], cnt, 2, fresh, pred[L])
             self._accumulate(self.out_pred[:, self.target:], 2, tab[s, 3], ptrs[s], cnt, 1, fresh, f0[L])
             self._accumulate(self.static_batch.x.view(B, N), N, tab[s, 2], ptrs[s], cnt, N, fresh, xs[L])
-            if nxt_s is not None:
-                self.prefetch(nxt_s)
+
+        self._replays(dataset, topo, plan, before, after)
         if self.method == "saliency":
             nodes = acc
         elif self.method == "input_x_gradient":
@@ -267,16 +381,85 @@ class Attributor(StaticBatchFeed):
         else:
             nodes = (xs - self._base) * acc
         host_nodes, host_pw, host_pred, host_f0 = (t.cpu() for t in (nodes, pw, pred, f0))     # the one synchronisation
-        reorder = self.model.reorder_idxs if (self.args.reorder_pathway and self.model.reorder_idxs is not None) else None
-        pathways = host_pw.view(n, S3 // 3, 3)
-        if reorder is not None:
-            out = torch.empty_like(pathways)
-            out[:, reorder] = pathways
-            pathways = out
         delta = None
         if self.method == "integrated_gradients":
             delta = (host_pred[:, self.target].double() - host_f0[:, 0].double() - host_nodes.double().sum(1)).float()
-        return AttributionResult(host_nodes, gene_view(host_nodes), pathways, host_pred, delta)
+        return AttributionResult(host_nodes, gene_view(host_nodes), self._pathways(host_pw, n), host_pred, delta)
+
+    def _eg_device_plan(self, rows, dev, dummy):
+        """Sample pass tables per replay (eg_plan rows): alpha and weights [2, B] fp32, bank rows and slot pointers [2B + 1]
+        int32, F(x'_j) destinations [B] int64 (``dummy`` for slots whose prediction is not kept); one upload each."""
+        B = self.batch_size
+        ft, it, dst, meta = [], [], [], []
+        for slots, j, alpha, w, pos in rows:
+            m = slots.shape[0]
+            f = torch.zeros(2, B)
+            f[0, :m], f[1, :m] = alpha.float(), w.float()
+            i = torch.zeros(2 * B + 1, dtype=torch.int32)
+            i[:m] = j.to(torch.int32)
+            pat = slots[:, 0]
+            first = int(pat[0])
+            counts = torch.bincount(pat - first)
+            i[B + 1:B + 1 + counts.numel()] = torch.cumsum(counts, 0).to(torch.int32)
+            d = torch.full((B,), dummy, dtype=torch.int64)
+            d[:m] = torch.where(pos < 0, torch.full_like(pos, dummy), pos)
+            ft.append(f), it.append(i), dst.append(d)
+            meta.append((first, counts.numel(), bool(slots[0, 1] == 0), bool((w > 0).any()), bool((pos >= 0).any())))
+        up = [torch.stack(t).pin_memory().to(dev, non_blocking=True) for t in (ft, it, dst)]
+        return up[0], up[1], up[2], meta
+
+    def _expected_gradients(self, dataset, topo):
+        n, B, S = len(dataset), self.batch_size, self.samples
+        M = self._bank.shape[0]
+        dev = self.out_g.device
+        N = self.out_g.shape[1]
+        S3 = self.out_pw.shape[1]
+        draws = [eg_draws(self.seed, i, S, M) for i in range(n)]
+        rows = eg_plan(torch.stack([d[0] for d in draws]), torch.stack([d[1] for d in draws]), B, self.completeness)
+        ftab, itab, dst, meta = self._eg_device_plan(rows, dev, n * S)
+        plan1 = slot_plan(n, B, 1)
+        tab, ptrs, meta1 = self._device_plan(plan1, dev)
+        acc = torch.empty(n, N, dtype=torch.float32, device=dev)
+        f0 = torch.zeros(n * S + 1, dtype=torch.float32, device=dev)       # last entry: the slots whose value is not kept
+        pw = torch.empty(n, S3, dtype=torch.float32, device=dev)
+        pred = torch.empty(n, 2, dtype=torch.float32, device=dev)
+        self._bad.zero_()
+        xs = self.static_batch.x.view(B, N)
+
+        def before(s):
+            self.alpha.copy_(ftab[s, 0])
+            self.j.copy_(itab[s, :B])
+
+        def after(s):
+            first, cnt, fresh, weighted, kept = meta[s]
+            if weighted or fresh:
+                _cabi.check(_cabi.lib().mlg_attr_eg_accumulate(
+                    _cabi.fptr(self.out_g), _cabi.fptr(xs), _cabi.fptr(self._bank), M, _cabi.iptr(self.j),
+                    _cabi.fptr(ftab[s, 1]), _cabi.iptr(itab[s, B:]), cnt, N, 0 if fresh else 1,
+                    _cabi.fptr(acc[first:first + cnt]), _cabi.iptr(self._bad), _cabi.stream_ptr()), "mlg_attr_eg_accumulate")
+            if kept:
+                f0.index_copy_(0, dst[s], self.out_pred[:, self.target])
+
+        self._replays(dataset, topo, [r[0] for r in rows], before, after)
+
+        def before1(s):
+            self.alpha.copy_(tab[s, 0])                # alpha = 1: the interpolant is x, whatever bank row j holds
+
+        def after1(s):
+            first, cnt, fresh = meta1[s]
+            L = slice(first, first + cnt)
+            self._accumulate(self.out_pw, S3, tab[s, 2], ptrs[s], cnt, S3, fresh, pw[L])
+            self._accumulate(self.out_pred, 2, tab[s, 2], ptrs[s], cnt, 2, fresh, pred[L])
+
+        self._replays(dataset, topo, plan1, before1, after1)
+        host_nodes, host_pw, host_pred, host_f0, bad = (t.cpu() for t in (acc, pw, pred, f0, self._bad))  # one sync
+        if int(bad[0]):
+            raise RuntimeError("Attributor: a background row index was outside [0, %d)" % M)
+        delta = None
+        if self.completeness:
+            ref = host_f0[:n * S].view(n, S).double().mean(1)
+            delta = (host_pred[:, self.target].double() - ref - host_nodes.double().sum(1)).float()
+        return AttributionResult(host_nodes, gene_view(host_nodes), self._pathways(host_pw, n), host_pred, delta)
 
 
 def ctypes_ptr(t):
