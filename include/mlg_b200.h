@@ -519,6 +519,28 @@ int mlg_knockout_trunk(const float* xs, const float* baseline, int64_t N, int64_
                        void* workspace, int64_t workspace_bytes, float* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Pathway Shapley chains through the classifier head (csrc/pathway_shapley.cu).  The head's input grid is Hg x Wg cells
+ * (146 x 3 pca_dim); pat [n_pat, ld] / bg [M, ld] hold per-cell tables, element ch * Hg * Wg + cell = ReLU(conv2(ReLU(
+ * conv1(cell))))[ch] (64 channels; mlg_head_conv_pool_fwd with a 1 x 1 window).  The (kh, kw) max-pool has stride = kernel,
+ * floor mode: window w = (ho, wo) holds cells (ho kh + dh) * Wg + wo kw + dw.  w1p [Ho * Wo][64][H] is the first Linear's
+ * weight packed by window (w1p[w][ch][i] = W1[i, ch * Ho * Wo + w]), b1 [H], w1age [H] its age column (NULL: no age; then
+ * age is not read), age [n_pat], w3 [2, H] / b3 [2] the second Linear.  owner int32 [Hg * Wg]: the player of every cell
+ * (-1: none, always the patient's); player k's windows are win_idx[win_ptr[k] .. win_ptr[k+1]).  perm int32 [G, K]: G
+ * permutations of the K players (K <= 1024).  Chain (g, s), s < n_cp, walks perm[g] with patient row chain_pat[s] and
+ * background row chain_bg[g * n_cp + s], from all players at the background row to all at the patient's:
+ *     contrib[(s * G + g) * K + k] = p(after k joins) - p(before),  p0 / pT [(s * G + g)] = p at the start / at the end,
+ * p = softmax(W3 ReLU(h) + b3)[target] evaluated as sigmoid((W3[t] - W3[1 - t]) . ReLU(h) + b3[t] - b3[1 - t]).  Chains
+ * that share g run together; every sum has a fixed order that does not depend on the other chains, no atomics; a player
+ * that changes no window maximum gets exactly 0.  H % 32 == 0, H <= 512, Hg * Wg <= 4096.  An index outside its table
+ * (chain_pat outside [0, n_pat), chain_bg outside [0, M), a perm entry outside [0, K)) is never read: the chain's outputs
+ * become NaN and *bad (int32, device) is set to 1, never cleared by this call.  Capturable, no allocation, no workspace. */
+int mlg_shap_chains(const float* pat, int64_t n_pat, const float* bg, int64_t M, int64_t ld, int64_t Hg, int64_t Wg,
+                    int64_t kh, int64_t kw, const float* w1p, const float* b1, const float* w1age, const float* age,
+                    const float* w3, const float* b3, int target, int64_t H, const int32_t* owner, const int32_t* win_ptr,
+                    const int32_t* win_idx, int64_t K, const int32_t* perm, int64_t G, const int32_t* chain_pat,
+                    const int32_t* chain_bg, int64_t n_cp, float* contrib, float* p0, float* pT, int32_t* bad, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Gene -> pathway pool (models/multilevel_gnn.py:205-239): value mask, gather by gene_pca_match,
  * missing-gene mask, per-gene projection, segment sum -- without materialising [B,C,G,P].
  *     out[b,c,s,p] = sum_{g in seg(b,s)} vm[node] * x[node, c] * w[g,p],  node = b*N + match[b,g] (skipped if < 0)

@@ -14,5 +14,6 @@ from .models import (MultilevelGNN, VAE, DeeperGCN, DiffPool, DiffPoolLayer, SAG
                      dense_diff_pool, MODELS, get_model)
 from .attribution import Attributor, AttributionResult  # noqa: F401,E402
 from .knockout import Knockout, KnockoutResult  # noqa: F401,E402
+from .shapley import PathwayShapley, ShapleyResult  # noqa: F401,E402
 
 __version__ = "0.1.0"

@@ -139,6 +139,11 @@ _SIGNATURES = {
                                     _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp,
                                     _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_vp, _c_i64,
                                     _c_vp, _c_vp]),
+    # (pat, n_pat, bg, M, ld, Hg, Wg, kh, kw, w1p, b1, w1age, age, w3, b3, target, H, owner, win_ptr, win_idx, K, perm, G,
+    #  chain_pat, chain_bg, n_cp, contrib, p0, pT, bad, stream)
+    "mlg_shap_chains": (_c_int, [_c_vp, _c_i64, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64, _c_vp, _c_vp, _c_vp,
+                                 _c_vp, _c_vp, _c_vp, _c_int, _c_i64, _c_vp, _c_vp, _c_vp, _c_i64, _c_vp, _c_i64, _c_vp,
+                                 _c_vp, _c_i64, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp]),
     "mlg_pool_fwd": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64, _c_i64,
                               _c_i64, _c_int, _c_vp, _c_vp]),
     "mlg_pool_bwd_x": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_vp, _c_i64, _c_i64, _c_i64, _c_i64,
