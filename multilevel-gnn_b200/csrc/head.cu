@@ -602,6 +602,15 @@ struct MlpBwdP {
   float *g_a0, *g_W0, *g_b0, *g_W3, *g_b3;
 };
 
+// Rows of dL/dz1 per thread group in head_mlp_bwd_kernel's input-gradient pass: the smallest of 4, 8, 16 whose ngrp groups
+// cover all RT rows.  RT (32 or 64) is a multiple of each choice, so a group that starts below RT also ends at or below it:
+// no group reads past the RT x D dL/dz1 tile, and none is skipped.  A plain ceil(RT / ngrp) gives 5, 6 or 7 for
+// D in 320..480, which the unrolled loop cannot take.
+__host__ __device__ inline int mlp_bwd_rows_per_group(int RT, int ngrp) {
+  const int need = (RT + ngrp - 1) / ngrp;
+  return need <= 4 ? 4 : need <= 8 ? 8 : 16;
+}
+
 template <int RT, int KSL>
 __global__ void __launch_bounds__(512) head_mlp_bwd_kernel(const MlpBwdP P) {
   constexpr int KS = KSL, WLD = KSL + 1;
@@ -671,7 +680,7 @@ __global__ void __launch_bounds__(512) head_mlp_bwd_kernel(const MlpBwdP P) {
   // ---- input gradient slice: g_a0[r][k0 + k] = sum_n dz1[r][n] W0[n][k0 + k]; thread = (k, group of rows) ----
   if (P.g_a0) {
     const int k = threadIdx.x & (KS - 1), grp = threadIdx.x / KS, ngrp = blockDim.x / KS;
-    const int rpg = (RT + ngrp - 1) / ngrp;            // rows per group: 4, 8 or 16
+    const int rpg = mlp_bwd_rows_per_group(RT, ngrp);
     const int r0 = grp * rpg;
     float acc[16];
 #pragma unroll
@@ -887,12 +896,16 @@ extern "C" int mlg_head_mlp_bwd(const float* g_pred, const float* g_loss, const 
   const int RT = R <= 32 ? 32 : 64, ks = mlp_ks(R, D);
   const size_t smem = ((size_t)D * (ks + 1) + (size_t)ks * RT + (size_t)RT * D + 2 * RT) * 4;
   MLG_CHECK_ARG(smem <= 227 * 1024, "mlg_head_mlp_bwd: %lld rows x %lld hidden units exceed shared memory", (long long)R, (long long)D);
+  const int threads = D < 256 ? 256 : (int)D;
+  const int ngrp = threads / ks;
+  MLG_CHECK_ARG(mlp_bwd_rows_per_group(RT, ngrp) * ngrp >= RT, "mlg_head_mlp_bwd: %d row groups of at most 16 rows do not cover %d rows",
+                ngrp, RT);
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned blocks = (unsigned)mlp_slices(R, D, K);
 #define MLG_MLP_B(RR, KK)                                                                                                \
   do {                                                                                                                   \
     MLG_CUDA(cudaFuncSetAttribute(head_mlp_bwd_kernel<RR, KK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    head_mlp_bwd_kernel<RR, KK><<<blocks, (unsigned)(D < 256 ? 256 : D), smem, st>>>(P);                                                 \
+    head_mlp_bwd_kernel<RR, KK><<<blocks, (unsigned)threads, smem, st>>>(P);                                            \
   } while (0)
   if (RT == 32) MLG_MLP_B(32, 64);
   else if (ks == 64) MLG_MLP_B(64, 64);

@@ -264,11 +264,14 @@ def feature_loss(pca_feature, pca_w, info_mask, pathway_indexs, pca_loss=False, 
     return loss
 
 
-def multilevel_forward(sd, batch, args, training=False, return_acts=False):
+def multilevel_forward(sd, batch, args, training=False, return_acts=False, pool_arg=None):
     """MultilevelGNN.forward, models/multilevel_gnn.py:132-292, for the configuration family the
     shipped YAMLs select (node_embedding, sage/rsage GraphConv stack, optional dense/res/
     repeat_mask, value_att_mask, linear_projection pool, conv1x1 head).  Dropout layers are
-    identity (eval) -- parity runs use eval mode or p=0."""
+    identity (eval) -- parity runs use eval mode or p=0.
+    pool_arg [B, C, Ho, Wo] (optional): the element each max-pool window takes, as the index dh * kw + dw inside the window.
+    The pool then gathers that element instead of comparing, so that a window whose two largest values lie within rounding
+    of each other takes the same element, and routes its gradient to the same pixel, as the implementation under test."""
     n3 = sd["node_embedding"].shape[0] if "node_embedding" in sd else None
     mask_x = batch.x
     x = batch.x.reshape(-1, 1)
@@ -314,7 +317,14 @@ def multilevel_forward(sd, batch, args, training=False, return_acts=False):
     for ci in conv_keys:
         wt = sd["conv_model.%d.weight" % ci]
         x = F.relu(F.conv2d(x, wt, sd["conv_model.%d.bias" % ci], padding=wt.shape[-1] // 2))
-    x = F.max_pool2d(x, (args.pathway_pool_dim, args.pca_pool_dim))
+    if pool_arg is None:
+        x = F.max_pool2d(x, (args.pathway_pool_dim, args.pca_pool_dim))
+    else:
+        kh, kw = args.pathway_pool_dim, args.pca_pool_dim
+        b, c, h, w = x.shape
+        ho, wo = h // kh, w // kw
+        win = x[:, :, :ho * kh, :wo * kw].reshape(b, c, ho, kh, wo, kw).permute(0, 1, 2, 4, 3, 5).reshape(b, c, ho, wo, kh * kw)
+        x = win.gather(4, pool_arg.long().unsqueeze(-1)).squeeze(-1)
     x = torch.flatten(x, start_dim=1)
     if args.use_age:
         x = torch.cat([x, batch.age[:, None]], dim=-1)

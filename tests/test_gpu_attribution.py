@@ -71,21 +71,28 @@ def _input_grads(model, batch, Rw, explicit=False):
     return torch.autograd.grad(loss, [x, age, feat], allow_unused=True)
 
 
-FULL = [("gbm", 3), ("kirc", 3), ("lgg", 3), ("gbm", 40), ("lgg", 64)]
+FULL = [("gbm", 3), ("kirc", 3), ("lgg", 3), ("gbm", 40), ("lgg", 64), ("gbm", 32), ("kirc", 64)]
+CHUNKED = 32       # from this width on: the float64 oracle over chunks of graphs (test_gpu_batch_widths.py)
 
 
-@pytest.mark.parametrize("cfg,bsz", FULL, ids=["gbm_b3", "kirc_b3", "lgg_b3", "gbm_b40", "lgg_b64"])
+@pytest.mark.parametrize("cfg,bsz", FULL, ids=["gbm_b3", "kirc_b3", "lgg_b3", "gbm_b40", "lgg_b64", "gbm_b32", "kirc_b64"])
 def test_input_gradients_full_size_vs_oracle(mlg, cfg, bsz):
+    from test_gpu_batch_widths import ORACLE_CHUNK, forward_chunks, oracle_params
     model, args = _model(mlg, cfg, seed=41 + bsz)
     model.eval()
     batch = mlg.synth.multilevel_batch(batch_size=bsz, seed=41 + bsz)
     sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
-    cb = types.SimpleNamespace(**vars(batch))
-    cb.x = batch.x.clone().requires_grad_()
-    cb.age = batch.age.clone().requires_grad_()
-    pred_r, feat_r = R.multilevel_forward(sd, cb, args)
-    Rw = torch.randn(feat_r.shape, generator=torch.Generator().manual_seed(bsz))
-    g_r = torch.autograd.grad(pred_r[:, 1].sum() + (feat_r * Rw).sum(), [cb.x, cb.age, feat_r], allow_unused=True)
+    # the objective is a sum over graphs: each chunk's input gradients are those of the whole batch
+    chunked = bsz >= CHUNKED
+    dtype = torch.float64 if chunked else torch.float32
+    Rw, parts = None, []
+    for g0, g1, cb, pred_r, feat_r, _ in forward_chunks(oracle_params(sd, (), dtype), batch, args, 3 * mlg.MultilevelGNN.GENES,
+                                                        chunk=ORACLE_CHUNK if chunked else bsz, dtype=dtype, input_grad=True):
+        if Rw is None:
+            Rw = torch.randn((bsz,) + tuple(feat_r.shape[1:]), generator=torch.Generator().manual_seed(bsz))
+        parts.append(torch.autograd.grad(pred_r[:, 1].sum() + (feat_r * Rw[g0:g1].to(dtype)).sum(), [cb.x, cb.age, feat_r],
+                                         allow_unused=True))
+    g_r = [None if parts[0][i] is None else torch.cat([p[i] for p in parts]) for i in range(3)]
     _to_dev(model)
     g = _input_grads(model, batch.to(DEV), Rw.to(DEV))
     tag = "%s B=%d" % (cfg, bsz)

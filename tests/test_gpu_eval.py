@@ -59,24 +59,30 @@ def _batch(mlg, pts, topo):
     return mlg.data.to_device(mlg.data.collate(pts, topo, pin=False), topo, DEV)
 
 
-FULL = [("gbm", 3), ("kirc", 3), ("lgg", 3), ("gbm", 40)]
+FULL = [("gbm", 3), ("kirc", 3), ("lgg", 3), ("gbm", 40), ("gbm", 32), ("kirc", 64), ("gbm", 256)]
+CHUNKED = 32       # from this width on: the float64 oracle over chunks of graphs (test_gpu_batch_widths.py)
 
 
-@pytest.mark.parametrize("cfg,bsz", FULL, ids=["gbm_b3", "kirc_b3", "lgg_b3", "gbm_b40"])
+@pytest.mark.parametrize("cfg,bsz", FULL, ids=["gbm_b3", "kirc_b3", "lgg_b3", "gbm_b40", "gbm_b32", "kirc_b64", "gbm_b256"])
 def test_predict_full_size_vs_oracle(mlg, cfg, bsz):
     """pred and pca_feature of predict against oracle.multilevel_forward on the CPU; the model is left in TRAINING mode
     (predict must not apply dropout) and comes back in it."""
+    from test_gpu_batch_widths import ORACLE_CHUNK, forward_chunks, oracle_params
     model, args = _model(mlg, cfg, seed=31 + bsz)
     batch = mlg.synth.multilevel_batch(batch_size=bsz, seed=31 + bsz)
     sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
-    pred_r, feat_r = R.multilevel_forward(sd, types.SimpleNamespace(**vars(batch)), args)
     _to_dev(model).train()
     pred, feat = model.predict(batch.to(DEV))
     assert model.training
     assert not pred.requires_grad and pred.grad_fn is None and feat.grad_fn is None
     tag = "%s B=%d predict" % (cfg, bsz)
-    _check(pred, pred_r, tag + " pred")
-    _check(feat, feat_r, tag + " pca_feature")
+    chunked = bsz >= CHUNKED
+    dtype = torch.float64 if chunked else torch.float32
+    with torch.no_grad():
+        for g0, g1, _, pred_r, feat_r, _ in forward_chunks(oracle_params(sd, (), dtype), batch, args, 3 * mlg.MultilevelGNN.GENES,
+                                                           chunk=ORACLE_CHUNK if chunked else bsz, dtype=dtype):
+            _check(pred[g0:g1], pred_r, "%s graphs %d..%d pred" % (tag, g0, g1 - 1))
+            _check(feat[g0:g1], feat_r, "%s graphs %d..%d pca_feature" % (tag, g0, g1 - 1))
 
 
 def test_predict_matches_eager_eval(mlg):

@@ -49,24 +49,24 @@ def _multilevel_case(mlg, cfg, bsz, seed, **overrides):
     return model, args, batch, weight, sd
 
 
-FULL = [("gbm", 3, {}), ("kirc", 3, {}), ("lgg", 3, {"gnn_name": "rsage"}), ("lgg", 3, {}), ("gbm", 40, {})]
+FULL = [("gbm", 3, {}), ("kirc", 3, {}), ("lgg", 3, {"gnn_name": "rsage"}), ("lgg", 3, {}), ("gbm", 40, {}),
+        ("gbm", 32, {}), ("kirc", 64, {}), ("lgg", 64, {}), ("gbm", 256, {})]
+# the benchmarked widths (gbm 32, kirc / lgg 64, the strong-scaling leg's 256 graphs on one GPU) take the float64 oracle over
+# chunks of graphs (test_gpu_batch_widths.py); the small batches keep the one fp32 pass they always had
+CHUNKED = 32
 
 
-@pytest.mark.parametrize("cfg,bsz,over", FULL, ids=["gbm_b3", "kirc_b3", "lgg_rsage_b3", "lgg_b3", "gbm_b40"])
+@pytest.mark.parametrize("cfg,bsz,over", FULL, ids=["gbm_b3", "kirc_b3", "lgg_rsage_b3", "lgg_b3", "gbm_b40", "gbm_b32", "kirc_b64",
+                                                     "lgg_b64", "gbm_b256"])
 def test_multilevel_full_size_vs_oracle(mlg, cfg, bsz, over):
     """pred, pooled features, per-layer activations, feature loss, BCE loss and EVERY parameter gradient of the default
     CUDA path at N = 15 405 / G = 25 015 against oracle.multilevel_forward + feature_loss + bce_loss on the CPU."""
+    from test_gpu_batch_widths import ORACLE_CHUNK, oracle_params, train_oracle
     model, args, batch, weight, sd = _multilevel_case(mlg, cfg, bsz, seed=21 + bsz, **over)
-    # --- oracle (CPU, autograd through the reference's op order) ---
     names = [k for k, p in model.named_parameters() if p.requires_grad and not k.endswith("lin_l.weight")]
-    leaf = {k: (v.clone().requires_grad_() if k in names else v) for k, v in sd.items()}
-    cb = _cpu_batch(batch)
-    pred_r, feat_r, acts_r = R.multilevel_forward(leaf, cb, args, return_acts=True)
-    fl_r = R.feature_loss(feat_r, leaf["learnable_pca_params"], leaf["info_mask"], model.pathway_indexs,
-                          pca_loss=args.pca_loss, pca_indep_loss=args.pca_indep_loss)
-    loss_r = R.bce_loss(pred_r, cb.y.reshape(-1, 2), weight if args.weight_balance else None) + fl_r
-    g_r = torch.autograd.grad(loss_r, [leaf[k] for k in names], allow_unused=True)
+    n = 3 * mlg.MultilevelGNN.GENES
     # --- CUDA path, shipped defaults ---
+    pathway_indexs = model.pathway_indexs.clone()
     model.to(DEV)
     model.pathway_indexs = model.pathway_indexs.to(DEV)
     acts = {}
@@ -82,10 +82,22 @@ def test_multilevel_full_size_vs_oracle(mlg, cfg, bsz, over):
     params = dict(model.named_parameters())
     g = torch.autograd.grad(loss, [params[k] for k in names], allow_unused=True)
     tag = "%s B=%d" % (cfg, bsz)
-    _check(pred, pred_r, tag + " pred")
-    _check(feat, feat_r, tag + " pca_feature")
-    for k in ("gnn0", "gnn1"):
-        _check(acts[k], acts_r[k], tag + " " + k)
+
+    # --- oracle (CPU, autograd through the reference's op order), compared chunk by chunk ---
+    def visit(g0, g1, pred_r, feat_r, acts_r):
+        part = "%s graphs %d..%d" % (tag, g0, g1 - 1)
+        _check(pred[g0:g1], pred_r, part + " pred")
+        _check(feat[g0:g1], feat_r, part + " pca_feature")
+        for k in ("gnn0", "gnn1"):
+            _check(acts[k][g0 * n:g1 * n], acts_r[k], part + " " + k)
+
+    chunked = bsz >= CHUNKED
+    loss_r, g_r = train_oracle(oracle_params(sd, names, torch.float64 if chunked else torch.float32), names, _cpu_batch(batch),
+                               args, n, pathway_indexs, weight if args.weight_balance else None,
+                               chunk=ORACLE_CHUNK if chunked else bsz, dtype=torch.float64 if chunked else torch.float32,
+                               visit=visit)
+    fl_r = R.feature_loss(None, sd["learnable_pca_params"], sd["info_mask"], pathway_indexs, pca_loss=args.pca_loss,
+                          pca_indep_loss=args.pca_indep_loss)
     _check(torch.as_tensor(fl).reshape(()), torch.as_tensor(fl_r).reshape(()), tag + " feature_loss")
     _check(loss, loss_r, tag + " loss")
     for k, a, c in zip(names, g, g_r):

@@ -504,12 +504,13 @@ def test_pool_linearity_and_oracle(mlg):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("P", [1, 2, 3, 5, 8])
-@pytest.mark.parametrize("bsz", [3, 8, 13])
+@pytest.mark.parametrize("bsz", [3, 8, 13, 32, 64, 256])
 def test_pool_c32_lane_group_kernels(mlg, P, bsz):
     """C == 32 pool kernels (8-lane groups on 128-bit lanes, mlg_pool_fwd / mlg_pool_bwd): forward and both gradients
     against autograd of the oracle's gather / scatter formula (models/multilevel_gnn.py:212-239), with the value mask, for
     every packed-butterfly width (P -> 1, 2, 4, 8 values per group) and replica counts that leave idle lane groups (3),
-    fill one warp exactly (8) and end in a partial chunk (13)."""
+    fill one warp exactly (8), end in a partial chunk (13), and the benchmarked widths (32, 64, 256: 4, 8 and 32 warps of
+    8 replicas, workspace [ceil(B / 8), G, P], pool.cu:675-681)."""
     from multilevel_gnn_b200 import functional as Fn, graph, synth
     genes, slots, C = 200, 1500, 32
     b = synth.multilevel_batch(batch_size=bsz, genes=genes, slots=slots, intra_edges=100, seed=21)
@@ -585,7 +586,7 @@ def ctypes_ptr(t):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("bsz", [3, 16, 40])
+@pytest.mark.parametrize("bsz", [3, 16, 17, 40, 64, 256])
 def test_node_major_gradient_between_pool_and_aggregation(mlg, bsz):
     """mlg_pool_bwd_layout(gx_node_major=1) writes the same gradient as mlg_pool_bwd, at row i * B + b instead of b * N + i,
     and mlg_gather_sum_nm on it equals mlg_gather_sum on the graph-major tensor (backward aggregation of the transform-first
